@@ -3,6 +3,7 @@
 bench.py -- cell-updates/s (float64) of the finite-volume time step on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+                    [--dump-outputs DIR]
 
 N > 1 is launched by the driver with torch.distributed.run (one rank per GPU); the grid
 is then N y-slabs of the per-GPU size (weak scaling) with NCCL halo exchange and an
@@ -154,6 +155,27 @@ def build_problem(pyclaw, workload, n, nranks, torch):
     else:
         raise SystemExit("unknown workload %s" % workload)
     return state, solver
+
+
+DUMP_CELLS = 1 << 20   # cells kept per field by --dump-outputs: 5 x 2^20 float64 = 40 MB for Euler
+
+
+def dump_outputs(outdir, solution, solver):
+    """Write what the caller of solver.evolve_to_time holds after the last timed step, as float64
+    .npy files: q (all cells, or on a larger grid the same DUMP_CELLS cells drawn by
+    numpy.random.default_rng(0), shape [meqn, cells]), t, and the step's cflmax / dtmin / dtmax."""
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    q = solution.state.q.as_subclass(torch.Tensor)   # [m, i, j]
+    meqn, cells = q.shape[0], q[0].numel()
+    if cells > DUMP_CELLS:
+        flat = np.sort(np.random.default_rng(0).choice(cells, DUMP_CELLS, replace=False))
+        idx = [torch.as_tensor(a, device=q.device) for a in np.unravel_index(flat, q.shape[1:])]
+        q = q[(slice(None),) + tuple(idx)]
+    np.save(os.path.join(outdir, "q.npy"), q.reshape(meqn, -1).cpu().numpy())
+    for name, v in (("t", solution.t), ("cflmax", solver.status["cflmax"]),
+                    ("dtmin", solver.status["dtmin"]), ("dtmax", solver.status["dtmax"])):
+        np.save(os.path.join(outdir, name + ".npy"), np.array([v], dtype=np.float64))
 
 
 class ClockSampler(threading.Thread):
@@ -378,7 +400,12 @@ def main():
     ap.add_argument("--no-quiescent-leg", action="store_true", help="skip timing the application's own (quiescent) field")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer e2e leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the solution they computed to DIR/<name>.npy "
+                         "(rank 0's slab at N > 1) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU solution: it needs --impl ours")
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
 
@@ -512,6 +539,9 @@ def main():
     run = timed_run(field, args.steps, max(args.warmup, 3), True)
     value, ms, accepted, clocks = run["value"], run["ms"], run["accepted"], run["clocks"]
     state, solver, solution = run["state"], run["solver"], run["solution"]
+    if args.dump_outputs and rank == 0:
+        # before the e2e leg below, which steps this solution further
+        dump_outputs(args.dump_outputs, solution, solver)
     _lib.set_variant(args.arithmetic)
 
     # ---- e2e at N > 1: every rank uploads its slab from pinned host memory, takes one step
