@@ -381,9 +381,57 @@ def annulus(mx=40, my=120, petsc=False, tfinal=1.0, outdir=None):
     return _run(pyclaw, solver, state, tfinal, 10, outdir)
 
 
+def euler3d(mx=64, my=64, mz=64, petsc=False, tfinal=0.1, dim_split=True, outdir=None):
+    """3-D Euler equations (Roe solver with entropy fix, pyclaw.riemann.euler_3d): a spherical blast
+    wave in the unit box with reflecting walls.  Gas at rest, rho = 1; pressure 10 inside the sphere
+    of radius 0.2 around the centre, 0.1 outside.  dim_split=False runs the unsplit step with
+    transverse corrections (order_trans = 22)."""
+    pyclaw = _pc(petsc)
+    solver = pyclaw.ClawSolver3D()
+    solver.rp = pyclaw.riemann.euler_3d
+    solver.dim_split = dim_split
+    solver.mwaves, solver.limiters = 3, pyclaw.limiters.tvd.MC
+    for i in range(3):
+        solver.bc_lower[i] = solver.bc_upper[i] = pyclaw.BC.reflecting
+    grid = pyclaw.Grid([pyclaw.Dimension('x', 0.0, 1.0, mx), pyclaw.Dimension('y', 0.0, 1.0, my),
+                        pyclaw.Dimension('z', 0.0, 1.0, mz)])
+    state = pyclaw.State(grid, 5)
+    gamma = 1.4
+    state.aux_global.update(gamma=gamma, gamma1=gamma - 1.0)
+    grid.compute_c_center()
+    X, Y, Z = grid._c_center
+    r = np.sqrt((X - 0.5) ** 2 + (Y - 0.5) ** 2 + (Z - 0.5) ** 2)
+    p = np.where(r <= 0.2, 10.0, 0.1)
+    q0 = np.zeros((5,) + X.shape, order='F')
+    q0[0] = 1.0
+    q0[4] = p / (gamma - 1.0)
+    state.q[...] = q0
+    return _run(pyclaw, solver, state, tfinal, 10, outdir)
+
+
+def advection3d(mx=32, my=32, mz=32, petsc=False, tfinal=1.0, dim_split=True, u=1.0, v=0.5, w=0.25, outdir=None):
+    """3-D constant-coefficient advection (pyclaw.riemann.advection_3d) of a Gaussian in the
+    periodic unit box with velocity (u, v, w)."""
+    pyclaw = _pc(petsc)
+    solver = pyclaw.ClawSolver3D()
+    solver.rp = pyclaw.riemann.advection_3d
+    solver.dim_split = dim_split
+    solver.mwaves, solver.limiters = 1, pyclaw.limiters.tvd.MC
+    for i in range(3):
+        solver.bc_lower[i] = solver.bc_upper[i] = pyclaw.BC.periodic
+    grid = pyclaw.Grid([pyclaw.Dimension('x', 0.0, 1.0, mx), pyclaw.Dimension('y', 0.0, 1.0, my),
+                        pyclaw.Dimension('z', 0.0, 1.0, mz)])
+    state = pyclaw.State(grid, 1)
+    state.aux_global.update(u=u, v=v, w=w)
+    grid.compute_c_center()
+    X, Y, Z = grid._c_center
+    state.q[0] = np.exp(-50.0 * ((X - 0.5) ** 2 + (Y - 0.5) ** 2 + (Z - 0.5) ** 2))
+    return _run(pyclaw, solver, state, tfinal, 10, outdir)
+
+
 APPS = {f.__name__: f for f in (acoustics1d, acoustics2d, vc_acoustics2d, shockbubble, shallow1d, shallow2d,
                                 shallow_sphere, stegoton, psystem, acoustics3d, burgers, wcblast,
-                                vc_advection1d, annulus)}
+                                vc_advection1d, annulus, euler3d, advection3d)}
 
 
 def main(argv):

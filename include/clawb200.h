@@ -57,10 +57,16 @@ extern "C" {
 #define CLAWB200_RP_EULER1D 13        /* rp1_euler_with_efix (apps/euler/1d/wcblast); params {gamma,gamma1} */
 /* A Riemann solver supplied by the user as a header and compiled into a variant of the library
  * (pyclaw_b200/csrc/sweep_user.cu, `python -m pyclaw_b200.build --user-rp header.cuh`): the
- * reference's link-time RP_SOURCE seam (Makefile.rules:1-26).  meqn / mwaves / maux come from it. */
+ * reference's link-time RP_SOURCE seam (Makefile.rules:1-26).  meqn / mwaves / maux come from it.
+ * The header defines `template <int IXY> struct RpUser` (1-D / 2-D) and / or `template <int IXYZ>
+ * struct RpUser3` (3-D: solve = rpn3, transverse<ICOOR> = rpt3, double_transverse<ICOOR> = rptt3; the
+ * interface is documented in pyclaw_b200/csrc/rp.cuh and examples/user_rp/rp_acoustics3d_user.cuh). */
 #define CLAWB200_RP_USER 100
-#define CLAWB200_RP_ACOUSTICS3D_VC 8 /* rpn3_vc_acoustics (test/acoustics/3d); aux {impedance, c};
-                                        3-D, dimensional splitting only */
+/* 3-D solvers (clawb200_step3ds / clawb200_step3, both with rpn3 / rpt3 / rptt3) */
+#define CLAWB200_RP_ACOUSTICS3D_VC 8 /* rpn3/rpt3/rptt3_vc_acoustics (test/acoustics/3d); aux {impedance, c} */
+#define CLAWB200_RP_ADVECTION3D 14   /* rpn3/rpt3/rptt3_advection; params {u, v, w}; meqn = mwaves = 1 */
+#define CLAWB200_RP_EULER3D 15       /* rpn3/rpt3/rptt3_euler, Roe + Harten-Hyman entropy fix; params {gamma,
+                                        gamma1}; q = (rho, rho u, rho v, rho w, E), meqn 5, mwaves 3 */
 
 /* Boundary condition ids = pyclaw.BC (src/pyclaw/solver.py:17-23) */
 #define CLAWB200_BC_CUSTOM 0
@@ -88,7 +94,7 @@ extern "C" {
 /* Problem description: what the reference spreads over the f2py argument lists, the
  * `method` array (clawpack.py:192-212) and the cparam / ClawParams module state. */
 typedef struct clawb200_problem {
-    int ndim;                      /* 1 or 2 */
+    int ndim;                      /* 1, 2 or 3 */
     int meqn, mwaves, maux, mbc;
     int mx, my;                    /* interior cells (my = 1 in 1-D) */
     double dx, dy;
@@ -215,7 +221,9 @@ int clawb200_bc_fill(const clawb200_problem *p, double *q, int narr, int idim, i
  * algorithm, idir = 1, 2, 3.  p->ndim = 3; p->mx, my, dx, dy as usual, the third dimension
  * travels as (mz, dz); the field is q[m][k][j][i] with p->pitch = padded row length and
  * p->mstride >= pitch*(my+2mbc)*(mz+2mbc).  q_out receives qold in cells the sweep does not
- * touch; q_in != q_out. */
+ * touch; q_in != q_out.  p->rp_id: any 3-D solver above (meqn / mwaves / maux checked per solver);
+ * the environment variable CLAWB200_STEP3DS_PLANES=1 (an A/B knob of the vc-acoustics kernels) makes
+ * every other solver fail with CLAWB200_ERR_UNSUPPORTED. */
 int clawb200_step3ds(const clawb200_problem *p, int mz, double dz, const double *q_in, double *q_out,
                      const double *aux, double dt, int idir, double *cfl_dev, void *stream);
 /* classic3.step3 (src/fortran/3d/classic/step3.f:2-594 with flux3.f:5-595 and the rpt3 / rptt3
@@ -223,7 +231,8 @@ int clawb200_step3ds(const clawb200_problem *p, int mz, double dz, const double 
  * clawb200_step3ds.  p->method[2] = 0, 10, 11, 20, 21 or 22 (flux3.f:42-68; ClawSolver3D.no_trans
  * = 0, trans_inc = 11, trans_cor = 22).  qold has its ghost cells filled; the interior of qnew is
  * the result (qnew receives qold elsewhere); qold != qnew.  `scratch` is caller-owned device memory
- * of clawb200_step3_scratch_doubles(p) doubles (the per-cell flux increments of one sweep family). */
+ * of clawb200_step3_scratch_doubles(p) = 14 * meqn * mstride doubles (the per-cell flux increments of
+ * one sweep family). */
 long long clawb200_step3_scratch_doubles(const clawb200_problem *p);
 int clawb200_step3(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
                    const double *aux, double dt, double *scratch, double *cfl_dev, void *stream);
@@ -253,7 +262,8 @@ int clawb200_halo_unpack(const clawb200_problem *p, double *q, int narr, int row
  * the very device functions that are inlined into the sweeps.
  * Structure of arrays: ql[m][n], qr[m][n] (left / right state of each interface), auxl[ma][n],
  * auxr[ma][n] (aux of the cell on either side; NULL for solvers that read none),
- * wave[m*mwaves+mw][n], s[mw][n], amdq[m][n], apdq[m][n].  ixy = 1 | 2 (ignored in 1-D).
+ * wave[m*mwaves+mw][n], s[mw][n], amdq[m][n], apdq[m][n].  ixy = 1 | 2 (ignored in 1-D), 1 | 2 | 3
+ * for the 3-D solvers (p->ndim = 3: rpn3; transverse solves are 2-D only).
  * clawb200_rp_transverse: rpt2 with the Roe data of the interface (ql, qr); imp = 1 splits asdq
  * moving into the left cell, imp = 2 into the right cell. */
 int clawb200_rp_solve(const clawb200_problem *p, int ixy, long long n, const double *ql,

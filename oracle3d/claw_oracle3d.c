@@ -1,0 +1,577 @@
+/*
+ * claw_oracle3d.c -- CPU restatement of the 3-D classic steps for the 3-D Riemann solvers without
+ * aux data (TEST INFRASTRUCTURE ONLY, never linked into the product), next to oracle/claw_oracle.c,
+ * which holds the same steps for the variable-coefficient acoustics solver:
+ *   src/fortran/3d/classic/step3ds.f:2-376 with flux3.f:176-237 (dimensional splitting)
+ *   src/fortran/3d/classic/step3.f:2-594 with flux3.f:5-595 (unsplit, method(3) = 0, 10, 11, 20, 21, 22)
+ *   limiter.f / philim.f
+ * in the statement order of oracle/claw_oracle.c (flux3_ds, oracle_step3ds, flux3, oracle_step3,
+ * limiter, philim), with the rp_id switch of this file's solvers.  The solvers live in the external
+ * clawpack/riemann repository (un-vendored): rpn3 / rpt3 / rptt3_advection and rpn3 / rpt3 /
+ * rptt3_euler (Roe + Harten-Hyman entropy fix), restated from the published algorithm (LeVeque 2002,
+ * sec. 15.3 and 18.8), parity unpinned.
+ * Strict IEEE double: compiled without FMA contraction (oracle3d/Makefile).
+ */
+#include <math.h>
+#include <stdlib.h>
+#include <string.h>
+
+#define RP_ADVECTION3D 14 /* p[0..2] = u, v, w          */
+#define RP_EULER3D 15     /* p[0] = gamma, p[1] = gamma1 */
+
+typedef struct {
+    int rp_id;
+    double p[8];
+} rp_ctx3;
+
+static inline double dmax2(double a, double b) { return (a > b) ? a : b; }
+static inline double dmin2(double a, double b) { return (a < b) ? a : b; }
+
+/* slice indexing: Fortran index i in [1-mbc, maxm+mbc] -> offset i+mbc-1 */
+#define IX(i) ((i) + mbc - 1)
+#define Q2(arr, m, i) arr[(m) + meqn * IX(i)]
+#define WV(m, mw, i) wave[(m) + meqn * ((mw) + mwaves * IX(i))]
+#define SP(mw, i) s[(mw) + mwaves * IX(i)]
+
+/* ixyz = 1, 2, 3 is the sweep direction; the transverse direction icoor = 2 (y-like) / 3 (z-like)
+   has velocity component rp3_dir(ixyz, icoor) */
+static inline int rp3_dir(int ixyz, int icoor) { return (ixyz - 1 + icoor - 1) % 3 + 1; }
+
+/* ---- rpn3 / rpt3 / rptt3_advection ---- */
+static void rpn3_advection(const rp_ctx3 *c, int ixyz, int mbc, int mx, const double *ql, const double *qr,
+                           double *wave, double *s, double *amdq, double *apdq)
+{
+    const int meqn = 1, mwaves = 1;
+    for (int i = 2 - mbc; i <= mx + mbc; i++) {
+        WV(0, 0, i) = Q2(ql, 0, i) - Q2(qr, 0, i - 1);
+        SP(0, i) = c->p[ixyz - 1];
+        Q2(amdq, 0, i) = dmin2(SP(0, i), 0.0) * WV(0, 0, i);
+        Q2(apdq, 0, i) = dmax2(SP(0, i), 0.0) * WV(0, 0, i);
+    }
+}
+
+/* rpt3_advection (and rptt3_advection, the same split of an already split fluctuation) */
+static void rpt3_advection(const rp_ctx3 *c, int ixyz, int icoor, int mbc, int mx, const double *asdq,
+                           double *bmasdq, double *bpasdq)
+{
+    const int meqn = 1;
+    const double st = c->p[rp3_dir(ixyz, icoor) - 1];
+    for (int i = 2 - mbc; i <= mx + mbc; i++) {
+        Q2(bmasdq, 0, i) = dmin2(st, 0.0) * Q2(asdq, 0, i);
+        Q2(bpasdq, 0, i) = dmax2(st, 0.0) * Q2(asdq, 0, i);
+    }
+}
+
+/* ---- rpn3 / rpt3 / rptt3_euler ---- */
+/* Roe averages of the interface between l and r: roe = {u, v, w, enth, a, u^2 + v^2 + w^2} */
+static void euler3_roe(double gamma1, const double *l, const double *r, double *roe)
+{
+    double rhsqrtl = sqrt(l[0]), rhsqrtr = sqrt(r[0]);
+    double pl = gamma1 * (l[4] - 0.5 * (l[1] * l[1] + l[2] * l[2] + l[3] * l[3]) / l[0]);
+    double pr = gamma1 * (r[4] - 0.5 * (r[1] * r[1] + r[2] * r[2] + r[3] * r[3]) / r[0]);
+    double rhsq2 = rhsqrtl + rhsqrtr;
+    for (int k = 0; k < 3; k++) roe[k] = (l[1 + k] / rhsqrtl + r[1 + k] / rhsqrtr) / rhsq2;
+    double enth = (((l[4] + pl) / rhsqrtl + (r[4] + pr) / rhsqrtr)) / rhsq2;
+    double uvw2 = roe[0] * roe[0] + roe[1] * roe[1] + roe[2] * roe[2];
+    roe[3] = enth;
+    roe[4] = sqrt(gamma1 * (enth - 0.5 * uvw2));
+    roe[5] = uvw2;
+}
+
+/* d split into the eigenvectors of the Roe matrix of direction mt (velocity component 1..3):
+   wave 0 at un - a, wave 1 at un (entropy and both shear jumps), wave 2 at un + a */
+static void euler3_waves(int mt, double gamma1, const double *roe, const double *d, double wv[5][3], double *sp)
+{
+    const int m1 = mt % 3 + 1, m2 = (mt + 1) % 3 + 1;
+    double un = roe[mt - 1], u1 = roe[m1 - 1], u2 = roe[m2 - 1];
+    double enth = roe[3], a = roe[4], uvw2 = roe[5];
+    double a3 = gamma1 / (a * a) * ((enth - uvw2) * d[0] + roe[0] * d[1] + roe[1] * d[2] + roe[2] * d[3] - d[4]);
+    double b1 = d[m1] - u1 * d[0], b2 = d[m2] - u2 * d[0];
+    double a5 = (d[mt] + (a - un) * d[0] - a * a3) / (2.0 * a);
+    double a1 = d[0] - a3 - a5;
+    wv[0][0] = a1; wv[mt][0] = a1 * (un - a); wv[m1][0] = a1 * u1; wv[m2][0] = a1 * u2;
+    wv[4][0] = a1 * (enth - un * a); sp[0] = un - a;
+    wv[0][1] = a3; wv[mt][1] = a3 * un; wv[m1][1] = a3 * u1 + b1; wv[m2][1] = a3 * u2 + b2;
+    wv[4][1] = a3 * 0.5 * uvw2 + b1 * u1 + b2 * u2; sp[1] = un;
+    wv[0][2] = a5; wv[mt][2] = a5 * (un + a); wv[m1][2] = a5 * u1; wv[m2][2] = a5 * u2;
+    wv[4][2] = a5 * (enth + un * a); sp[2] = un + a;
+}
+
+/* rpn3_euler: the operations of rp1_euler_with_efix (oracle/claw_oracle.c, rpn_euler1d) with the
+   full kinetic energy; with v = w = 0 they are the same operations on the same values */
+static void rpn3_euler(const rp_ctx3 *c, int ixyz, int mbc, int mx, const double *ql, const double *qr,
+                       double *wave, double *s, double *amdq, double *apdq)
+{
+    const int meqn = 5, mwaves = 3, mu = ixyz;
+    const double gamma1 = c->p[1];
+    for (int i = 2 - mbc; i <= mx + mbc; i++) {
+        const double *l = &Q2(qr, 0, i - 1), *r = &Q2(ql, 0, i);
+        double roe[6], d[5], wv[5][3], sp[3], am[5];
+        euler3_roe(gamma1, l, r, roe);
+        for (int m = 0; m < 5; m++) d[m] = r[m] - l[m];
+        euler3_waves(mu, gamma1, roe, d, wv, sp);
+        /* Harten-Hyman entropy fix on the acoustic waves, left-going fluctuation first */
+        int done = 0;
+        double ulx = l[1] / l[0], uly = l[2] / l[0], ulz = l[3] / l[0];
+        double cl = sqrt(gamma1 * (gamma1 + 1.0) * (l[4] / l[0] - 0.5 * (ulx * ulx + uly * uly + ulz * ulz)));
+        double s0 = l[mu] / l[0] - cl;
+        if (s0 >= 0.0 && sp[0] > 0.0) {
+            for (int m = 0; m < 5; m++) am[m] = 0.0;
+            done = 1;
+        }
+        if (!done) {
+            double q1[5];
+            for (int m = 0; m < 5; m++) q1[m] = l[m] + wv[m][0];
+            double p1 = gamma1 * (q1[4] - 0.5 * (q1[1] * q1[1] + q1[2] * q1[2] + q1[3] * q1[3]) / q1[0]);
+            double c1 = sqrt((gamma1 + 1.0) * p1 / q1[0]);
+            double s1 = q1[mu] / q1[0] - c1;
+            double sfract;
+            if (s0 < 0.0 && s1 > 0.0) sfract = s0 * (s1 - sp[0]) / (s1 - s0);
+            else if (sp[0] < 0.0) sfract = sp[0];
+            else sfract = 0.0;
+            for (int m = 0; m < 5; m++) am[m] = sfract * wv[m][0];
+            if (sp[1] >= 0.0) done = 1;
+        }
+        if (!done) {
+            for (int m = 0; m < 5; m++) am[m] = am[m] + sp[1] * wv[m][1];
+            double urx = r[1] / r[0], ury = r[2] / r[0], urz = r[3] / r[0];
+            double cr = sqrt(gamma1 * (gamma1 + 1.0) * (r[4] / r[0] - 0.5 * (urx * urx + ury * ury + urz * urz)));
+            double s3 = r[mu] / r[0] + cr;
+            double q2[5];
+            for (int m = 0; m < 5; m++) q2[m] = r[m] - wv[m][2];
+            double p2 = gamma1 * (q2[4] - 0.5 * (q2[1] * q2[1] + q2[2] * q2[2] + q2[3] * q2[3]) / q2[0]);
+            double c2 = sqrt((gamma1 + 1.0) * p2 / q2[0]);
+            double s2 = q2[mu] / q2[0] + c2;
+            double sfract = 0.0;
+            int add = 1;
+            if (s2 < 0.0 && s3 > 0.0) sfract = s2 * (s3 - sp[2]) / (s3 - s2);
+            else if (sp[2] < 0.0) sfract = sp[2];
+            else add = 0;
+            if (add) for (int m = 0; m < 5; m++) am[m] = am[m] + sfract * wv[m][2];
+        }
+        for (int m = 0; m < 5; m++) {
+            double df = 0.0;
+            for (int mw = 0; mw < 3; mw++) df = df + sp[mw] * wv[m][mw];
+            Q2(amdq, m, i) = am[m];
+            Q2(apdq, m, i) = df - am[m];
+            for (int mw = 0; mw < 3; mw++) WV(m, mw, i) = wv[m][mw];
+        }
+        for (int mw = 0; mw < 3; mw++) SP(mw, i) = sp[mw];
+    }
+}
+
+/* rpt3_euler (and rptt3_euler, the same split of an already split fluctuation): asdq split with the
+   eigenvectors of the Roe matrix of direction icoor at the Roe averages of interface i, q(:, i-1) | q(:, i) */
+static void rpt3_euler(const rp_ctx3 *c, int ixyz, int icoor, int mbc, int mx, const double *q1d,
+                       const double *asdq, double *bmasdq, double *bpasdq)
+{
+    const int meqn = 5;
+    const double gamma1 = c->p[1];
+    for (int i = 2 - mbc; i <= mx + mbc; i++) {
+        double roe[6], wv[5][3], sp[3];
+        euler3_roe(gamma1, &Q2(q1d, 0, i - 1), &Q2(q1d, 0, i), roe);
+        euler3_waves(rp3_dir(ixyz, icoor), gamma1, roe, &Q2(asdq, 0, i), wv, sp);
+        for (int m = 0; m < 5; m++) {
+            Q2(bmasdq, m, i) = dmin2(sp[0], 0.0) * wv[m][0] + dmin2(sp[1], 0.0) * wv[m][1] + dmin2(sp[2], 0.0) * wv[m][2];
+            Q2(bpasdq, m, i) = dmax2(sp[0], 0.0) * wv[m][0] + dmax2(sp[1], 0.0) * wv[m][1] + dmax2(sp[2], 0.0) * wv[m][2];
+        }
+    }
+}
+
+/* ---- the rp_id switches ---- */
+static void rpn3(const rp_ctx3 *c, int ixyz, int mbc, int mx, const double *ql, const double *qr, double *wave,
+                 double *s, double *amdq, double *apdq)
+{
+    if (c->rp_id == RP_EULER3D) rpn3_euler(c, ixyz, mbc, mx, ql, qr, wave, s, amdq, apdq);
+    else rpn3_advection(c, ixyz, mbc, mx, ql, qr, wave, s, amdq, apdq);
+}
+/* rpt3 and rptt3: neither solver reads aux data, so neither depends on imp / impt */
+static void rpt3(const rp_ctx3 *c, int ixyz, int icoor, int mbc, int mx, const double *q1d, const double *asdq,
+                 double *bmasdq, double *bpasdq)
+{
+    if (c->rp_id == RP_EULER3D) rpt3_euler(c, ixyz, icoor, mbc, mx, q1d, asdq, bmasdq, bpasdq);
+    else rpt3_advection(c, ixyz, icoor, mbc, mx, asdq, bmasdq, bpasdq);
+}
+static int known(int rp_id) { return rp_id == RP_ADVECTION3D || rp_id == RP_EULER3D; }
+
+/* ---- limiter.f / philim.f (as oracle/claw_oracle.c) ---- */
+static double philim(double a, double b, int meth)
+{
+    double r = b / a;
+    switch (meth) {
+    case 2: return dmax2(dmax2(0.0, dmin2(1.0, 2.0 * r)), dmin2(2.0, r));
+    case 3: return (r + fabs(r)) / (1.0 + fabs(r));
+    case 4: {
+        double c = (1.0 + r) / 2.0;
+        return dmax2(0.0, dmin2(dmin2(c, 2.0), 2.0 * r));
+    }
+    case 5: return r;
+    default: return dmax2(0.0, dmin2(1.0, r)); /* philim.f:19: out-of-range ids fall through to minmod */
+    }
+}
+
+static void limiter(int meqn, int mwaves, int mbc, int mx, double *wave, const double *s, const int *mthlim)
+{
+    for (int mw = 0; mw < mwaves; mw++) {
+        if (mthlim[mw] == 0) continue;
+        double dotr = 0.0;
+        for (int i = 0; i <= mx + 1; i++) {
+            double wnorm2 = 0.0;
+            double dotl = dotr;
+            dotr = 0.0;
+            for (int m = 0; m < meqn; m++) {
+                wnorm2 = wnorm2 + WV(m, mw, i) * WV(m, mw, i);
+                dotr = dotr + WV(m, mw, i) * WV(m, mw, i + 1);
+            }
+            if (i == 0) continue;
+            if (wnorm2 == 0.0) continue;
+            double wlimitr;
+            if (SP(mw, i) > 0.0)
+                wlimitr = philim(wnorm2, dotl, mthlim[mw]);
+            else
+                wlimitr = philim(wnorm2, dotr, mthlim[mw]);
+            for (int m = 0; m < meqn; m++) WV(m, mw, i) = wlimitr * WV(m, mw, i);
+        }
+    }
+}
+
+/* the normal part of flux3.f:176-241 on one slice (q1d, uniform dtdx): qadd, fadd and cqxx; returns cfl */
+static double flux3_normal(const rp_ctx3 *c, int ixyz, int meqn, int mwaves, int mbc, int mx, const double *q1d,
+                           double dtdx, int order, const int *mthlim, double *wave, double *s, double *amdq,
+                           double *apdq, double *cqxx, double *qadd, double *fadd)
+{
+    int limit = 0;
+    for (int mw = 0; mw < mwaves; mw++) if (mthlim[mw] > 0) limit = 1;
+    for (int i = 1 - mbc; i <= mx + mbc; i++)
+        for (int m = 0; m < meqn; m++) { Q2(qadd, m, i) = 0.0; Q2(fadd, m, i) = 0.0; Q2(cqxx, m, i) = 0.0; }
+    rpn3(c, ixyz, mbc, mx, q1d, q1d, wave, s, amdq, apdq);
+    for (int i = 1; i <= mx + 1; i++)
+        for (int m = 0; m < meqn; m++) Q2(qadd, m, i) = Q2(qadd, m, i) - dtdx * Q2(apdq, m, i);
+    for (int i = 1; i <= mx + 1; i++)
+        for (int m = 0; m < meqn; m++) Q2(qadd, m, i - 1) = Q2(qadd, m, i - 1) - dtdx * Q2(amdq, m, i);
+    double cfl1d = 0.0;
+    for (int i = 1; i <= mx + 1; i++)
+        for (int mw = 0; mw < mwaves; mw++)
+            cfl1d = dmax2(dmax2(cfl1d, dtdx * SP(mw, i)), -dtdx * SP(mw, i));
+    if (order == 1) return cfl1d;
+    if (limit) limiter(meqn, mwaves, mbc, mx, wave, s, mthlim);
+    for (int i = 2 - mbc; i <= mx + mbc; i++) {
+        double dtdxave = 0.5 * (dtdx + dtdx);
+        for (int m = 0; m < meqn; m++) Q2(cqxx, m, i) = 0.0;
+        for (int mw = 0; mw < mwaves; mw++)
+            for (int m = 0; m < meqn; m++)
+                Q2(cqxx, m, i) = Q2(cqxx, m, i) + 0.5 * fabs(SP(mw, i)) * (1.0 - fabs(SP(mw, i)) * dtdxave) * WV(m, mw, i);
+        for (int m = 0; m < meqn; m++) Q2(fadd, m, i) = Q2(fadd, m, i) + Q2(cqxx, m, i);
+    }
+    return cfl1d;
+}
+
+/* ------------------------------------------------------------------------- */
+/* step3ds.f:2-376 (method(3) < 0), idir = 1, 2, 3; sweeps cover one ghost     */
+/* layer of the other two directions.  q(meqn, 1-mbc:mx+mbc, ..., 1-mbc:mz+mbc) */
+/* ------------------------------------------------------------------------- */
+double oracle3d_step3ds(int rp_id, const double *rp_params, int meqn, int mwaves, int mbc, int mx, int my, int mz,
+                        const double *qold, double *qnew, double dx, double dy, double dz, double dt,
+                        const int *method, const int *mthlim, int idir)
+{
+    if (!known(rp_id) || method[5] > 0) return -1.0;
+    rp_ctx3 c;
+    c.rp_id = rp_id;
+    memcpy(c.p, rp_params, 8 * sizeof(double));
+    int maxm = mx > my ? mx : my;
+    if (mz > maxm) maxm = mz;
+    const int n = maxm + 2 * mbc;
+    double *v[7];
+    for (int a = 0; a < 7; a++) v[a] = (double *)calloc((size_t)n * meqn * mwaves, sizeof(double));
+    double *q1d = v[0], *wave = v[1], *s = v[2], *amdq = v[3], *apdq = v[4], *qadd = v[5], *fadd = v[6];
+    double *cqxx = (double *)calloc((size_t)n * meqn, sizeof(double));
+    const size_t NXs = mx + 2 * mbc, NYs = my + 2 * mbc;
+#define Q4(arr, m, i, j, k) arr[(m) + (size_t)meqn * (((i) + mbc - 1) + NXs * (((j) + mbc - 1) + NYs * ((k) + mbc - 1)))]
+    const double dtd[3] = {dt / dx, dt / dy, dt / dz};
+    const int len[3] = {mx, my, mz};
+    double cfl = 0.0;
+    const int d = idir - 1;
+    const int o1 = (d == 0) ? 1 : 0, o2 = (d == 2) ? 1 : 2;
+    int idx[3];
+    for (idx[o2] = 0; idx[o2] <= len[o2] + 1; idx[o2]++)
+        for (idx[o1] = 0; idx[o1] <= len[o1] + 1; idx[o1]++) {
+            for (int l = 1 - mbc; l <= len[d] + mbc; l++) {
+                idx[d] = l;
+                for (int m = 0; m < meqn; m++) Q2(q1d, m, l) = Q4(qold, m, idx[0], idx[1], idx[2]);
+            }
+            double cfl1d = flux3_normal(&c, idir, meqn, mwaves, mbc, len[d], q1d, dtd[d], method[1], mthlim, wave, s,
+                                        amdq, apdq, cqxx, qadd, fadd);
+            cfl = dmax2(cfl, cfl1d);
+            for (int l = 1; l <= len[d]; l++) {
+                idx[d] = l;
+                for (int m = 0; m < meqn; m++) {
+                    double upd = dtd[d] * (Q2(fadd, m, l + 1) - Q2(fadd, m, l));
+                    Q4(qnew, m, idx[0], idx[1], idx[2]) = Q4(qnew, m, idx[0], idx[1], idx[2]) + Q2(qadd, m, l) - upd;
+                }
+            }
+        }
+    for (int a = 0; a < 7; a++) free(v[a]);
+    free(cqxx);
+    return cfl;
+}
+
+/* gadd / hadd (meqn, 2, -1:1, 1-mbc:maxm+mbc): k = 1..2, j = -1..1 */
+#define GH(arr, m, k, j, i) arr[(m) + meqn * (((k) - 1) + 2 * (((j) + 1) + 3 * IX(i)))]
+
+/* flux3.f:5-595 for a slice without aux data; qadd, fadd, gadd, hadd */
+static double flux3(const rp_ctx3 *c, int ixyz, int meqn, int mwaves, int mbc, int mx, int n1d, const double *q1d,
+                    double dtdx, double dtdy, double dtdz, const int *method, const int *mthlim, double *wave,
+                    double *s, double *qadd, double *fadd, double *gadd, double *hadd, double **v)
+{
+    double *amdq = v[0], *apdq = v[1], *cqxx = v[2];
+    double *bmamdq = v[3], *bmapdq = v[4], *bpamdq = v[5], *bpapdq = v[6];
+    double *cmamdq = v[7], *cmapdq = v[8], *cpamdq = v[9], *cpapdq = v[10];
+    double *cmamdq2 = v[11], *cmapdq2 = v[12], *cpamdq2 = v[13], *cpapdq2 = v[14];
+    double *bmcqxxp = v[15], *bpcqxxp = v[16], *bmcqxxm = v[17], *bpcqxxm = v[18];
+    double *cmcqxxp = v[19], *cpcqxxp = v[20], *cmcqxxm = v[21], *cpcqxxm = v[22];
+    double *bmcmamdq = v[23], *bmcmapdq = v[24], *bpcmamdq = v[25], *bpcmapdq = v[26];
+    double *bmcpamdq = v[27], *bmcpapdq = v[28], *bpcpamdq = v[29], *bpcpapdq = v[30];
+    (void)n1d;
+    for (int i = 1 - mbc; i <= mx + mbc; i++)
+        for (int m = 0; m < meqn; m++)
+            for (int k = 1; k <= 2; k++)
+                for (int j = -1; j <= 1; j++) { GH(gadd, m, k, j, i) = 0.0; GH(hadd, m, k, j, i) = 0.0; }
+    int m3, m4;
+    if (method[2] < 0) { m3 = -1; m4 = 0; }
+    else { m3 = method[2] / 10; m4 = method[2] - 10 * m3; }
+    double cfl1d = flux3_normal(c, ixyz, meqn, mwaves, mbc, mx, q1d, dtdx, method[1], mthlim, wave, s, amdq, apdq,
+                                cqxx, qadd, fadd);
+    if (m3 <= 0) return cfl1d;
+
+#define RPT3(icoor, as, bm, bp) rpt3(c, ixyz, icoor, mbc, mx, q1d, as, bm, bp)
+    RPT3(2, amdq, bmamdq, bpamdq);
+    RPT3(2, apdq, bmapdq, bpapdq);
+    RPT3(3, amdq, cmamdq, cpamdq);
+    RPT3(3, apdq, cmapdq, cpapdq);
+    if (m3 == 2) { /* cqxx split with imp = 1 and imp = 2 (flux3.f:262-283): the same split here */
+        RPT3(2, cqxx, bmcqxxm, bpcqxxm);
+        RPT3(2, cqxx, bmcqxxp, bpcqxxp);
+        RPT3(3, cqxx, cmcqxxm, cpcqxxm);
+        RPT3(3, cqxx, cmcqxxp, cpcqxxp);
+    }
+    /* ---- G fluxes (y-like direction) ---- */
+    if (m4 == 1) {
+        for (int i = 0; i <= mx + 2; i++)
+            for (int m = 0; m < meqn; m++) {
+                Q2(cpapdq2, m, i) = Q2(cpapdq, m, i); Q2(cpamdq2, m, i) = Q2(cpamdq, m, i);
+                Q2(cmapdq2, m, i) = Q2(cmapdq, m, i); Q2(cmamdq2, m, i) = Q2(cmamdq, m, i);
+            }
+    } else if (m4 == 2) {
+        for (int i = 0; i <= mx + 2; i++)
+            for (int m = 0; m < meqn; m++) {
+                Q2(cpapdq2, m, i) = Q2(cpapdq, m, i) - 3.0 * Q2(cpcqxxp, m, i);
+                Q2(cpamdq2, m, i) = Q2(cpamdq, m, i) + 3.0 * Q2(cpcqxxm, m, i);
+                Q2(cmapdq2, m, i) = Q2(cmapdq, m, i) - 3.0 * Q2(cmcqxxp, m, i);
+                Q2(cmamdq2, m, i) = Q2(cmamdq, m, i) + 3.0 * Q2(cmcqxxm, m, i);
+            }
+    }
+    if (m4 > 0) { /* rptt3 */
+        RPT3(2, cpapdq2, bmcpapdq, bpcpapdq);
+        RPT3(2, cpamdq2, bmcpamdq, bpcpamdq);
+        RPT3(2, cmapdq2, bmcmapdq, bpcmapdq);
+        RPT3(2, cmamdq2, bmcmamdq, bpcmamdq);
+    }
+    const double sixth = 1.0 / 6.0;
+    for (int i = 1; i <= mx + 1; i++)
+        for (int m = 0; m < meqn; m++) {
+            const double dl = dtdx, dr = dtdx;
+            GH(gadd, m, 1, 0, i - 1) = GH(gadd, m, 1, 0, i - 1) - 0.5 * dl * Q2(bmamdq, m, i);
+            GH(gadd, m, 2, 0, i - 1) = GH(gadd, m, 2, 0, i - 1) - 0.5 * dl * Q2(bpamdq, m, i);
+            GH(gadd, m, 1, 0, i) = GH(gadd, m, 1, 0, i) - 0.5 * dr * Q2(bmapdq, m, i);
+            GH(gadd, m, 2, 0, i) = GH(gadd, m, 2, 0, i) - 0.5 * dr * Q2(bpapdq, m, i);
+            if (m4 > 0) {
+                GH(gadd, m, 2, 0, i) = GH(gadd, m, 2, 0, i) + sixth * dr * dtdz * (Q2(bpcpapdq, m, i) - Q2(bpcmapdq, m, i));
+                GH(gadd, m, 1, 0, i) = GH(gadd, m, 1, 0, i) + sixth * dr * dtdz * (Q2(bmcpapdq, m, i) - Q2(bmcmapdq, m, i));
+                GH(gadd, m, 2, 1, i) = GH(gadd, m, 2, 1, i) - sixth * dr * dtdz * Q2(bpcpapdq, m, i);
+                GH(gadd, m, 1, 1, i) = GH(gadd, m, 1, 1, i) - sixth * dr * dtdz * Q2(bmcpapdq, m, i);
+                GH(gadd, m, 2, -1, i) = GH(gadd, m, 2, -1, i) + sixth * dr * dtdz * Q2(bpcmapdq, m, i);
+                GH(gadd, m, 1, -1, i) = GH(gadd, m, 1, -1, i) + sixth * dr * dtdz * Q2(bmcmapdq, m, i);
+                GH(gadd, m, 2, 0, i - 1) = GH(gadd, m, 2, 0, i - 1) + sixth * dl * dtdz * (Q2(bpcpamdq, m, i) - Q2(bpcmamdq, m, i));
+                GH(gadd, m, 1, 0, i - 1) = GH(gadd, m, 1, 0, i - 1) + sixth * dl * dtdz * (Q2(bmcpamdq, m, i) - Q2(bmcmamdq, m, i));
+                GH(gadd, m, 2, 1, i - 1) = GH(gadd, m, 2, 1, i - 1) - sixth * dl * dtdz * Q2(bpcpamdq, m, i);
+                GH(gadd, m, 1, 1, i - 1) = GH(gadd, m, 1, 1, i - 1) - sixth * dl * dtdz * Q2(bmcpamdq, m, i);
+                GH(gadd, m, 2, -1, i - 1) = GH(gadd, m, 2, -1, i - 1) + sixth * dl * dtdz * Q2(bpcmamdq, m, i);
+                GH(gadd, m, 1, -1, i - 1) = GH(gadd, m, 1, -1, i - 1) + sixth * dl * dtdz * Q2(bmcmamdq, m, i);
+            }
+            if (m3 >= 2) {
+                GH(gadd, m, 2, 0, i) = GH(gadd, m, 2, 0, i) + dr * Q2(bpcqxxp, m, i);
+                GH(gadd, m, 1, 0, i) = GH(gadd, m, 1, 0, i) + dr * Q2(bmcqxxp, m, i);
+                GH(gadd, m, 2, 0, i - 1) = GH(gadd, m, 2, 0, i - 1) - dl * Q2(bpcqxxm, m, i);
+                GH(gadd, m, 1, 0, i - 1) = GH(gadd, m, 1, 0, i - 1) - dl * Q2(bmcqxxm, m, i);
+            }
+        }
+    /* ---- H fluxes (z-like direction) ---- */
+    if (m4 == 2) {
+        for (int i = 0; i <= mx + 2; i++)
+            for (int m = 0; m < meqn; m++) {
+                Q2(bpapdq, m, i) = Q2(bpapdq, m, i) - 3.0 * Q2(bpcqxxp, m, i);
+                Q2(bpamdq, m, i) = Q2(bpamdq, m, i) + 3.0 * Q2(bpcqxxm, m, i);
+                Q2(bmapdq, m, i) = Q2(bmapdq, m, i) - 3.0 * Q2(bmcqxxp, m, i);
+                Q2(bmamdq, m, i) = Q2(bmamdq, m, i) + 3.0 * Q2(bmcqxxm, m, i);
+            }
+    }
+    if (m4 > 0) { /* rptt3 */
+        RPT3(3, bpapdq, bmcpapdq, bpcpapdq);
+        RPT3(3, bpamdq, bmcpamdq, bpcpamdq);
+        RPT3(3, bmapdq, bmcmapdq, bpcmapdq);
+        RPT3(3, bmamdq, bmcmamdq, bpcmamdq);
+    }
+    for (int i = 1; i <= mx + 1; i++)
+        for (int m = 0; m < meqn; m++) {
+            const double dl = dtdx, dr = dtdx;
+            GH(hadd, m, 1, 0, i - 1) = GH(hadd, m, 1, 0, i - 1) - 0.5 * dl * Q2(cmamdq, m, i);
+            GH(hadd, m, 2, 0, i - 1) = GH(hadd, m, 2, 0, i - 1) - 0.5 * dl * Q2(cpamdq, m, i);
+            GH(hadd, m, 1, 0, i) = GH(hadd, m, 1, 0, i) - 0.5 * dr * Q2(cmapdq, m, i);
+            GH(hadd, m, 2, 0, i) = GH(hadd, m, 2, 0, i) - 0.5 * dr * Q2(cpapdq, m, i);
+            if (m4 > 0) {
+                GH(hadd, m, 2, 0, i) = GH(hadd, m, 2, 0, i) + sixth * dr * dtdy * (Q2(bpcpapdq, m, i) - Q2(bpcmapdq, m, i));
+                GH(hadd, m, 1, 0, i) = GH(hadd, m, 1, 0, i) + sixth * dr * dtdy * (Q2(bmcpapdq, m, i) - Q2(bmcmapdq, m, i));
+                GH(hadd, m, 2, 1, i) = GH(hadd, m, 2, 1, i) - sixth * dr * dtdy * Q2(bpcpapdq, m, i);
+                GH(hadd, m, 1, 1, i) = GH(hadd, m, 1, 1, i) - sixth * dr * dtdy * Q2(bmcpapdq, m, i);
+                GH(hadd, m, 2, -1, i) = GH(hadd, m, 2, -1, i) + sixth * dr * dtdy * Q2(bpcmapdq, m, i);
+                GH(hadd, m, 1, -1, i) = GH(hadd, m, 1, -1, i) + sixth * dr * dtdy * Q2(bmcmapdq, m, i);
+                GH(hadd, m, 2, 0, i - 1) = GH(hadd, m, 2, 0, i - 1) + sixth * dl * dtdy * (Q2(bpcpamdq, m, i) - Q2(bpcmamdq, m, i));
+                GH(hadd, m, 1, 0, i - 1) = GH(hadd, m, 1, 0, i - 1) + sixth * dl * dtdy * (Q2(bmcpamdq, m, i) - Q2(bmcmamdq, m, i));
+                GH(hadd, m, 2, 1, i - 1) = GH(hadd, m, 2, 1, i - 1) - sixth * dl * dtdy * Q2(bpcpamdq, m, i);
+                GH(hadd, m, 1, 1, i - 1) = GH(hadd, m, 1, 1, i - 1) - sixth * dl * dtdy * Q2(bmcpamdq, m, i);
+                GH(hadd, m, 2, -1, i - 1) = GH(hadd, m, 2, -1, i - 1) + sixth * dl * dtdy * Q2(bpcmamdq, m, i);
+                GH(hadd, m, 1, -1, i - 1) = GH(hadd, m, 1, -1, i - 1) + sixth * dl * dtdy * Q2(bmcmamdq, m, i);
+            }
+            if (m3 >= 2) {
+                GH(hadd, m, 2, 0, i) = GH(hadd, m, 2, 0, i) + dr * Q2(cpcqxxp, m, i);
+                GH(hadd, m, 1, 0, i) = GH(hadd, m, 1, 0, i) + dr * Q2(cmcqxxp, m, i);
+                GH(hadd, m, 2, 0, i - 1) = GH(hadd, m, 2, 0, i - 1) - dl * Q2(cpcqxxm, m, i);
+                GH(hadd, m, 1, 0, i - 1) = GH(hadd, m, 1, 0, i - 1) - dl * Q2(cmcqxxm, m, i);
+            }
+        }
+#undef RPT3
+    return cfl1d;
+}
+
+/* step3.f:2-594.  qnew == qold on entry; q(meqn, 1-mbc:mx+mbc, ...). */
+double oracle3d_step3(int rp_id, const double *rp_params, int meqn, int mwaves, int mbc, int mx, int my, int mz,
+                      const double *qold, double *qnew, double dx, double dy, double dz, double dt,
+                      const int *method, const int *mthlim)
+{
+    if (!known(rp_id) || method[5] > 0) return -1.0;
+    rp_ctx3 c;
+    c.rp_id = rp_id;
+    memcpy(c.p, rp_params, 8 * sizeof(double));
+    int maxm = mx > my ? mx : my;
+    if (mz > maxm) maxm = mz;
+    const int n1d = maxm + 2 * mbc;
+    const size_t nm = (size_t)n1d * meqn;
+    double *q1d = (double *)calloc(nm, sizeof(double)), *qadd = (double *)calloc(nm, sizeof(double));
+    double *fadd = (double *)calloc(nm, sizeof(double));
+    double *gadd = (double *)calloc(nm * 6, sizeof(double)), *hadd = (double *)calloc(nm * 6, sizeof(double));
+    double *wave = (double *)calloc(nm * mwaves, sizeof(double)), *s = (double *)calloc((size_t)n1d * mwaves, sizeof(double));
+    double *v[31];
+    for (int a = 0; a < 31; a++) v[a] = (double *)calloc(nm, sizeof(double));
+    const size_t NXs = mx + 2 * mbc, NYs = my + 2 * mbc;
+    const double dtd[3] = {dt / dx, dt / dy, dt / dz};
+    const int len[3] = {mx, my, mz};
+    double cfl = 0.0;
+    for (int d = 0; d < 3; d++) {
+        const int e = (d + 1) % 3, f = (d + 2) % 3; /* y-like, z-like directions of this sweep */
+        const int o1 = (d == 0) ? 1 : 0;            /* the two other directions: lower one is the inner loop */
+        const int o2 = (d == 2) ? 1 : 2;
+        const double dtde = dtd[e], dtdf = dtd[f];
+        int idx[3];
+        for (idx[o2] = 0; idx[o2] <= len[o2] + 1; idx[o2]++)
+            for (idx[o1] = 0; idx[o1] <= len[o1] + 1; idx[o1]++) {
+                for (int l = 1 - mbc; l <= len[d] + mbc; l++) {
+                    idx[d] = l;
+                    for (int m = 0; m < meqn; m++) Q2(q1d, m, l) = Q4(qold, m, idx[0], idx[1], idx[2]);
+                }
+                double cfl1d = flux3(&c, d + 1, meqn, mwaves, mbc, len[d], n1d, q1d, dtd[d], dtde, dtdf, method, mthlim,
+                                     wave, s, qadd, fadd, gadd, hadd, v);
+                cfl = dmax2(cfl, cfl1d);
+                /* step3.f:185-220 (x), 340-377 (y), 497-534 (z); (eo, fo) = offset in the y-like / z-like direction */
+                for (int l = 1; l <= len[d]; l++)
+                    for (int m = 0; m < meqn; m++) {
+                        int p[3];
+#define QN(eo, fo) (p[0] = idx[0], p[1] = idx[1], p[2] = idx[2], p[d] = l, p[e] += (eo), p[f] += (fo), &Q4(qnew, m, p[0], p[1], p[2]))
+                        double *t;
+                        t = QN(0, 0);
+                        *t = *t + Q2(qadd, m, l) - dtd[d] * (Q2(fadd, m, l + 1) - Q2(fadd, m, l))
+                             - dtde * (GH(gadd, m, 2, 0, l) - GH(gadd, m, 1, 0, l))
+                             - dtdf * (GH(hadd, m, 2, 0, l) - GH(hadd, m, 1, 0, l));
+                        t = QN(-1, 0);
+                        *t = *t - dtde * GH(gadd, m, 1, 0, l) - dtdf * (GH(hadd, m, 2, -1, l) - GH(hadd, m, 1, -1, l));
+                        t = QN(-1, -1);
+                        *t = *t - dtde * GH(gadd, m, 1, -1, l) - dtdf * GH(hadd, m, 1, -1, l);
+                        t = QN(0, -1);
+                        *t = *t - dtde * (GH(gadd, m, 2, -1, l) - GH(gadd, m, 1, -1, l)) - dtdf * GH(hadd, m, 1, 0, l);
+                        t = QN(1, -1);
+                        *t = *t + dtde * GH(gadd, m, 2, -1, l) - dtdf * GH(hadd, m, 1, 1, l);
+                        t = QN(1, 0);
+                        *t = *t + dtde * GH(gadd, m, 2, 0, l) - dtdf * (GH(hadd, m, 2, 1, l) - GH(hadd, m, 1, 1, l));
+                        t = QN(1, 1);
+                        *t = *t + dtde * GH(gadd, m, 2, 1, l) + dtdf * GH(hadd, m, 2, 1, l);
+                        t = QN(0, 1);
+                        *t = *t - dtde * (GH(gadd, m, 2, 1, l) - GH(gadd, m, 1, 1, l)) + dtdf * GH(hadd, m, 2, 0, l);
+                        t = QN(-1, 1);
+                        *t = *t - dtde * GH(gadd, m, 1, 1, l) + dtdf * GH(hadd, m, 2, -1, l);
+#undef QN
+                    }
+            }
+    }
+    free(q1d); free(qadd); free(fadd); free(gadd); free(hadd); free(wave); free(s);
+    for (int a = 0; a < 31; a++) free(v[a]);
+    return cfl;
+}
+#undef Q4
+
+/* ------------------------------------------------------------------------- */
+/* Pointwise rpn3 / rpt3 (property tests): n interfaces ql | qr (structure of */
+/* arrays [m][n]), presented as a 3-cell slice left | right | right (mbc = 1,  */
+/* mx = 1, interface i = 1).  asdq == NULL: rpn3 into wave, s, amdq, apdq;     */
+/* otherwise rpt3 / rptt3 of asdq in direction icoor into bm, bp.              */
+/* ------------------------------------------------------------------------- */
+void oracle3d_rp_point(int rp_id, const double *rp_params, int ixyz, int meqn, int mwaves, long long n,
+                       const double *ql, const double *qr, double *wave_o, double *s_o, double *amdq_o,
+                       double *apdq_o, int icoor, const double *asdq_i, double *bm_o, double *bp_o)
+{
+    const int mbc = 1, mx = 1, nc = 3;
+    rp_ctx3 c;
+    c.rp_id = rp_id;
+    memcpy(c.p, rp_params, 8 * sizeof(double));
+    double *q = (double *)calloc((size_t)meqn * nc, sizeof(double));
+    double *wave = (double *)calloc((size_t)meqn * mwaves * nc, sizeof(double));
+    double *s = (double *)calloc((size_t)mwaves * nc, sizeof(double));
+    double *amdq = (double *)calloc((size_t)meqn * nc, sizeof(double));
+    double *apdq = (double *)calloc((size_t)meqn * nc, sizeof(double));
+    double *asdq = (double *)calloc((size_t)meqn * nc, sizeof(double));
+    double *bm = (double *)calloc((size_t)meqn * nc, sizeof(double));
+    double *bp = (double *)calloc((size_t)meqn * nc, sizeof(double));
+    for (long long k = 0; k < n; k++) {
+        for (int m = 0; m < meqn; m++) {
+            Q2(q, m, 0) = ql[m * n + k];
+            Q2(q, m, 1) = qr[m * n + k];
+            Q2(q, m, 2) = qr[m * n + k];
+        }
+        if (!asdq_i) {
+            rpn3(&c, ixyz, mbc, mx, q, q, wave, s, amdq, apdq);
+            for (int m = 0; m < meqn; m++) {
+                for (int mw = 0; mw < mwaves; mw++) wave_o[(m * mwaves + mw) * n + k] = WV(m, mw, 1);
+                amdq_o[m * n + k] = Q2(amdq, m, 1);
+                apdq_o[m * n + k] = Q2(apdq, m, 1);
+            }
+            for (int mw = 0; mw < mwaves; mw++) s_o[mw * n + k] = SP(mw, 1);
+        } else {
+            for (int m = 0; m < meqn; m++)
+                for (int i = 0; i <= 2; i++) Q2(asdq, m, i) = asdq_i[m * n + k];
+            rpt3(&c, ixyz, icoor, mbc, mx, q, asdq, bm, bp);
+            for (int m = 0; m < meqn; m++) {
+                bm_o[m * n + k] = Q2(bm, m, 1);
+                bp_o[m * n + k] = Q2(bp, m, 1);
+            }
+        }
+    }
+    free(q); free(wave); free(s); free(amdq); free(apdq); free(asdq); free(bm); free(bp);
+}

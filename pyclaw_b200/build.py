@@ -1,7 +1,7 @@
 """Builds the CUDA library in-tree with nvcc for sm_100a.
 
     python -m pyclaw_b200.build [--force] [-v] [--fma | --all]
-    python -m pyclaw_b200.build --user-rp my_rp.cuh [--name mine] [--fma]     (plugin seam, see below)
+    python -m pyclaw_b200.build --user-rp my_rp.cuh [--name mine] [--fma] [--ndims 3]   (plugin seam, see below)
 
 Two builds of the same sources:
   libclawb200.so      -fmad=false : strict IEEE, bit-for-bit agreement with the reference's
@@ -13,8 +13,9 @@ Two builds of the same sources:
 -lineinfo keeps the ncu source page usable.
 
 Riemann-solver plugin seam: `--user-rp header.cuh` compiles a user-supplied solver (a header with
-`template <int IXY> struct RpUser`, see examples/user_rp/rp_kpp.cuh) into
-libclawb200_user_<name>.so -- the reference does the same at link time with RP_SOURCE in each
+`template <int IXY> struct RpUser`, see examples/user_rp/rp_kpp.cuh, and/or the 3-D
+`template <int IXYZ> struct RpUser3`, see examples/user_rp/rp_acoustics3d_user.cuh, selected with
+`--ndims 3` or `--ndims 1,2,3`) into libclawb200_user_<name>.so -- the reference does the same at link time with RP_SOURCE in each
 application's Makefile (Makefile.rules:1-26).  pyclaw.riemann.from_header() builds and binds it.
 """
 import os
@@ -35,10 +36,12 @@ UNITS = {
     "sweep_misc.cu": _COMMON,
     "sweep_fused.cu": _COMMON + ["fused.cuh"],
     "step1.cu": _COMMON,
-    "step3.cu": _COMMON,
+    "step3.cu": _COMMON + ["step3.cuh"],          # 3-D steps (step3.cuh): vc-acoustics
+    "step3_euler.cu": _COMMON + ["step3.cuh"],    # ... 3-D Euler
+    "step3_misc.cu": _COMMON + ["step3.cuh"],     # ... 3-D advection
     "rp_point.cu": _COMMON,
     "sharpclaw.cu": _COMMON + ["sharpclaw.cuh"],
-    "sweep_user.cu": _COMMON + ["sharpclaw.cuh"],   # the user-supplied Riemann solver (a stub without one)
+    "sweep_user.cu": _COMMON + ["sharpclaw.cuh", "step3.cuh"],   # the user-supplied Riemann solver (a stub without one)
 }
 SOURCES = list(UNITS)
 HEADERS = sorted({h for hs in UNITS.values() for h in hs})
@@ -112,10 +115,22 @@ def user_lib_path(name, fma=False):
     return os.path.join(CSRC, "libclawb200_user_%s%s.so" % (name, "_fma" if fma else ""))
 
 
-def build_user(header, name=None, fma=False, force=False, verbose=False):
+def user_flags(ndims):
+    """The defines that tell csrc/sweep_user.cu which structs the header has: RpUser (1-D / 2-D)
+    unless `ndims` lacks 1 and 2, RpUser3 when it contains 3."""
+    flags = []
+    if 3 in ndims:
+        flags.append("-DCLAWB200_USER_RP3")
+    if not set(ndims) & {1, 2}:
+        flags.append("-DCLAWB200_USER_NO_RP")
+    return flags
+
+
+def build_user(header, name=None, fma=False, force=False, verbose=False, ndims=(1, 2)):
     """A variant of the library with a user-supplied Riemann solver (csrc/sweep_user.cu): the
-    header defines `template <int IXY> struct RpUser` with the interface of the solvers in
-    rp.cuh.  Only sweep_user.cu is compiled; every other object comes from the base build.
+    header defines `template <int IXY> struct RpUser` (ndims 1, 2) and / or `template <int IXYZ>
+    struct RpUser3` (ndims 3) with the interfaces of the solvers in rp.cuh.  Only sweep_user.cu is
+    compiled; every other object comes from the base build.
     Returns the path of libclawb200_user_<name>[_fma].so."""
     header = os.path.abspath(header)
     if not os.path.exists(header):
@@ -133,7 +148,7 @@ def build_user(header, name=None, fma=False, force=False, verbose=False):
     os.makedirs(objdir, exist_ok=True)
     obj = os.path.join(objdir, "sweep_user.o")
     cmd = [nvcc] + flags + (["-Xptxas", "-v"] if verbose else []) + \
-        ['-DCLAWB200_USER_RP_HEADER="%s"' % header, "-c", "-o", obj, "sweep_user.cu"]
+        ['-DCLAWB200_USER_RP_HEADER="%s"' % header] + user_flags(ndims) + ["-c", "-o", obj, "sweep_user.cu"]
     subprocess.check_call(cmd, cwd=CSRC)
     base = os.path.join(CSRC, "_obj", "fma" if fma else "strict")
     objs = [obj] + [os.path.join(base, s[:-3] + ".o") for s in SOURCES if s != "sweep_user.cu"]
@@ -156,7 +171,9 @@ if __name__ == "__main__":
     if "--user-rp" in sys.argv:
         hdr = sys.argv[sys.argv.index("--user-rp") + 1]
         nm = sys.argv[sys.argv.index("--name") + 1] if "--name" in sys.argv else None
-        print(build_user(hdr, nm, fma="--fma" in sys.argv, force="--force" in sys.argv, verbose="-v" in sys.argv))
+        nd = tuple(int(d) for d in sys.argv[sys.argv.index("--ndims") + 1].split(",")) if "--ndims" in sys.argv else (1, 2)
+        print(build_user(hdr, nm, fma="--fma" in sys.argv, force="--force" in sys.argv, verbose="-v" in sys.argv,
+                         ndims=nd))
     elif "--all" in sys.argv:
         print(*build_all(force="--force" in sys.argv))
     else:

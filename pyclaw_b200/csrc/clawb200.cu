@@ -203,23 +203,54 @@ extern "C" int clawb200_step2ds(const clawb200_problem *p, const double *q_in, d
 }
 
 // ---------------------------------------------------------------------------
-// 3-D, dimensional splitting (step3ds.f:2-376; clawpack.py:656-676).  A 3-D field is
-// q[m][k][j][i]; every sweep is a set of independent 1-D problems, so the 2-D engines do the
-// work on 2-D views of the array: x- and y-sweeps plane by plane (k = 0..mz+1), z-sweeps on
-// the (i, k) slices j = 0..my+1 (row stride = one plane).  The arithmetic of flux3.f with
-// method(3) < 0 is that of flux2.f (the 0.5 of the correction flux is applied per term
-// instead of to the sum, an exact scaling).
+// 3-D, dimensional splitting (step3ds.f:2-376; clawpack.py:656-676) and the unsplit step.  A 3-D
+// field is q[m][k][j][i].  Both run the kernels of step3.cuh for every 3-D solver; for vc-acoustics
+// CLAWB200_STEP3DS_PLANES=1 runs a split sweep on the 2-D engines instead, on 2-D views of the array:
+// x- and y-sweeps plane by plane (k = 0..mz+1), z-sweeps on the (i, k) slices j = 0..my+1 (row
+// stride = one plane).  The arithmetic of flux3.f with method(3) < 0 is that of flux2.f (the 0.5 of
+// the correction flux is applied per term instead of to the sum, an exact scaling).
 // ---------------------------------------------------------------------------
+// The Riemann solver of a 3-D step: the shape it is compiled for and the aux data it reads.
+static int check_rp3(const clawb200_problem *p, bool have_aux)
+{
+    int meqn = 0, mwaves = 0, maux = 0;
+    switch (p->rp_id) {
+    case CLAWB200_RP_ACOUSTICS3D_VC: meqn = 4; mwaves = 2; maux = 2; break;
+    case CLAWB200_RP_ADVECTION3D: meqn = 1; mwaves = 1; break;
+    case CLAWB200_RP_EULER3D: meqn = 5; mwaves = 3; break;
+    case CLAWB200_RP_USER: {
+        int rc = claw_user_shape(3, &meqn, &mwaves, &maux);
+        if (rc) return rc;
+    } break;
+    default: return fail(CLAWB200_ERR_UNSUPPORTED, "no 3-D version of this Riemann solver");
+    }
+    if (p->meqn != meqn || p->mwaves != mwaves) return fail(CLAWB200_ERR_INVALID, "meqn/mwaves do not match the Riemann solver");
+    if (maux > 0 && (p->maux < maux || !have_aux))
+        return fail(CLAWB200_ERR_INVALID, p->rp_id == CLAWB200_RP_ACOUSTICS3D_VC
+                                              ? "aux array required: {impedance, sound speed}"
+                                              : "aux array required: the Riemann solver reads more aux components than maux");
+    return 0;
+}
+
+// the 3-D steps (step3.cuh), one translation unit per solver: idir = 1, 2, 3 one split sweep, 0 unsplit
+static int step3_dispatch(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
+                          const double *aux, double dt, int idir, double *scratch, double *cfl_dev, cudaStream_t st)
+{
+    switch (p->rp_id) {
+    case CLAWB200_RP_ACOUSTICS3D_VC: return claw_step3_acoustics(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
+    case CLAWB200_RP_EULER3D: return claw_step3_euler(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
+    case CLAWB200_RP_ADVECTION3D: return claw_step3_advection(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
+    default: return claw_step3_user(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
+    }
+}
+
 extern "C" int clawb200_step3ds(const clawb200_problem *p, int mz, double dz, const double *q_in,
                                 double *q_out, const double *aux, double dt, int idir,
                                 double *cfl_dev, void *stream)
 {
     int rc = check_problem(p, 3);
     if (rc) return rc;
-    if (p->rp_id != CLAWB200_RP_ACOUSTICS3D_VC)
-        return fail(CLAWB200_ERR_UNSUPPORTED, "no 3-D version of this Riemann solver");
-    if (p->meqn != 4 || p->mwaves != 2) return fail(CLAWB200_ERR_INVALID, "meqn/mwaves do not match the Riemann solver");
-    if (p->maux < 2 || !aux) return fail(CLAWB200_ERR_INVALID, "aux array required: {impedance, sound speed}");
+    if ((rc = check_rp3(p, aux != nullptr))) return rc;
     if (p->method[5] > 0) return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for the 3-D sweeps");
     if (p->mbc < 2) return fail(CLAWB200_ERR_INVALID, "classic solvers need mbc >= 2");
     if (mz < 1 || !(dz > 0.0)) return fail(CLAWB200_ERR_INVALID, "mz, dz must be positive");
@@ -229,11 +260,13 @@ extern "C" int clawb200_step3ds(const clawb200_problem *p, int mz, double dz, co
     const long long plane = (long long)nx * ny;
     if (p->mstride < plane * nz) return fail(CLAWB200_ERR_INVALID, "mstride smaller than the padded field");
     cudaStream_t st = (cudaStream_t)stream;
-    // One launch over the whole padded field (step3.cu): swept cells are updated, all others copied.
+    // One launch over the whole padded field (step3.cuh): swept cells are updated, all others copied.
     // CLAWB200_STEP3DS_PLANES=1 keeps round 1's composition from the 2-D engines (one launch per
     // plane after a copy of the field) for A/B measurements.
     static const bool planes = [] { const char *e = getenv("CLAWB200_STEP3DS_PLANES"); return e && atoi(e) != 0; }();
-    if (!planes) return claw_step3ds(p, mz, dz, q_in, q_out, aux, dt, idir, cfl_dev, st);
+    if (!planes) return step3_dispatch(p, mz, dz, q_in, q_out, aux, dt, idir, nullptr, cfl_dev, st);
+    if (p->rp_id != CLAWB200_RP_ACOUSTICS3D_VC)
+        return fail(CLAWB200_ERR_UNSUPPORTED, "CLAWB200_STEP3DS_PLANES is compiled for the vc-acoustics solver only");
     // step3ds.f: "qold and qnew are identical on entry"; cells the sweep does not touch keep qold
     CUDA_OK(cudaMemcpyAsync(q_out, q_in, sizeof(double) * (size_t)p->meqn * p->mstride,
                             cudaMemcpyDeviceToDevice, st));
@@ -278,10 +311,7 @@ static int check_step3(const clawb200_problem *p, int mz, double dz, const doubl
 {
     int rc = check_problem(p, 3);
     if (rc) return rc;
-    if (p->rp_id != CLAWB200_RP_ACOUSTICS3D_VC)
-        return fail(CLAWB200_ERR_UNSUPPORTED, "no 3-D version of this Riemann solver");
-    if (p->meqn != 4 || p->mwaves != 2) return fail(CLAWB200_ERR_INVALID, "meqn/mwaves do not match the Riemann solver");
-    if (p->maux < 2 || !aux) return fail(CLAWB200_ERR_INVALID, "aux array required: {impedance, sound speed}");
+    if ((rc = check_rp3(p, aux != nullptr))) return rc;
     if (p->method[5] > 0) return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for the 3-D sweeps");
     if (p->mbc < 2) return fail(CLAWB200_ERR_INVALID, "classic solvers need mbc >= 2");
     if (mz < 1 || !(dz > 0.0)) return fail(CLAWB200_ERR_INVALID, "mz, dz must be positive");
@@ -299,7 +329,7 @@ static int check_step3(const clawb200_problem *p, int mz, double dz, const doubl
 extern "C" long long clawb200_step3_scratch_doubles(const clawb200_problem *p)
 {
     if (!p) return fail(CLAWB200_ERR_INVALID, "null problem");
-    return claw_step3_scratch_doubles(p->mstride);
+    return claw_step3_scratch_doubles(p->meqn, p->mstride);
 }
 
 extern "C" int clawb200_step3(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
@@ -309,7 +339,7 @@ extern "C" int clawb200_step3(const clawb200_problem *p, int mz, double dz, cons
     if (rc) return rc;
     if (!qold || !qnew || !scratch) return fail(CLAWB200_ERR_INVALID, "null argument");
     if (qold == qnew) return fail(CLAWB200_ERR_INVALID, "qold and qnew must differ");
-    return claw_step3(p, mz, dz, qold, qnew, aux, dt, scratch, cfl_dev, (cudaStream_t)stream);
+    return step3_dispatch(p, mz, dz, qold, qnew, aux, dt, 0, scratch, cfl_dev, (cudaStream_t)stream);
 }
 
 __global__ void bc_kernel(double *q, long long mstride, int pitch, int narr, int nx, int ny,
@@ -1048,7 +1078,11 @@ static int check_rp_point(const clawb200_problem *p, int ixy, long long n)
     if (!p) return fail(CLAWB200_ERR_INVALID, "null problem");
     if (n < 0) return fail(CLAWB200_ERR_INVALID, "negative n");
     if (p->ndim == 2 && ixy != 1 && ixy != 2) return fail(CLAWB200_ERR_INVALID, "ixy must be 1 or 2");
-    if (p->ndim != 1 && p->ndim != 2) return fail(CLAWB200_ERR_UNSUPPORTED, "pointwise entry: 1-D and 2-D solvers");
+    if (p->ndim == 3) {
+        if (ixy < 1 || ixy > 3) return fail(CLAWB200_ERR_INVALID, "ixy must be 1, 2 or 3");
+        return check_rp3(p, true); // rp_point.cu checks auxl / auxr
+    }
+    if (p->ndim != 1 && p->ndim != 2) return fail(CLAWB200_ERR_UNSUPPORTED, "pointwise entry: 1-D, 2-D and 3-D solvers");
     return check_rp_shape(p);
 }
 
@@ -1160,7 +1194,7 @@ extern "C" int clawb200_step3_host(const clawb200_problem *p, int mz, double dz,
     const double *d_aux;
     if ((rc = host_upload_aux(P, aux, &d_aux))) return rc;
     double *scratch = nullptr;
-    CUDA_OK(cudaMalloc(&scratch, sizeof(double) * (size_t)claw_step3_scratch_doubles(P.mstride)));
+    CUDA_OK(cudaMalloc(&scratch, sizeof(double) * (size_t)claw_step3_scratch_doubles(P.meqn, P.mstride)));
     if (!(rc = clawb200_cfl_reset(g_hs.d_cfl, g_hs.st)))
         rc = clawb200_step3(&P, mz, dz, g_hs.d_a, g_hs.d_b, d_aux, dt, scratch, g_hs.d_cfl, g_hs.st);
     if (!rc) rc = host_download(P, g_hs.d_b, qnew);

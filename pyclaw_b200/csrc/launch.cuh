@@ -5,7 +5,7 @@
 // parallel): clawb200.cu (C ABI, boundary fills, layout / halo kernels, host entry points),
 // sweep_euler_x.cu / sweep_euler_y.cu, sweep_sphere.cu, sweep_misc.cu (instantiations of the
 // classic sweeps per Riemann-solver family), sweep_user.cu (the user-supplied solver), step1.cu,
-// rp_point.cu, sharpclaw.cu.
+// step3.cu / step3_euler.cu / step3_misc.cu (the 3-D steps), rp_point.cu, sharpclaw.cu.
 #pragma once
 #include <cuda_runtime.h>
 #include <cstdio>
@@ -121,15 +121,20 @@ int claw_y_ac3d(int idir, const SweepArgs &A, cudaStream_t st); // 3-D acoustics
 // single-pass unsplit step (sweep_fused.cu): solvers without aux / capa whose windows fit in registers
 bool claw_fused_available(int rp_id, const SweepArgs &A);
 int claw_fused(int rp_id, const SweepArgs &A, cudaStream_t st);
-// 3-D steps (step3.cu): one dimensionally split sweep in one launch; the unsplit step
-int claw_step3ds(const clawb200_problem *p, int mz, double dz, const double *q_in, double *q_out,
-                 const double *aux, double dt, int idir, double *cfl_dev, cudaStream_t st);
-long long claw_step3_scratch_doubles(long long mstride);
-int claw_step3(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
-               const double *aux, double dt, double *scratch, double *cfl_dev, cudaStream_t st);
+// 3-D steps (step3.cuh), one translation unit per solver family (step3.cu, step3_euler.cu,
+// step3_misc.cu, sweep_user.cu): idir = 1, 2, 3 one dimensionally split sweep, idir = 0 the unsplit step
+long long claw_step3_scratch_doubles(int meqn, long long mstride);
+int claw_step3_acoustics(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
+                         const double *aux, double dt, int idir, double *scratch, double *cfl_dev, cudaStream_t st);
+int claw_step3_euler(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
+                     const double *aux, double dt, int idir, double *scratch, double *cfl_dev, cudaStream_t st);
+int claw_step3_advection(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
+                         const double *aux, double dt, int idir, double *scratch, double *cfl_dev, cudaStream_t st);
+int claw_step3_user(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
+                    const double *aux, double dt, int idir, double *scratch, double *cfl_dev, cudaStream_t st);
 // the user-supplied solver (sweep_user.cu), id CLAWB200_RP_USER
 struct ScArgs;
-int claw_user_shape(int ndim, int *meqn, int *mwaves, int *maux);
+int claw_user_shape(int ndim, int *meqn, int *mwaves, int *maux); // ndim = 3: RpUser3
 int claw_x_user(bool trans, const SweepArgs &A, cudaStream_t st);
 int claw_y_user(bool trans, const SweepArgs &A, cudaStream_t st);
 int claw_step1_user(const SweepArgs &A, int mx, cudaStream_t st);

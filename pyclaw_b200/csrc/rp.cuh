@@ -35,6 +35,8 @@
 #define CLAW_RP_ADVECTION_COLOR 11
 #define CLAW_RP_VC_ADVECTION 12
 #define CLAW_RP_EULER1D 13
+#define CLAW_RP_ADVECTION3D 14
+#define CLAW_RP_EULER3D 15
 #define CLAW_RP_USER 100 // a solver compiled in from a user header (sweep_user.cu)
 
 // Solvers that return f-waves (jumps in the flux) instead of waves: the sweeps then use the
@@ -1032,8 +1034,9 @@ struct RpElasticFwave {
 // ---------------------------------------------------------------------------
 // 3-D acoustics in a heterogeneous medium.  clawpack/riemann rpn3_vc_acoustics.f (external;
 // test/acoustics/3d).  q = (p, u, v, w); aux = {impedance Z, sound speed c} of each cell.
-// IXYZ = 1, 2, 3 is the sweep direction.  Normal solve only: the 3-D path here is the
-// dimensionally split one (step3ds.f), which never calls rpt3 / rptt3.
+// IXYZ = 1, 2, 3 is the sweep direction.  The 3-D interface (transverse<ICOOR> = rpt3,
+// double_transverse<ICOOR> = rptt3) is defined below with the other 3-D solvers; the 2-D
+// `transverse` is the one the 2-D engines compile (CLAWB200_STEP3DS_PLANES: split sweeps only).
 // ---------------------------------------------------------------------------
 template <int IXYZ>
 struct RpAcoustics3D {
@@ -1081,6 +1084,30 @@ struct RpAcoustics3D {
     {
 #pragma unroll
         for (int m = 0; m < 4; m++) { bm[m] = 0.0; bp[m] = 0.0; }
+    }
+
+    // rpt3 / rptt3_vc_acoustics: asdq split along the line of three cells through (e0, f0) of the
+    // transverse aux neighbourhood in direction ICOOR (velocity component rp3_dir(IXYZ, ICOOR))
+    template <int ICOOR, class AR, class AX>
+    __device__ __forceinline__ static void split(AR &ar, const AX &aux, int e0, int f0, const double (&asdq)[4],
+                                                 double (&bm)[4], double (&bp)[4]);
+    template <int ICOOR, class AR, class AX>
+    __device__ __forceinline__ static void transverse(AR &ar, const RpParams &, const double (&)[NROE],
+                                                      const double (&)[4], const double (&)[4], const AX &aux, int,
+                                                      const double (&asdq)[4], double (&bm)[4], double (&bp)[4])
+    {
+        split<ICOOR>(ar, aux, 0, 0, asdq, bm, bp);
+    }
+    // the material of the plane (ICOOR = 2) or row (ICOOR = 3) the first split moved into
+    template <int ICOOR, class AR, class AX>
+    __device__ __forceinline__ static void double_transverse(AR &ar, const RpParams &, const double (&)[NROE],
+                                                             const double (&)[4], const double (&)[4], const AX &aux,
+                                                             int, int impt, const double (&bsasdq)[4], double (&cm)[4],
+                                                             double (&cp)[4])
+    {
+        const int off = (impt == 1) ? -1 : 1;
+        if (ICOOR == 2) split<ICOOR>(ar, aux, 0, off, bsasdq, cm, cp);
+        else split<ICOOR>(ar, aux, off, 0, bsasdq, cm, cp);
     }
 };
 
@@ -1303,5 +1330,239 @@ struct RpEuler1D {
     {
 #pragma unroll
         for (int m = 0; m < 3; m++) { bm[m] = 0.0; bp[m] = 0.0; }
+    }
+};
+
+
+// ===========================================================================
+// 3-D solvers of the unsplit and dimensionally split 3-D steps (step3.cuh).  One struct per sweep
+// direction IXYZ = 1, 2, 3 with the three routines of clawpack/riemann's 3-D interface:
+//
+//   solve(ar, P, l, r, axl, axr, wave, s, amdq, apdq, roe)            rpn3 at one interface (the
+//       signature of the 2-D solve above; roe[] carries what rpt3 / rptt3 need of the interface)
+//   transverse<ICOOR>(ar, P, roe, ql, qr, aux, imp, asdq, bm, bp)     rpt3: asdq split in the
+//       y-like (ICOOR = 2) or z-like (ICOOR = 3) direction of the sweep into its down- / up-going
+//       parts; imp = 1 for amdq (it enters the cell left of the interface), 2 for apdq
+//   double_transverse<ICOOR>(ar, P, roe, ql, qr, aux, imp, impt, bsasdq, cm, cp)   rptt3: a
+//       fluctuation already split in the OTHER transverse direction (impt = 1 / 2: its down- /
+//       up-going part) split again in direction ICOOR
+//
+// ql / qr are the states left and right of the interface.  `aux` holds the aux data of the 3x3
+// cells around the cell the fluctuation enters, in the plane normal to the sweep: aux(ma, e, f),
+// e / f = -1..1 the offset in the y-like / z-like direction (flux3.f's aux1 / aux2 / aux3 slices:
+// auxN <-> e = N - 2, their third index k <-> f = k - 2).  "y-like" is direction IXYZ % 3 + 1,
+// "z-like" the remaining one.
+// ===========================================================================
+template <int MAUX>
+struct AuxNbhd {
+    double v[MAUX > 0 ? MAUX : 1][3][3];
+    __device__ __forceinline__ double operator()(int ma, int e, int f) const { return v[ma][e + 1][f + 1]; }
+};
+
+// velocity component (1, 2, 3) of the direction ICOOR (1 = the sweep, 2 = y-like, 3 = z-like)
+__host__ __device__ constexpr int rp3_dir(int ixyz, int icoor) { return (ixyz - 1 + icoor - 1) % 3 + 1; }
+
+template <int IXYZ>
+template <int ICOOR, class AR, class AX>
+__device__ __forceinline__ void RpAcoustics3D<IXYZ>::split(AR &ar, const AX &aux, int e0, int f0, const double (&asdq)[4],
+                                                          double (&bm)[4], double (&bp)[4])
+{
+    constexpr int IU = rp3_dir(IXYZ, ICOOR);
+    constexpr int de = (ICOOR == 2) ? 1 : 0, df = (ICOOR == 3) ? 1 : 0;
+    const double zm = aux(0, e0 - de, f0 - df), zz = aux(0, e0, f0), zp = aux(0, e0 + de, f0 + df);
+    const double cm = aux(1, e0 - de, f0 - df), cp = aux(1, e0 + de, f0 + df);
+    const double a1 = ar.div(-asdq[0] + asdq[IU] * zz, zm + zz);
+    const double a2 = ar.div(asdq[0] + asdq[IU] * zz, zz + zp);
+#pragma unroll
+    for (int m = 0; m < 4; m++) { bm[m] = 0.0; bp[m] = 0.0; }
+    bm[0] = cm * a1 * zm;
+    bp[0] = cp * a2 * zp;
+    bm[IU] = -cm * a1;
+    bp[IU] = cp * a2;
+}
+
+// 3-D constant-coefficient advection q_t + u q_x + v q_y + w q_z = 0 (rpn3 / rpt3 /
+// rptt3_advection, clawpack/riemann; external, restated): params {u, v, w}.
+template <int IXYZ>
+struct RpAdvection3 {
+    static constexpr int ID = CLAW_RP_ADVECTION3D;
+    static constexpr int MEQN = 1, MWAVES = 1, NROE = 1, MAUX = 0;
+
+    template <class AR>
+    __device__ __forceinline__ static void solve(AR &, const RpParams &P, const double (&l)[1], const double (&r)[1],
+                                                 const AuxCell &, const AuxCell &, double (&wave)[1][1],
+                                                 double (&s)[1], double (&amdq)[1], double (&apdq)[1],
+                                                 double (&roe)[NROE])
+    {
+        wave[0][0] = r[0] - l[0];
+        s[0] = P.p[IXYZ - 1];
+        amdq[0] = dmin2(s[0], 0.0) * wave[0][0];
+        apdq[0] = dmax2(s[0], 0.0) * wave[0][0];
+        roe[0] = 0.0;
+    }
+    template <int ICOOR, class AR>
+    __device__ __forceinline__ static void transverse(AR &, const RpParams &P, const double (&)[NROE],
+                                                      const double (&)[1], const double (&)[1], const AuxNbhd<MAUX> &,
+                                                      int, const double (&asdq)[1], double (&bm)[1], double (&bp)[1])
+    {
+        const double st = P.p[rp3_dir(IXYZ, ICOOR) - 1];
+        bm[0] = dmin2(st, 0.0) * asdq[0];
+        bp[0] = dmax2(st, 0.0) * asdq[0];
+    }
+    template <int ICOOR, class AR>
+    __device__ __forceinline__ static void double_transverse(AR &ar, const RpParams &P, const double (&roe)[NROE],
+                                                             const double (&ql)[1], const double (&qr)[1],
+                                                             const AuxNbhd<MAUX> &aux, int imp, int,
+                                                             const double (&bsasdq)[1], double (&cm)[1], double (&cp)[1])
+    {
+        transverse<ICOOR>(ar, P, roe, ql, qr, aux, imp, bsasdq, cm, cp);
+    }
+};
+
+// 3-D Euler equations, Roe solver with the Harten-Hyman entropy fix (rpn3 / rpt3 / rptt3_euler,
+// clawpack/riemann; external, restated from the published algorithm, LeVeque 2002 sec. 15.3 and
+// 18.8).  q = (rho, rho u, rho v, rho w, E); params {gamma, gamma1}.  Three waves: u - c, u (the
+// entropy jump and both shear jumps), u + c.  With v = w = 0 the normal solve performs the
+// operations of RpEuler1D (rp1_euler_with_efix) on the same values.
+// roe[] = {u, v, w, enth, a, u^2 + v^2 + w^2} of the interface.
+template <class AR>
+__device__ __forceinline__ void euler3_roe(AR &ar, double gamma1, const double (&l)[5], const double (&r)[5],
+                                           double (&roe)[6])
+{
+    const double rhsqrtl = ar.sqrt(l[0]), rhsqrtr = ar.sqrt(r[0]);
+    const Recip rrl = ar.rcp(l[0]), rrr = ar.rcp(r[0]);
+    const double pl = gamma1 * (l[4] - ar.div(0.5 * (l[1] * l[1] + l[2] * l[2] + l[3] * l[3]), rrl));
+    const double pr = gamma1 * (r[4] - ar.div(0.5 * (r[1] * r[1] + r[2] * r[2] + r[3] * r[3]), rrr));
+    const double rhsq2 = rhsqrtl + rhsqrtr;
+    const Recip rsl = ar.rcp(rhsqrtl), rsr = ar.rcp(rhsqrtr), rs2 = ar.rcp(rhsq2);
+#pragma unroll
+    for (int k = 0; k < 3; k++) roe[k] = ar.div(ar.div(l[1 + k], rsl) + ar.div(r[1 + k], rsr), rs2);
+    const double enth = ar.div((ar.div(l[4] + pl, rsl) + ar.div(r[4] + pr, rsr)), rs2);
+    const double uvw2 = roe[0] * roe[0] + roe[1] * roe[1] + roe[2] * roe[2];
+    roe[3] = enth;
+    roe[4] = ar.sqrt(gamma1 * (enth - 0.5 * uvw2));
+    roe[5] = uvw2;
+}
+
+// d (a jump or a fluctuation) split into the eigenvectors of the Roe matrix of direction MT
+// (velocity component 1, 2, 3): wave 0 at un - a, wave 1 at un, wave 2 at un + a
+template <int MT, class AR>
+__device__ __forceinline__ void euler3_waves(AR &ar, double gamma1, const double (&roe)[6], const double (&d)[5],
+                                             double (&wave)[5][3], double (&s)[3])
+{
+    constexpr int M1 = MT % 3 + 1, M2 = (MT + 1) % 3 + 1; // the two momenta across direction MT
+    const double un = roe[MT - 1], u1 = roe[M1 - 1], u2 = roe[M2 - 1];
+    const double enth = roe[3], a = roe[4], uvw2 = roe[5];
+    const double a3 = ar.div(gamma1, a * a) *
+                      ((enth - uvw2) * d[0] + roe[0] * d[1] + roe[1] * d[2] + roe[2] * d[3] - d[4]);
+    const double b1 = d[M1] - u1 * d[0], b2 = d[M2] - u2 * d[0];
+    const double a5 = ar.div(d[MT] + (a - un) * d[0] - a * a3, 2.0 * a);
+    const double a1 = d[0] - a3 - a5;
+    wave[0][0] = a1; wave[MT][0] = a1 * (un - a); wave[M1][0] = a1 * u1; wave[M2][0] = a1 * u2;
+    wave[4][0] = a1 * (enth - un * a); s[0] = un - a;
+    wave[0][1] = a3; wave[MT][1] = a3 * un; wave[M1][1] = a3 * u1 + b1; wave[M2][1] = a3 * u2 + b2;
+    wave[4][1] = a3 * 0.5 * uvw2 + b1 * u1 + b2 * u2; s[1] = un;
+    wave[0][2] = a5; wave[MT][2] = a5 * (un + a); wave[M1][2] = a5 * u1; wave[M2][2] = a5 * u2;
+    wave[4][2] = a5 * (enth + un * a); s[2] = un + a;
+}
+
+template <int IXYZ>
+struct RpEuler3 {
+    static constexpr int ID = CLAW_RP_EULER3D;
+    static constexpr int MEQN = 5, MWAVES = 3, NROE = 6, MAUX = 0;
+    static constexpr int MU = IXYZ;
+
+    template <class AR>
+    __device__ __forceinline__ static void solve(AR &ar, const RpParams &P, const double (&l)[5], const double (&r)[5],
+                                                 const AuxCell &, const AuxCell &, double (&wave)[5][3],
+                                                 double (&s)[3], double (&amdq)[5], double (&apdq)[5],
+                                                 double (&roe)[NROE])
+    {
+        const double gamma1 = P.p[1];
+        euler3_roe(ar, gamma1, l, r, roe);
+        double d[5];
+#pragma unroll
+        for (int m = 0; m < 5; m++) d[m] = r[m] - l[m];
+        euler3_waves<MU>(ar, gamma1, roe, d, wave, s);
+        // Harten-Hyman entropy fix on the acoustic waves, left-going fluctuation first
+        const Recip rrl = ar.rcp(l[0]), rrr = ar.rcp(r[0]);
+        bool done = false;
+        const double ulx = ar.div(l[1], rrl), uly = ar.div(l[2], rrl), ulz = ar.div(l[3], rrl);
+        const double cl = ar.sqrt(gamma1 * (gamma1 + 1.0) * (ar.div(l[4], rrl) - 0.5 * (ulx * ulx + uly * uly + ulz * ulz)));
+        const double s0 = ar.div(l[MU], rrl) - cl;
+        if (s0 >= 0.0 && s[0] > 0.0) {
+#pragma unroll
+            for (int m = 0; m < 5; m++) amdq[m] = 0.0;
+            done = true;
+        }
+        if (!done) {
+            double q1[5];
+#pragma unroll
+            for (int m = 0; m < 5; m++) q1[m] = l[m] + wave[m][0];
+            const Recip r1 = ar.rcp(q1[0]);
+            const double p1 = gamma1 * (q1[4] - ar.div(0.5 * (q1[1] * q1[1] + q1[2] * q1[2] + q1[3] * q1[3]), r1));
+            const double c1 = ar.sqrt(ar.div((gamma1 + 1.0) * p1, r1));
+            const double s1 = ar.div(q1[MU], r1) - c1;
+            double sfract;
+            if (s0 < 0.0 && s1 > 0.0) sfract = ar.div(s0 * (s1 - s[0]), s1 - s0);
+            else if (s[0] < 0.0) sfract = s[0];
+            else sfract = 0.0;
+#pragma unroll
+            for (int m = 0; m < 5; m++) amdq[m] = sfract * wave[m][0];
+            if (s[1] >= 0.0) done = true;
+        }
+        if (!done) {
+#pragma unroll
+            for (int m = 0; m < 5; m++) amdq[m] = amdq[m] + s[1] * wave[m][1];
+            const double urx = ar.div(r[1], rrr), ury = ar.div(r[2], rrr), urz = ar.div(r[3], rrr);
+            const double cr = ar.sqrt(gamma1 * (gamma1 + 1.0) * (ar.div(r[4], rrr) - 0.5 * (urx * urx + ury * ury + urz * urz)));
+            const double s3 = ar.div(r[MU], rrr) + cr;
+            double q2[5];
+#pragma unroll
+            for (int m = 0; m < 5; m++) q2[m] = r[m] - wave[m][2];
+            const Recip r2 = ar.rcp(q2[0]);
+            const double p2 = gamma1 * (q2[4] - ar.div(0.5 * (q2[1] * q2[1] + q2[2] * q2[2] + q2[3] * q2[3]), r2));
+            const double c2 = ar.sqrt(ar.div((gamma1 + 1.0) * p2, r2));
+            const double s2 = ar.div(q2[MU], r2) + c2;
+            double sfract = 0.0;
+            bool add = true;
+            if (s2 < 0.0 && s3 > 0.0) sfract = ar.div(s2 * (s3 - s[2]), s3 - s2);
+            else if (s[2] < 0.0) sfract = s[2];
+            else add = false;
+            if (add) {
+#pragma unroll
+                for (int m = 0; m < 5; m++) amdq[m] = amdq[m] + sfract * wave[m][2];
+            }
+        }
+#pragma unroll
+        for (int m = 0; m < 5; m++) {
+            double df = 0.0;
+#pragma unroll
+            for (int mw = 0; mw < 3; mw++) df = df + s[mw] * wave[m][mw];
+            apdq[m] = df - amdq[m];
+        }
+    }
+    // rpt3 / rptt3: asdq split with the eigenvectors of the Roe matrix of direction ICOOR at the
+    // interface's Roe averages (no aux data: both routines are the same split)
+    template <int ICOOR, class AR>
+    __device__ __forceinline__ static void transverse(AR &ar, const RpParams &P, const double (&roe)[NROE],
+                                                      const double (&)[5], const double (&)[5], const AuxNbhd<MAUX> &,
+                                                      int, const double (&asdq)[5], double (&bm)[5], double (&bp)[5])
+    {
+        double wave[5][3], s[3];
+        euler3_waves<rp3_dir(IXYZ, ICOOR)>(ar, P.p[1], roe, asdq, wave, s);
+#pragma unroll
+        for (int m = 0; m < 5; m++) {
+            bm[m] = dmin2(s[0], 0.0) * wave[m][0] + dmin2(s[1], 0.0) * wave[m][1] + dmin2(s[2], 0.0) * wave[m][2];
+            bp[m] = dmax2(s[0], 0.0) * wave[m][0] + dmax2(s[1], 0.0) * wave[m][1] + dmax2(s[2], 0.0) * wave[m][2];
+        }
+    }
+    template <int ICOOR, class AR>
+    __device__ __forceinline__ static void double_transverse(AR &ar, const RpParams &P, const double (&roe)[NROE],
+                                                             const double (&ql)[5], const double (&qr)[5],
+                                                             const AuxNbhd<MAUX> &aux, int imp, int,
+                                                             const double (&bsasdq)[5], double (&cm)[5], double (&cp)[5])
+    {
+        transverse<ICOOR>(ar, P, roe, ql, qr, aux, imp, bsasdq, cm, cp);
     }
 };

@@ -11,7 +11,8 @@
 // Layout: structure of arrays, ql[m][n], wave[(m * mwaves + mw)][n], s[mw][n].
 #include "launch.cuh"
 
-template <class RP>
+// TRANS = false: solvers without the 2-D transverse solve (the 3-D ones)
+template <class RP, bool TRANS>
 __global__ void rp_point_kernel(long long n, RpParams P, const double *__restrict__ ql,
                                 const double *__restrict__ qr, const double *__restrict__ auxl,
                                 const double *__restrict__ auxr, double *__restrict__ wave,
@@ -40,6 +41,7 @@ __global__ void rp_point_kernel(long long n, RpParams P, const double *__restric
 #pragma unroll
         for (int mw = 0; mw < MW; mw++) s[mw * n + i] = sp[mw];
     }
+    if constexpr (TRANS) {
     if (asdq) { // rpt2: split asdq with the Roe data of this interface (imp = 1: the cell on the left)
         double a[MEQN], b1[MEQN], b2[MEQN];
 #pragma unroll
@@ -48,9 +50,10 @@ __global__ void rp_point_kernel(long long n, RpParams P, const double *__restric
 #pragma unroll
         for (int m = 0; m < MEQN; m++) { bm[m * n + i] = b1[m]; bp[m * n + i] = b2[m]; }
     }
+    }
 }
 
-template <class RP>
+template <class RP, bool TRANS = true>
 static int rp_point_launch(long long n, const RpParams &P, const double *ql, const double *qr, const double *auxl,
                            const double *auxr, double *wave,
                            double *s, double *amdq, double *apdq, int imp, const double *asdq, double *bm,
@@ -59,13 +62,13 @@ static int rp_point_launch(long long n, const RpParams &P, const double *ql, con
     if (n <= 0) return 0;
     if (RP::MAUX > 0 && (!auxl || !auxr)) return fail(CLAWB200_ERR_INVALID, "this Riemann solver reads aux_l / aux_r");
     if (RP::MAUX > 0 && asdq) return fail(CLAWB200_ERR_UNSUPPORTED, "pointwise transverse solves: solvers without aux only");
-    rp_point_kernel<RP><<<(unsigned)((n + 127) / 128), 128, 0, st>>>(n, P, ql, qr, auxl, auxr, wave, s, amdq, apdq,
+    rp_point_kernel<RP, TRANS><<<(unsigned)((n + 127) / 128), 128, 0, st>>>(n, P, ql, qr, auxl, auxr, wave, s, amdq, apdq,
                                                                     imp, asdq, bm, bp);
     CUDA_OK(cudaGetLastError());
     return 0;
 }
 
-// ixy = 1 | 2 selects the sweep direction of a 2-D solver; auxl / auxr may be null for solvers without aux
+// ixy = 1 | 2 (| 3) selects the sweep direction of a 2-D (3-D) solver; auxl / auxr may be null for solvers without aux
 int claw_rp_point(const clawb200_problem *p, int ixy, long long n, const double *ql, const double *qr,
                   const double *auxl, const double *auxr, double *wave, double *s, double *amdq, double *apdq, int imp, const double *asdq,
                   double *bm, double *bp, cudaStream_t st)
@@ -75,6 +78,17 @@ int claw_rp_point(const clawb200_problem *p, int ixy, long long n, const double 
     RpParams P;
     for (int i = 0; i < 8; i++) P.p[i] = p->rp_params[i];
 #define GO(RPT) return rp_point_launch<RPT>(n, P, ql, qr, auxl, auxr, wave, s, amdq, apdq, imp, asdq, bm, bp, st)
+#define GO3(RPF) return ixy == 1 ? rp_point_launch<RPF<1>, false>(n, P, ql, qr, auxl, auxr, wave, s, amdq, apdq, 0, nullptr, nullptr, nullptr, st) \
+                   : ixy == 2 ? rp_point_launch<RPF<2>, false>(n, P, ql, qr, auxl, auxr, wave, s, amdq, apdq, 0, nullptr, nullptr, nullptr, st) \
+                              : rp_point_launch<RPF<3>, false>(n, P, ql, qr, auxl, auxr, wave, s, amdq, apdq, 0, nullptr, nullptr, nullptr, st)
+    if (p->ndim == 3) { // rpn3, ixy = 1, 2, 3 (the caller has rejected transverse solves)
+        switch (p->rp_id) {
+        case CLAWB200_RP_ACOUSTICS3D_VC: GO3(RpAcoustics3D);
+        case CLAWB200_RP_ADVECTION3D: GO3(RpAdvection3);
+        case CLAWB200_RP_EULER3D: GO3(RpEuler3);
+        default: return fail(CLAWB200_ERR_UNSUPPORTED, "pointwise entry: no 3-D version of this solver");
+        }
+    }
     if (p->ndim == 1) {
         if (asdq) return fail(CLAWB200_ERR_INVALID, "1-D solvers have no transverse solve");
         switch (p->rp_id) {
@@ -109,4 +123,5 @@ int claw_rp_point(const clawb200_problem *p, int ixy, long long n, const double 
     default: return fail(CLAWB200_ERR_UNSUPPORTED, "pointwise entry: not compiled for this solver");
     }
 #undef GO
+#undef GO3
 }

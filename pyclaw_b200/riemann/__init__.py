@@ -8,7 +8,7 @@ keys of ``state.aux_global`` (the cparam common block the script fills).
 """
 from .._lib import (RP_ACOUSTICS, RP_ADVECTION, RP_EULER5, RP_SHALLOW, RP_SPHERE, RP_NEL_FWAVE,
                     RP_PSYSTEM, RP_ACOUSTICS3D_VC, RP_VC_ACOUSTICS, RP_BURGERS, RP_ADVECTION_COLOR,
-                    RP_VC_ADVECTION, RP_EULER1D)
+                    RP_VC_ADVECTION, RP_EULER1D, RP_ADVECTION3D, RP_EULER3D)
 
 
 class RiemannSolver(object):
@@ -27,13 +27,13 @@ class RiemannSolver(object):
     def __call__(self, q_l, q_r, aux_l=None, aux_r=None, aux_global=None, ixy=1):
         """The reference's Python Riemann-solver contract (doc/rp.rst:7-62, clawpack.py:349):
         ``wave, s, amdq, apdq = rp(q_l, q_r, aux_l, aux_r, aux_global)`` on arrays of interfaces,
-        evaluated by the CUDA solver that the sweeps inline.  q_l, q_r: [meqn, n] CUDA tensors
+        evaluated by the CUDA solver that the sweeps inline (ixy = 1, 2, 3 for a 3-D solver).  q_l, q_r: [meqn, n] CUDA tensors
         (left / right state of each interface); returns CUDA tensors wave[meqn, mwaves, n],
         s[mwaves, n], amdq[meqn, n], apdq[meqn, n].  aux_l, aux_r: [maux, n] or None."""
         import ctypes
         import torch
         from .. import _lib
-        ndim = 2 if 2 in self.ndims else 1
+        ndim = 2 if 2 in self.ndims else (1 if 1 in self.ndims else 3)
         q_l = q_l.contiguous().to(torch.float64)
         q_r = q_r.contiguous().to(torch.float64)
         meqn, n = q_l.shape
@@ -62,7 +62,7 @@ class RiemannSolver(object):
         base = 'fma' if arithmetic == 'fma' else 'strict'
         if base not in self.lib:
             from ..build import build_user
-            self.lib[base] = build_user(self.header, self.name, fma=(base == 'fma'))
+            self.lib[base] = build_user(self.header, self.name, fma=(base == 'fma'), ndims=self.ndims)
         key = 'user:%s:%s' % (self.name, base)
         _lib.LIB_PATHS[key] = self.lib[base]
         return key
@@ -107,6 +107,9 @@ psystem = RiemannSolver("psystem", RP_PSYSTEM, 3, 2, [], (2,), fwave=True, maux=
 
 # 3-D acoustics in a heterogeneous medium (test/acoustics/3d): aux = {impedance, sound speed}
 vc_acoustics_3d = RiemannSolver("vc_acoustics_3d", RP_ACOUSTICS3D_VC, 4, 2, [], (3,), maux=2)
+# 3-D constant-coefficient advection and 3-D Euler (Roe + entropy fix; q = rho, rho u, rho v, rho w, E)
+advection_3d = RiemannSolver("advection_3d", RP_ADVECTION3D, 1, 1, ["u", "v", "w"], (3,))
+euler_3d = RiemannSolver("euler_3d", RP_EULER3D, 5, 3, ["gamma", "gamma1"], (3,))
 
 # further solvers of the reference's applications (set solver.rp to use them)
 vc_acoustics = RiemannSolver("vc_acoustics", RP_VC_ACOUSTICS, 3, 2, [], (2,), maux=2)          # aux {rho, c}
@@ -118,7 +121,9 @@ euler_with_efix = RiemannSolver("euler_with_efix", RP_EULER1D, 3, 3, ["gamma", "
 def from_header(header, name=None, meqn=1, mwaves=1, ndims=(2,), param_names=(), optional=(), defaults=None,
                 fwave=False, maux=0, build=True):
     """A user-supplied Riemann solver: ``header`` defines ``template <int IXY> struct RpUser`` with the
-    interface of the solvers in pyclaw_b200/csrc/rp.cuh (examples/user_rp/rp_kpp.cuh).  It is
+    interface of the solvers in pyclaw_b200/csrc/rp.cuh (examples/user_rp/rp_kpp.cuh) and, when
+    ``ndims`` contains 3, ``template <int IXYZ> struct RpUser3`` with the 3-D interface (rpn3 / rpt3 /
+    rptt3; examples/user_rp/rp_acoustics3d_user.cuh).  It is
     compiled into a variant of the library (pyclaw_b200.build.build_user; nvcc must be on PATH
     unless the variant was built before) and returned as a descriptor for ``solver.rp``.
 
@@ -137,7 +142,7 @@ def from_header(header, name=None, meqn=1, mwaves=1, ndims=(2,), param_names=(),
     rs.header = header
     rs.lib = {}
     if build:
-        rs.lib['strict'] = build_user(header, name)
+        rs.lib['strict'] = build_user(header, name, ndims=rs.ndims)
     elif os.path.exists(user_lib_path(name)):
         rs.lib['strict'] = user_lib_path(name)
     else:
@@ -146,7 +151,7 @@ def from_header(header, name=None, meqn=1, mwaves=1, ndims=(2,), param_names=(),
 
 
 _BY_NAME = {s.name: s for s in (vc_acoustics, burgers, advection_color, vc_advection, euler_with_efix,
-                                vc_acoustics_3d, acoustics, advection, euler_5wave, shallow_roe_with_efix, shallow_sphere,
+                                vc_acoustics_3d, advection_3d, euler_3d, acoustics, advection, euler_5wave, shallow_roe_with_efix, shallow_sphere,
                                 nonlinear_elasticity_fwave, psystem)}
 _BY_NAME.update({"euler": euler_5wave, "shallow": shallow_roe_with_efix})
 
