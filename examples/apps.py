@@ -381,15 +381,30 @@ def annulus(mx=40, my=120, petsc=False, tfinal=1.0, outdir=None):
     return _run(pyclaw, solver, state, tfinal, 10, outdir)
 
 
-def euler3d(mx=64, my=64, mz=64, petsc=False, tfinal=0.1, dim_split=True, outdir=None):
+def _solver3d(pyclaw, solver_type, dim_split):
+    """ClawSolver3D (dimensional splitting or the unsplit step), or SharpClawSolver3D (WENO5, SSP104).
+    SharpClaw's 3-D Courant number is the largest of the three directions, not their sum, so the
+    SharpClaw variant runs at cfl_desired = 0.8, cfl_max = 0.9: three directions at 0.8 add up to the
+    2.4 that SSP104 allows in one dimension."""
+    if solver_type == 'sharpclaw':
+        solver = pyclaw.SharpClawSolver3D()
+        solver.cfl_desired, solver.cfl_max = 0.8, 0.9
+        return solver
+    if solver_type != 'classic':
+        raise ValueError("solver_type must be 'classic' or 'sharpclaw'")
+    solver = pyclaw.ClawSolver3D()
+    solver.dim_split = dim_split
+    return solver
+
+
+def euler3d(mx=64, my=64, mz=64, petsc=False, tfinal=0.1, dim_split=True, outdir=None, solver_type='classic'):
     """3-D Euler equations (Roe solver with entropy fix, pyclaw.riemann.euler_3d): a spherical blast
     wave in the unit box with reflecting walls.  Gas at rest, rho = 1; pressure 10 inside the sphere
     of radius 0.2 around the centre, 0.1 outside.  dim_split=False runs the unsplit step with
-    transverse corrections (order_trans = 22)."""
+    transverse corrections (order_trans = 22); solver_type='sharpclaw' runs SharpClawSolver3D."""
     pyclaw = _pc(petsc)
-    solver = pyclaw.ClawSolver3D()
+    solver = _solver3d(pyclaw, solver_type, dim_split)
     solver.rp = pyclaw.riemann.euler_3d
-    solver.dim_split = dim_split
     solver.mwaves, solver.limiters = 3, pyclaw.limiters.tvd.MC
     for i in range(3):
         solver.bc_lower[i] = solver.bc_upper[i] = pyclaw.BC.reflecting
@@ -409,13 +424,13 @@ def euler3d(mx=64, my=64, mz=64, petsc=False, tfinal=0.1, dim_split=True, outdir
     return _run(pyclaw, solver, state, tfinal, 10, outdir)
 
 
-def advection3d(mx=32, my=32, mz=32, petsc=False, tfinal=1.0, dim_split=True, u=1.0, v=0.5, w=0.25, outdir=None):
+def advection3d(mx=32, my=32, mz=32, petsc=False, tfinal=1.0, dim_split=True, u=1.0, v=0.5, w=0.25, outdir=None,
+                solver_type='classic'):
     """3-D constant-coefficient advection (pyclaw.riemann.advection_3d) of a Gaussian in the
-    periodic unit box with velocity (u, v, w)."""
+    periodic unit box with velocity (u, v, w); solver_type='sharpclaw' runs SharpClawSolver3D."""
     pyclaw = _pc(petsc)
-    solver = pyclaw.ClawSolver3D()
+    solver = _solver3d(pyclaw, solver_type, dim_split)
     solver.rp = pyclaw.riemann.advection_3d
-    solver.dim_split = dim_split
     solver.mwaves, solver.limiters = 1, pyclaw.limiters.tvd.MC
     for i in range(3):
         solver.bc_lower[i] = solver.bc_upper[i] = pyclaw.BC.periodic

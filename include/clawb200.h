@@ -187,6 +187,17 @@ int clawb200_sharpclaw_stage(const clawb200_problem *p, const double *q, const d
                              double *out, double *dq_out, const double *aux, double dt,
                              int mode, double ca, double cb, double div, double *cfl_dev,
                              void *stream);
+/* The same stage in 3-D (p->ndim = 3; clawb200_sharpclaw_stage fails with CLAWB200_ERR_INVALID on
+ * a 3-D problem).  Field layout of clawb200_step3ds; p->rp_id any 3-D solver.  dq is flux1 summed
+ * over the x-, y- and z-slices of the grid (DESIGN.md §1): ((0 + dq_x) + dq_y) + dq_z per cell.  The
+ * x/y partial of dq is held in dq_out if given, otherwise in out: out, dq_out and qa must be three
+ * different buffers, none of them q; mode 3 needs dq_out.  CLAWB200_ERR_UNSUPPORTED for a capacity
+ * function (method[5] > 0), WENO orders above 5 (CLAWB200_WENO_TABLES) and the wave-based
+ * reconstructions. */
+int clawb200_sharpclaw_stage3(const clawb200_problem *p, int mz, double dz, const double *q,
+                              const double *qa, double *out, double *dq_out, const double *aux,
+                              double dt, int mode, double ca, double cb, double div,
+                              double *cfl_dev, void *stream);
 
 /* The stage-free combination in the middle of SSP104 (sharpclaw.py:195-196), fused:
  *     s2 = q/25. + (9./25)*s1 ;  s1 = 15.*s2 - 5.*s1
@@ -308,6 +319,10 @@ int clawb200_step2_host(const clawb200_problem *p, const double *qold, double *q
  * (dq, cfl) = sharpclaw2.flux2(q, auxbc, dt, t, mbc, maxm, mx, my)     (ndim = 2) */
 int clawb200_sharpclaw_dq_host(const clawb200_problem *p, const double *q, double *dq,
                                const double *aux, double dt, double *cfl);
+/* (dq, cfl) = flux3 of clawb200_sharpclaw_stage3 on host arrays q(meqn, mx+2mbc, my+2mbc, mz+2mbc)
+ * (Fortran order); dq is zero outside the interior.  The reference has no 3-D SharpClaw module. */
+int clawb200_sharpclaw_dq3_host(const clawb200_problem *p, int mz, double dz, const double *q,
+                                double *dq, const double *aux, double dt, double *cfl);
 
 /* (qnew, cfl) = classic3.step3ds(maxm, mbc, mx, my, mz, qold, qnew, auxbc, dx, dy, dz, dt, method,
  *                                mthlim, aux1, aux2, aux3, work, idir) */

@@ -1,6 +1,7 @@
-"""CPU restatement of the 3-D classic steps for the aux-free 3-D solvers -- TEST INFRASTRUCTURE ONLY
-(never imported by pyclaw_b200/).  ctypes driver of oracle3d/liboracle3d.so (claw_oracle3d.c), with
-the array conventions of oracle/pyclaw_oracle.py: Fortran-ordered q[m, i, j, k]."""
+"""CPU restatement of the 3-D classic steps for the aux-free 3-D solvers and of SharpClaw in 3-D (flux3,
+sc_flux3) -- TEST INFRASTRUCTURE ONLY (never imported by pyclaw_b200/).  ctypes driver of
+oracle3d/liboracle3d.so (claw_oracle3d.c), with the array conventions of oracle/pyclaw_oracle.py:
+Fortran-ordered q[m, i, j, k]."""
 import ctypes
 import os
 import subprocess
@@ -11,6 +12,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = None
 
 RP_ADVECTION3D, RP_EULER3D = 14, 15  # 3-D advection {u, v, w}; 3-D Euler, Roe + entropy fix {gamma, gamma1}
+RP_ACOUSTICS3D_VC = 8                # 3-D acoustics, aux = {impedance, sound speed} (SharpClaw only here)
+WENO_PYWENO_F32, WENO_PYWENO_F64, WENO_OLD, RECON_TVD2 = 0, 1, 2, 4  # as oracle/pyclaw_oracle.py
 
 _dp = ctypes.POINTER(ctypes.c_double)
 _ip = ctypes.POINTER(ctypes.c_int)
@@ -33,6 +36,10 @@ def lib():
         L.oracle3d_step3ds.argtypes = [i, _dp, i, i, i, i, i, i, _dp, _dp, d, d, d, d, _ip, _ip, i]
         L.oracle3d_step3.restype = d
         L.oracle3d_step3.argtypes = [i, _dp, i, i, i, i, i, i, _dp, _dp, d, d, d, d, _ip, _ip]
+        L.oracle3d_sc_flux1.restype = d
+        L.oracle3d_sc_flux1.argtypes = [i, _dp, i, i, i, i, i, _dp, _dp, _dp, d, d, i, i, _ip]
+        L.oracle3d_sc_flux3.restype = d
+        L.oracle3d_sc_flux3.argtypes = [i, _dp, i, i, i, i, i, i, i, _dp, _dp, _dp, d, d, d, d, i, _ip]
         L.oracle3d_rp_point.restype = None
         L.oracle3d_rp_point.argtypes = [i, _dp, i, i, i, ctypes.c_longlong, _dp, _dp, _dp, _dp, _dp, _dp, i, _dp,
                                         _dp, _dp]
@@ -101,3 +108,71 @@ def rp3_transverse(rp_id, rp_params, ixyz, icoor, ql, qr, asdq):
     lib().oracle3d_rp_point(rp_id, _p(_params(rp_params)), ixyz, meqn, 1, n, _p(ql), _p(qr), null, null, null, null,
                             icoor, _p(asdq), _p(bm), _p(bp))
     return bm, bp
+
+
+def _mthlim8(mthlim, meqn):
+    """tvd2 limiter per COMPONENT (reconstruct.f90:568-625): one entry is repeated, as solver.limiters"""
+    lim = list(mthlim) if mthlim is not None else [1]
+    if len(lim) == 1:
+        lim = lim * meqn
+    out = np.zeros(8, dtype=np.int32)
+    out[: len(lim)] = lim
+    return out
+
+
+def sc_flux1(rp_id, rp_params, mwaves, mbc, mx, q1d, dx, dt, ixyz, weno_variant, aux1d=None, mthlim=None):
+    """flux1 on one slice in direction ixyz = 1, 2, 3: q1d [meqn, mx+2mbc], aux1d [maux, mx+2mbc] or None.
+    Returns (dq1d, cfl)."""
+    q1d = np.asfortranarray(q1d, dtype=np.float64)
+    dq = np.zeros_like(q1d, order="F")
+    null = ctypes.cast(None, _dp)
+    maux = 0 if aux1d is None else aux1d.shape[0]
+    a = null if aux1d is None else _p(np.asfortranarray(aux1d, dtype=np.float64))
+    lim = _mthlim8(mthlim, q1d.shape[0])
+    cfl = lib().oracle3d_sc_flux1(rp_id, _p(_params(rp_params)), q1d.shape[0], mwaves, maux, mbc, mx, _p(q1d), a,
+                                  _p(dq), dx, dt, ixyz, weno_variant, lim.ctypes.data_as(_ip))
+    return dq, _check(cfl)
+
+
+def sc_flux3(rp_id, rp_params, mwaves, mbc, mx, my, mz, q, dx, dy, dz, dt, weno_variant, aux=None, mthlim=None):
+    """SharpClaw's dq in 3-D (DESIGN.md §1): q [meqn, mx+2mbc, my+2mbc, mz+2mbc] with ghost cells filled,
+    aux [maux, ...] or None.  Returns (dq, cfl); dq is zero outside the interior."""
+    assert q.flags["F_CONTIGUOUS"]
+    dq = np.zeros_like(q, order="F")
+    null = ctypes.cast(None, _dp)
+    maux = 0 if aux is None else aux.shape[0]
+    a = null if aux is None else _p(np.asfortranarray(aux, dtype=np.float64))
+    lim = _mthlim8(mthlim, q.shape[0])
+    cfl = lib().oracle3d_sc_flux3(rp_id, _p(_params(rp_params)), q.shape[0], mwaves, maux, mbc, mx, my, mz, _p(q), a,
+                                  _p(dq), dx, dy, dz, dt, weno_variant, lim.ctypes.data_as(_ip))
+    return dq, _check(cfl)
+
+
+def sharpclaw3d_solver(rp_id, rp_params, mwaves):
+    """oracle/pyclaw_oracle.py's OracleSolver (kind 'sharpclaw': time integrators, boundary conditions,
+    variable dt with rejected steps, solver.py:602-717) with the 3-D dq of sc_flux3.  lim_type 1 / 2 / 3
+    select tvd2 / PyWENO weno5 (weno_variant, f32 by default) / the hand-written weno5."""
+    import sys
+    sys.path.insert(0, os.path.dirname(_HERE))
+    from oracle import pyclaw_oracle as po
+
+    class SharpClaw3D(po.OracleSolver):
+        def _dq(self, q, t):
+            self._bcs(q, t)
+            mbc = self.mbc
+            variant = {1: RECON_TVD2, 3: WENO_OLD}.get(self.lim_type, self.weno_variant)
+            mx, my, mz = self.n
+            dq, cfl = sc_flux3(self.rp_id, self.rp_params, self.mwaves, mbc, mx, my, mz, self.qbc, self.d[0],
+                               self.d[1], self.d[2], self.dt, variant, aux=self.auxbc, mthlim=self.limiters)
+            self.cfl = cfl
+            if cfl > self.cfl_max:
+                raise po._CFLError()
+            return po._interior(dq, mbc)
+
+        def setup(self, q, aux, d):
+            lim_type = self.lim_type
+            self.lim_type = 2  # the base class would set the 1-D / 2-D oracle's global tvd2 limiters
+            super().setup(q, aux, d)
+            self.lim_type = lim_type
+
+    return SharpClaw3D("sharpclaw", 3, rp_id, rp_params, mwaves)

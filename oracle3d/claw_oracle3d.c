@@ -575,3 +575,344 @@ void oracle3d_rp_point(int rp_id, const double *rp_params, int ixyz, int meqn, i
     }
     free(q); free(wave); free(s); free(amdq); free(apdq); free(asdq); free(bm); free(bp);
 }
+
+/* =========================================================================================== */
+/* SharpClaw in 3-D (the reference has none): flux1 (src/fortran/1d/sharpclaw/flux1.f90:2-195)  */
+/* over the x-, y- and z-slices of the grid, flux2.f90:2-96 extended by one dimension            */
+/* (DESIGN.md §1).  The reconstructions, flux1 and rpn3_vc_acoustics are copied from             */
+/* oracle/claw_oracle.c (weno5_pyweno, weno5_old, tvd2, sc_flux1_capa without a capacity         */
+/* function, rpn3_vc_acoustics) and pinned against it bit for bit by tests/test_sc3_oracle.py.    */
+/* =========================================================================================== */
+#define RP_ACOUSTICS3D_VC 8 /* aux = impedance, sound speed */
+#define WENO_PYWENO_F32 0
+#define WENO_PYWENO_F64 1
+#define WENO_OLD 2
+#define RECON_TVD2 4
+
+/* rpn3_vc_acoustics.f (oracle/claw_oracle.c) */
+static void rpn3_vc_acoustics(int ixyz, int meqn, int mwaves, int mbc, int mx, int maux,
+                              const double *ql, const double *qr, const double *auxl,
+                              const double *auxr, double *wave, double *s, double *amdq,
+                              double *apdq)
+{
+    const int mu = ixyz;
+    for (int i = 2 - mbc; i <= mx + mbc; i++) {
+        double delta1 = Q2(ql, 0, i) - Q2(qr, 0, i - 1);
+        double delta2 = Q2(ql, mu, i) - Q2(qr, mu, i - 1);
+        double zi = auxl[0 + maux * IX(i)], zim = auxr[0 + maux * IX(i - 1)];
+        double a1 = (-delta1 + zi * delta2) / (zim + zi);
+        double a2 = (delta1 + zim * delta2) / (zim + zi);
+        for (int m = 0; m < meqn; m++) { WV(m, 0, i) = 0.0; WV(m, 1, i) = 0.0; }
+        WV(0, 0, i) = -a1 * zim;
+        WV(mu, 0, i) = a1;
+        SP(0, i) = -auxr[1 + maux * IX(i - 1)];
+        WV(0, 1, i) = a2 * zi;
+        WV(mu, 1, i) = a2;
+        SP(1, i) = auxl[1 + maux * IX(i)];
+        for (int m = 0; m < meqn; m++) {
+            Q2(amdq, m, i) = SP(0, i) * WV(m, 0, i);
+            Q2(apdq, m, i) = SP(1, i) * WV(m, 1, i);
+        }
+    }
+    (void)mwaves;
+}
+
+/* the normal solve of a SharpClaw slice: every 3-D solver of this file */
+static void rpn3_sc(const rp_ctx3 *c, int ixyz, int meqn, int mwaves, int mbc, int mx, int maux, const double *ql,
+                    const double *qr, const double *auxl, const double *auxr, double *wave, double *s, double *amdq,
+                    double *apdq)
+{
+    if (c->rp_id == RP_ACOUSTICS3D_VC)
+        rpn3_vc_acoustics(ixyz, meqn, mwaves, mbc, mx, maux, ql, qr, auxl, auxr, wave, s, amdq, apdq);
+    else rpn3(c, ixyz, mbc, mx, ql, qr, wave, s, amdq, apdq);
+}
+
+#define QP(arr, m, p) arr[(m) + meqn * ((p)-1)]
+
+/* weno.f90:5-102 (PyWENO generated), as oracle/claw_oracle.c weno5_pyweno */
+static void weno5_pyweno(const double *q, double *ql, double *qr, int meqn, int mx, int mbc,
+                         int f32lit)
+{
+#define LIT(x) (f32lit ? (double)(x##f) : (double)(x))
+    const double c333 = LIT(3.33333333333333), c1033 = LIT(10.3333333333333),
+                 c366 = LIT(3.66666666666667), c833 = LIT(8.33333333333333),
+                 c633 = LIT(6.33333333333333), c133 = LIT(1.33333333333333),
+                 c433 = LIT(4.33333333333333), c166 = LIT(1.66666666666667);
+    const double d01 = LIT(0.1), d06 = LIT(0.6), d03 = LIT(0.3), eps = LIT(1.0e-36);
+    const double r183 = LIT(1.83333333333333), r116 = LIT(1.16666666666667),
+                 r0333 = LIT(0.333333333333333), r0833 = LIT(0.833333333333333),
+                 r0166 = LIT(0.166666666666667);
+#undef LIT
+    for (int p = mbc; p <= mx + mbc + 1; p++) {
+        for (int m = 0; m < meqn; m++) {
+            double qm2 = QP(q, m, p - 2), qm1 = QP(q, m, p - 1), q0 = QP(q, m, p),
+                   qp1 = QP(q, m, p + 1), qp2 = QP(q, m, p + 2);
+            double sigma0 = ((c333)*q0) * q0 + ((-c1033) * q0) * qp1 + ((c366)*q0) * qp2 +
+                            ((c833)*qp1) * qp1 + ((-c633) * qp1) * qp2 + ((c133)*qp2) * qp2;
+            double sigma1 = ((c133)*qm1) * qm1 + ((-c433) * qm1) * q0 + ((c166)*qm1) * qp1 +
+                            ((c433)*q0) * q0 + ((-c433) * q0) * qp1 + ((c133)*qp1) * qp1;
+            double sigma2 = ((c133)*qm2) * qm2 + ((-c633) * qm2) * qm1 + ((c366)*qm2) * q0 +
+                            ((c833)*qm1) * qm1 + ((-c1033) * qm1) * q0 + ((c333)*q0) * q0;
+            double acc = 0.0;
+            double omega0 = d01 / ((sigma0 + eps) * (sigma0 + eps));
+            acc = acc + omega0;
+            double omega1 = d06 / ((sigma1 + eps) * (sigma1 + eps));
+            acc = acc + omega1;
+            double omega2 = d03 / ((sigma2 + eps) * (sigma2 + eps));
+            acc = acc + omega2;
+            omega0 = omega0 / acc;
+            omega1 = omega1 / acc;
+            omega2 = omega2 / acc;
+            acc = 0.0;
+            double omega3 = d03 / ((sigma0 + eps) * (sigma0 + eps));
+            acc = acc + omega3;
+            double omega4 = d06 / ((sigma1 + eps) * (sigma1 + eps));
+            acc = acc + omega4;
+            double omega5 = d01 / ((sigma2 + eps) * (sigma2 + eps));
+            acc = acc + omega5;
+            omega3 = omega3 / acc;
+            omega4 = omega4 / acc;
+            omega5 = omega5 / acc;
+            double fr0 = (r183)*q0 + (-r116) * qp1 + (r0333)*qp2;
+            double fr1 = (r0333)*qm1 + (r0833)*q0 + (-r0166) * qp1;
+            double fr2 = (-r0166) * qm2 + (r0833)*qm1 + (r0333)*q0;
+            double fr3 = (r0333)*q0 + (r0833)*qp1 + (-r0166) * qp2;
+            double fr4 = (-r0166) * qm1 + (r0833)*q0 + (r0333)*qp1;
+            double fr5 = (r0333)*qm2 + (-r116) * qm1 + (r183)*q0;
+            QP(ql, m, p) = omega0 * fr0 + omega1 * fr1 + omega2 * fr2;
+            QP(qr, m, p) = omega3 * fr3 + omega4 * fr4 + omega5 * fr5;
+        }
+    }
+}
+
+/* reconstruct.f90:120-185 (hand-written weno5, lim_type = 3), as oracle/claw_oracle.c weno5_old */
+static void weno5_old(const double *q, double *ql, double *qr, int meqn, int mx, int mbc,
+                      double *dq1m, double *uu)
+{
+    const double epweno = (double)1.e-36f; /* "1.e-36" is a REAL(4) literal, reconstruct.f90:7 */
+    int mx2 = mx + 2 * mbc;
+    for (int m = 0; m < meqn; m++) {
+        for (int p = 2; p <= mx2; p++) dq1m[p] = QP(q, m, p) - QP(q, m, p - 1);
+        for (int m1 = 1; m1 <= 2; m1++) {
+            int im = (m1 == 1) ? 1 : -1;
+            int ione = im, inone = -im, intwo = -2 * im;
+            for (int p = mbc; p <= mx2 - mbc + 1; p++) {
+                double t1 = im * (dq1m[p + intwo] - dq1m[p + inone]);
+                double t2 = im * (dq1m[p + inone] - dq1m[p]);
+                double t3 = im * (dq1m[p] - dq1m[p + ione]);
+                double e1 = dq1m[p + intwo] - 3. * dq1m[p + inone];
+                double e2 = dq1m[p + inone] + dq1m[p];
+                double e3 = 3. * dq1m[p] - dq1m[p + ione];
+                double tt1 = 13. * (t1 * t1) + 3. * (e1 * e1);
+                double tt2 = 13. * (t2 * t2) + 3. * (e2 * e2);
+                double tt3 = 13. * (t3 * t3) + 3. * (e3 * e3);
+                tt1 = (epweno + tt1) * (epweno + tt1);
+                tt2 = (epweno + tt2) * (epweno + tt2);
+                tt3 = (epweno + tt3) * (epweno + tt3);
+                double s1 = tt2 * tt3;
+                double s2 = 6. * tt1 * tt3;
+                double s3 = 3. * tt1 * tt2;
+                double t0 = 1. / (s1 + s2 + s3);
+                s1 = s1 * t0;
+                s3 = s3 * t0;
+                uu[(m1 - 1) + 2 * p] =
+                    (s1 * (t2 - t1) + (0.5 * s3 - 0.25) * (t3 - t2)) / 3. +
+                    (-QP(q, m, p - 2) + 7. * (QP(q, m, p - 1) + QP(q, m, p)) - QP(q, m, p + 1)) / 12.;
+            }
+        }
+        for (int p = mbc; p <= mx2 - mbc + 1; p++) {
+            QP(qr, m, p - 1) = uu[0 + 2 * p];
+            QP(ql, m, p) = uu[1 + 2 * p];
+        }
+    }
+}
+
+/* gfortran's MIN / MAX: a NaN argument loses (oracle/claw_oracle.c) */
+static inline double fmin_g(double a1, double a2) { return (a2 < a1 || a1 != a1) ? a2 : a1; }
+static inline double fmax_g(double a1, double a2) { return (a2 > a1 || a1 != a1) ? a2 : a1; }
+
+/* reconstruct.f90:568-625 (tvd2), as oracle/claw_oracle.c tvd2 with the limiter per component
+   passed in (mthlim[m]) instead of set beforehand; the first cell uses its own backward difference */
+static void tvd2(const double *q, double *ql, double *qr, int meqn, int mx, int mbc, const int *mthlim)
+{
+    const int mx2 = mx + 2 * mbc;
+    for (int m = 0; m < meqn; m++) {
+        double dqp = QP(q, m, 3) - QP(q, m, 2);
+        for (int p = 3; p <= mx2 - 2; p++) {
+            double dqm = dqp;
+            dqp = QP(q, m, p + 1) - QP(q, m, p);
+            double r = dqp / dqm;
+            double qlimitr = 0.0;
+            switch (mthlim[m]) {
+            case 1: qlimitr = fmax_g(0.0, fmin_g(1.0, r)); break;
+            case 2: qlimitr = fmax_g(fmax_g(0.0, fmin_g(1.0, 2.0 * r)), fmin_g(2.0, r)); break;
+            case 3: qlimitr = (r + fabs(r)) / (1.0 + fabs(r)); break;
+            case 4: {
+                double c = (1.0 + r) / 2.0;
+                qlimitr = fmax_g(0.0, fmin_g(fmin_g(c, 2.0), 2.0 * r));
+            } break;
+            case 5: {
+                const double beta = 2.0, xgamma = 2.0, alpha = 1.0 / 3.0;
+                double pp = (2.0 + r) / 3.0;
+                double amax = fmax_g(fmax_g(-alpha * r, 0.0), fmin_g(fmin_g(beta * r, pp), xgamma));
+                qlimitr = fmax_g(0.0, fmin_g(pp, amax));
+            } break;
+            default: qlimitr = 0.0;
+            }
+            QP(qr, m, p) = QP(q, m, p) + 0.5 * qlimitr * dqm;
+            QP(ql, m, p) = QP(q, m, p) - 0.5 * qlimitr * dqm;
+        }
+    }
+}
+
+typedef struct {
+    double *ql, *qr, *wave, *s, *amdq, *apdq, *amdq2, *apdq2, *dq1m, *uu, *auxl2, *auxr2;
+} sc_work;
+
+/* flux1.f90:2-195 on one slice (sc_flux1_capa of oracle/claw_oracle.c without a capacity function):
+   dq1d = 0 - dtdx (amdq(i+1) + apdq(i) + amdq2(i) + apdq2(i)) for i = 1..mx; returns the Courant number
+   of the interfaces 1..mx+1.  aux1d (maux, n) or NULL. */
+static double sc_flux1(const rp_ctx3 *c, const double *q1d, const double *aux1d, int maux, double *dq1d, double dt,
+                       double dxv, int ixyz, int meqn, int mwaves, int mx, int mbc, int weno_variant,
+                       const int *mthlim, sc_work *w)
+{
+    int n = mx + 2 * mbc;
+    double *ql = w->ql, *qr = w->qr, *wave = w->wave, *s = w->s;
+    double *amdq = w->amdq, *apdq = w->apdq, *amdq2 = w->amdq2, *apdq2 = w->apdq2;
+    const double dtdx = dt / dxv;
+    for (int k = 0; k < n * meqn; k++) dq1d[k] = 0.0;
+    memcpy(ql, q1d, sizeof(double) * n * meqn);
+    memcpy(qr, q1d, sizeof(double) * n * meqn);
+    if (weno_variant == RECON_TVD2) tvd2(q1d, ql, qr, meqn, mx, mbc, mthlim);
+    else if (weno_variant == WENO_OLD) weno5_old(q1d, ql, qr, meqn, mx, mbc, w->dq1m, w->uu);
+    else weno5_pyweno(q1d, ql, qr, meqn, mx, mbc, weno_variant == WENO_PYWENO_F32);
+    /* :128 rp(ql, qr, aux, aux) */
+    rpn3_sc(c, ixyz, meqn, mwaves, mbc, mx, maux, ql, qr, aux1d, aux1d, wave, s, amdq, apdq);
+    double cfl = 0.0;
+    for (int mw = 0; mw < mwaves; mw++)
+        for (int i = 1; i <= mx + 1; i++) cfl = dmax2(dmax2(cfl, dtdx * SP(mw, i)), -dtdx * SP(mw, i));
+    /* :170-175 swap so that interface i of the second solve is the in-cell problem */
+    for (int i = 1 - mbc + 1; i <= mx + mbc; i++)
+        for (int m = 0; m < meqn; m++) {
+            Q2(qr, m, i - 1) = Q2(ql, m, i);
+            Q2(ql, m, i) = Q2(qr, m, i);
+        }
+    const double *auxl2 = NULL, *auxr2 = NULL;
+    if (aux1d && maux > 0) { /* :177-184 auxr(i-1) = aux(i), auxl(i) = aux(i) */
+        memcpy(w->auxl2, aux1d, sizeof(double) * n * maux);
+        memcpy(w->auxr2, aux1d, sizeof(double) * n * maux);
+        for (int i = 1 - mbc + 1; i <= mx + mbc; i++)
+            for (int ma = 0; ma < maux; ma++) {
+                w->auxr2[ma + maux * IX(i - 1)] = aux1d[ma + maux * IX(i)];
+                w->auxl2[ma + maux * IX(i)] = aux1d[ma + maux * IX(i)];
+            }
+        auxl2 = w->auxl2;
+        auxr2 = w->auxr2;
+    }
+    rpn3_sc(c, ixyz, meqn, mwaves, mbc, mx, maux, ql, qr, auxl2, auxr2, wave, s, amdq2, apdq2);
+    for (int i = 1; i <= mx; i++)
+        for (int m = 0; m < meqn; m++)
+            Q2(dq1d, m, i) = Q2(dq1d, m, i) -
+                             dtdx * (Q2(amdq, m, i + 1) + Q2(apdq, m, i) + Q2(amdq2, m, i) + Q2(apdq2, m, i));
+    return cfl;
+}
+
+static int sc_known(int rp_id, int weno_variant)
+{
+    return (known(rp_id) || rp_id == RP_ACOUSTICS3D_VC) &&
+           (weno_variant == WENO_PYWENO_F32 || weno_variant == WENO_PYWENO_F64 || weno_variant == WENO_OLD ||
+            weno_variant == RECON_TVD2);
+}
+
+static void sc_work_alloc(sc_work *w, int n, int meqn, int mwaves, int maux)
+{
+    double **a[] = {&w->ql, &w->qr, &w->amdq, &w->apdq, &w->amdq2, &w->apdq2};
+    for (int k = 0; k < 6; k++) *a[k] = (double *)calloc((size_t)n * meqn, sizeof(double));
+    w->wave = (double *)calloc((size_t)n * meqn * mwaves, sizeof(double));
+    w->s = (double *)calloc((size_t)n * mwaves, sizeof(double));
+    w->dq1m = (double *)calloc(n + 2, sizeof(double));
+    w->uu = (double *)calloc(2 * (size_t)(n + 2), sizeof(double));
+    w->auxl2 = (double *)calloc((size_t)n * (maux > 0 ? maux : 1), sizeof(double));
+    w->auxr2 = (double *)calloc((size_t)n * (maux > 0 ? maux : 1), sizeof(double));
+}
+static void sc_work_free(sc_work *w)
+{
+    free(w->ql); free(w->qr); free(w->amdq); free(w->apdq); free(w->amdq2); free(w->apdq2);
+    free(w->wave); free(w->s); free(w->dq1m); free(w->uu); free(w->auxl2); free(w->auxr2);
+}
+
+/* One slice (flux1) on its own: q1d (meqn, mx+2mbc), aux1d (maux, mx+2mbc) or NULL, dq1d out.
+   ixyz = 1, 2, 3 is the direction of the slice.  Returns the Courant number, -1 if unsupported. */
+double oracle3d_sc_flux1(int rp_id, const double *rp_params, int meqn, int mwaves, int maux, int mbc, int mx,
+                         const double *q1d, const double *aux1d, double *dq1d, double dx, double dt, int ixyz,
+                         int weno_variant, const int *mthlim)
+{
+    if (!sc_known(rp_id, weno_variant)) return -1.0;
+    rp_ctx3 c;
+    c.rp_id = rp_id;
+    memcpy(c.p, rp_params, 8 * sizeof(double));
+    sc_work w;
+    sc_work_alloc(&w, mx + 2 * mbc, meqn, mwaves, maux);
+    double cfl = sc_flux1(&c, q1d, aux1d, maux, dq1d, dt, dx, ixyz, meqn, mwaves, mx, mbc, weno_variant, mthlim, &w);
+    sc_work_free(&w);
+    return cfl;
+}
+
+/* flux3 of SharpClaw in 3-D: q (meqn, NX, NY, NZ) Fortran order with ghost cells filled, aux (maux, ...)
+   or NULL, dq zero on entry; dq(:, i, j, k) = ((0 + dq_x) + dq_y) + dq_z on the interior.  Slices: x over
+   (j, k) in [0, my+1] x [0, mz+1], y over (i, k) in [0, mx+1] x [0, mz+1], z over (i, j) in [0, mx+1] x
+   [0, my+1].  Returns the largest Courant number of all slices, -1 if unsupported. */
+double oracle3d_sc_flux3(int rp_id, const double *rp_params, int meqn, int mwaves, int maux, int mbc, int mx,
+                         int my, int mz, const double *q, const double *aux, double *dq, double dx, double dy,
+                         double dz, double dt, int weno_variant, const int *mthlim)
+{
+    if (!sc_known(rp_id, weno_variant)) return -1.0;
+    if (rp_id == RP_ACOUSTICS3D_VC && (!aux || maux < 2)) return -1.0;
+    rp_ctx3 c;
+    c.rp_id = rp_id;
+    memcpy(c.p, rp_params, 8 * sizeof(double));
+    int maxm = mx > my ? mx : my;
+    if (mz > maxm) maxm = mz;
+    const int n = maxm + 2 * mbc;
+    const int ma = aux ? maux : 0;
+    sc_work w;
+    sc_work_alloc(&w, n, meqn, mwaves, ma);
+    double *q1d = (double *)calloc((size_t)n * meqn, sizeof(double));
+    double *dq1d = (double *)calloc((size_t)n * meqn, sizeof(double));
+    double *aux1d = (double *)calloc((size_t)n * (ma > 0 ? ma : 1), sizeof(double));
+    const size_t NXs = mx + 2 * mbc, NYs = my + 2 * mbc;
+#define OFF4(i, j, k) (((i) + mbc - 1) + NXs * (((j) + mbc - 1) + NYs * ((k) + mbc - 1)))
+#define Q4(arr, m, i, j, k) arr[(m) + (size_t)meqn * OFF4(i, j, k)]
+#define AUX4(a, i, j, k) aux[(a) + (size_t)ma * OFF4(i, j, k)]
+    const double dd[3] = {dx, dy, dz};
+    const int len[3] = {mx, my, mz};
+    double cfl = 0.0;
+    for (int d = 0; d < 3; d++) {
+        const int o1 = (d == 0) ? 1 : 0, o2 = (d == 2) ? 1 : 2;
+        int idx[3];
+        for (idx[o2] = 0; idx[o2] <= len[o2] + 1; idx[o2]++)
+            for (idx[o1] = 0; idx[o1] <= len[o1] + 1; idx[o1]++) {
+                for (int l = 1 - mbc; l <= len[d] + mbc; l++) {
+                    idx[d] = l;
+                    for (int m = 0; m < meqn; m++) Q2(q1d, m, l) = Q4(q, m, idx[0], idx[1], idx[2]);
+                    for (int a = 0; a < ma; a++) aux1d[a + ma * IX(l)] = AUX4(a, idx[0], idx[1], idx[2]);
+                }
+                double cfl1d = sc_flux1(&c, q1d, ma > 0 ? aux1d : NULL, ma, dq1d, dt, dd[d], d + 1, meqn, mwaves,
+                                        len[d], mbc, weno_variant, mthlim, &w);
+                cfl = dmax2(cfl, cfl1d);
+                const int interior = idx[o1] >= 1 && idx[o1] <= len[o1] && idx[o2] >= 1 && idx[o2] <= len[o2];
+                if (!interior) continue; /* ghost slices: Courant number only */
+                for (int l = 1; l <= len[d]; l++) {
+                    idx[d] = l;
+                    for (int m = 0; m < meqn; m++)
+                        Q4(dq, m, idx[0], idx[1], idx[2]) = Q4(dq, m, idx[0], idx[1], idx[2]) + Q2(dq1d, m, l);
+                }
+            }
+    }
+#undef AUX4
+#undef Q4
+#undef OFF4
+    free(q1d); free(dq1d); free(aux1d);
+    sc_work_free(&w);
+    return cfl;
+}

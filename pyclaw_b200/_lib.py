@@ -103,6 +103,7 @@ SIGNATURES = {
     "clawb200_step2_parts": [_pp, _dp, _dp, _dp, _d, _i, _dp, _vp],
     "clawb200_step2_rows": [_pp, _dp, _dp, _dp, _d, _i, _i, _dp, _vp],
     "clawb200_sharpclaw_stage": [_pp, _dp, _dp, _dp, _dp, _dp, _d, _i, _d, _d, _d, _dp, _vp],
+    "clawb200_sharpclaw_stage3": [_pp, _i, _d, _dp, _dp, _dp, _dp, _dp, _d, _i, _d, _d, _d, _dp, _vp],
     "clawb200_ssp104_combine": [_dp, _dp, _dp, ctypes.c_longlong, _vp],
     "clawb200_sphere_src2": [_pp, _dp, _dp, _d, _vp],
     "clawb200_bc_fill": [_pp, _dp, _i, _i, _i, _i, _i, _vp],
@@ -114,6 +115,7 @@ SIGNATURES = {
     "clawb200_step2ds_host": [_pp, _dp, _dp, _dp, _d, _i, _dref],
     "clawb200_step2_host": [_pp, _dp, _dp, _dp, _d, _dref],
     "clawb200_sharpclaw_dq_host": [_pp, _dp, _dp, _dp, _d, _dref],
+    "clawb200_sharpclaw_dq3_host": [_pp, _i, _d, _dp, _dp, _dp, _d, _dref],
     "clawb200_pack_weno_tables": [_i, _dp, _dp, _dp, _dp, _dp, _d, _dp],
     "clawb200_step3ds": [_pp, _i, _d, _dp, _dp, _dp, _d, _i, _dp, _vp],
     "clawb200_bc_fill3": [_pp, _i, _dp, _i, _i, _i, _i, _i, _vp],

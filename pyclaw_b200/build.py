@@ -41,7 +41,10 @@ UNITS = {
     "step3_misc.cu": _COMMON + ["step3.cuh"],     # ... 3-D advection
     "rp_point.cu": _COMMON,
     "sharpclaw.cu": _COMMON + ["sharpclaw.cuh"],
-    "sweep_user.cu": _COMMON + ["sharpclaw.cuh", "step3.cuh"],   # the user-supplied Riemann solver (a stub without one)
+    "sharpclaw3.cu": _COMMON + ["sharpclaw.cuh", "sharpclaw3.cuh"],        # 3-D SharpClaw stage: vc-acoustics
+    "sharpclaw3_euler.cu": _COMMON + ["sharpclaw.cuh", "sharpclaw3.cuh"],  # ... 3-D Euler
+    "sharpclaw3_misc.cu": _COMMON + ["sharpclaw.cuh", "sharpclaw3.cuh"],   # ... 3-D advection
+    "sweep_user.cu": _COMMON + ["sharpclaw.cuh", "sharpclaw3.cuh", "step3.cuh"],   # the user-supplied Riemann solver (a stub without one)
 }
 SOURCES = list(UNITS)
 HEADERS = sorted({h for hs in UNITS.values() for h in hs})

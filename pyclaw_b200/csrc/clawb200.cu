@@ -614,6 +614,7 @@ extern "C" int clawb200_sharpclaw_stage(const clawb200_problem *p, const double 
                                         double *cfl_dev, void *stream)
 {
     if (!p) return fail(CLAWB200_ERR_INVALID, "null problem");
+    if (p->ndim == 3) return fail(CLAWB200_ERR_INVALID, "3-D problem: the 3-D SharpClaw stage is clawb200_sharpclaw_stage3");
     int rc = check_problem(p, p->ndim);
     if (rc) return rc;
     if ((rc = check_rp_shape(p))) return rc;
@@ -623,6 +624,34 @@ extern "C" int clawb200_sharpclaw_stage(const clawb200_problem *p, const double 
     if (out == q) return fail(CLAWB200_ERR_INVALID, "out must not alias q");
     if ((rc = check_aux(p, aux, false))) return rc;
     return sharpclaw_launch(p, q, qa, out, dq_out, dt, mode, ca, cb, div, cfl_dev, (cudaStream_t)stream, aux);
+}
+
+extern "C" int clawb200_sharpclaw_stage3(const clawb200_problem *p, int mz, double dz, const double *q,
+                                         const double *qa, double *out, double *dq_out, const double *aux,
+                                         double dt, int mode, double ca, double cb, double div,
+                                         double *cfl_dev, void *stream)
+{
+    int rc = check_problem(p, 3);
+    if (rc) return rc;
+    if ((rc = check_rp3(p, aux != nullptr))) return rc;
+    if (p->method[5] > 0) return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa (capacity function) is not compiled for the 3-D SharpClaw stage");
+    const int wv = p->weno_variant;
+    if (wv == CLAWB200_WENO_TABLES) return fail(CLAWB200_ERR_UNSUPPORTED, "WENO orders above 5 are not compiled in 3-D");
+    if (wv != CLAWB200_WENO_PYWENO_F32 && wv != CLAWB200_WENO_PYWENO_F64 && wv != CLAWB200_WENO_OLD && wv != CLAWB200_RECON_TVD2)
+        return fail(CLAWB200_ERR_UNSUPPORTED, "3-D SharpClaw: weno_variant must be PyWENO (f32 / f64), the hand-written weno5 or tvd2");
+    if (p->mbc < 3) return fail(CLAWB200_ERR_INVALID, "WENO5 needs mbc >= 3");
+    if (mz < 1 || !(dz > 0.0)) return fail(CLAWB200_ERR_INVALID, "mz, dz must be positive");
+    if (mode < 0 || mode > 3) return fail(CLAWB200_ERR_INVALID, "bad stage mode");
+    if ((mode == 1 || mode == 2) && !qa) return fail(CLAWB200_ERR_INVALID, "this stage mode needs qa");
+    if (mode == 3 && !dq_out) return fail(CLAWB200_ERR_INVALID, "stage mode 3 needs dq_out in 3-D");
+    if (mode != 3 && !out) return fail(CLAWB200_ERR_INVALID, "this stage mode needs out");
+    if (!q || out == q || dq_out == q) return fail(CLAWB200_ERR_INVALID, "out and dq_out must not alias q");
+    if ((qa && (qa == out || qa == dq_out)) || (out && out == dq_out))
+        return fail(CLAWB200_ERR_INVALID, "out, dq_out and qa must be different buffers (the x/y partial of dq is held in one of them)");
+    const long long plane = (long long)p->pitch * (p->my + 2 * p->mbc);
+    if (p->mstride < plane * (mz + 2 * p->mbc)) return fail(CLAWB200_ERR_INVALID, "mstride smaller than the padded field");
+    if (mz + 2 > 65535) return fail(CLAWB200_ERR_UNSUPPORTED, "mz must be below 65534");
+    return sharpclaw_launch3(p, mz, dz, q, qa, out, dq_out, dt, mode, ca, cb, div, cfl_dev, (cudaStream_t)stream, aux);
 }
 
 // ---------------------------------------------------------------------------
@@ -1202,6 +1231,31 @@ extern "C" int clawb200_step3_host(const clawb200_problem *p, int mz, double dz,
     else cudaStreamSynchronize(g_hs.st);
     cudaFree(scratch);
     return rc;
+}
+
+// flux3 of the 3-D SharpClaw stage with host arrays q(meqn, mx+2mbc, my+2mbc, mz+2mbc)
+extern "C" int clawb200_sharpclaw_dq3_host(const clawb200_problem *p, int mz, double dz, const double *q,
+                                           double *dq, const double *aux, double dt, double *cfl)
+{
+    if (!p || !q || !dq) return fail(CLAWB200_ERR_INVALID, "null argument");
+    if (p->ndim != 3 || mz < 1) return fail(CLAWB200_ERR_INVALID, "3-D problem expected");
+    clawb200_problem P = *p;
+    P.dt_dev = nullptr;
+    const int nx = p->mx + 2 * p->mbc, ny = p->my + 2 * p->mbc, nz = mz + 2 * p->mbc;
+    P.pitch = nx;
+    P.mstride = (long long)nx * ny * nz;
+    int rc = g_hs.ensure((size_t)(P.meqn > P.maux ? P.meqn : P.maux) * P.mstride);
+    if (rc) return rc;
+    if ((rc = host_upload(P, q, g_hs.d_a))) return rc;
+    const double *d_aux;
+    if ((rc = host_upload_aux(P, aux, &d_aux))) return rc;
+    CUDA_OK(cudaMemsetAsync(g_hs.d_b, 0, (size_t)P.meqn * P.mstride * sizeof(double), g_hs.st));
+    if ((rc = clawb200_cfl_reset(g_hs.d_cfl, g_hs.st))) return rc;
+    if ((rc = clawb200_sharpclaw_stage3(&P, mz, dz, g_hs.d_a, nullptr, nullptr, g_hs.d_b, d_aux, dt,
+                                        CLAWB200_STAGE_DQ_ONLY, 0.0, 0.0, 1.0, g_hs.d_cfl, g_hs.st)))
+        return rc;
+    if ((rc = host_download(P, g_hs.d_b, dq))) return rc;
+    return host_finish(cfl);
 }
 
 // classic3.step3ds with host arrays q(meqn, mx+2mbc, my+2mbc, mz+2mbc) (clawpack.py:656-676)

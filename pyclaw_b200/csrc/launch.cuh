@@ -5,7 +5,8 @@
 // parallel): clawb200.cu (C ABI, boundary fills, layout / halo kernels, host entry points),
 // sweep_euler_x.cu / sweep_euler_y.cu, sweep_sphere.cu, sweep_misc.cu (instantiations of the
 // classic sweeps per Riemann-solver family), sweep_user.cu (the user-supplied solver), step1.cu,
-// step3.cu / step3_euler.cu / step3_misc.cu (the 3-D steps), rp_point.cu, sharpclaw.cu.
+// step3.cu / step3_euler.cu / step3_misc.cu (the 3-D steps), rp_point.cu, sharpclaw.cu,
+// sharpclaw3.cu / sharpclaw3_euler.cu / sharpclaw3_misc.cu (the 3-D SharpClaw stage).
 #pragma once
 #include <cuda_runtime.h>
 #include <cstdio>
@@ -139,6 +140,12 @@ int claw_x_user(bool trans, const SweepArgs &A, cudaStream_t st);
 int claw_y_user(bool trans, const SweepArgs &A, cudaStream_t st);
 int claw_step1_user(const SweepArgs &A, int mx, cudaStream_t st);
 int claw_sc_user(int ndim, bool old, const ScArgs &A, cudaStream_t st);
+// 3-D SharpClaw stage (sharpclaw3.cuh), one translation unit per solver family (sharpclaw3.cu,
+// sharpclaw3_euler.cu, sharpclaw3_misc.cu, sweep_user.cu)
+int claw_sc3_acoustics(bool old, const ScArgs &A, cudaStream_t st);
+int claw_sc3_euler(bool old, const ScArgs &A, cudaStream_t st);
+int claw_sc3_advection(bool old, const ScArgs &A, cudaStream_t st);
+int claw_sc3_user(bool old, const ScArgs &A, cudaStream_t st);
 int claw_rp_point_user(const clawb200_problem *p, int ixy, long long n, const double *ql, const double *qr,
                        const double *auxl, const double *auxr, double *wave, double *s, double *amdq,
                        double *apdq, int imp, const double *asdq, double *bm, double *bp, cudaStream_t st);
@@ -149,3 +156,6 @@ int claw_step1(int rp_id, const SweepArgs &A, int mx, cudaStream_t st);
 int sharpclaw_launch(const clawb200_problem *p, const double *q, const double *qa, double *out,
                      double *dq_out, double dt, int mode, double ca, double cb, double div,
                      double *cfl_dev, cudaStream_t st, const double *aux);
+int sharpclaw_launch3(const clawb200_problem *p, int mz, double dz, const double *q, const double *qa, double *out,
+                      double *dq_out, double dt, int mode, double ca, double cb, double div,
+                      double *cfl_dev, cudaStream_t st, const double *aux);

@@ -93,11 +93,11 @@ static int sc_launch1(const ScArgs &A, cudaStream_t st)
     return 0;
 }
 
-int sharpclaw_launch(const clawb200_problem *p, const double *q, const double *qa, double *out,
-                            double *dq_out, double dt, int mode, double ca, double cb, double div,
-                            double *cfl_dev, cudaStream_t st, const double *aux)
+// the stage arguments common to 1-D, 2-D and 3-D
+static int sc_args(ScArgs &A, const clawb200_problem *p, const double *q, const double *qa, double *out,
+                   double *dq_out, double dt, int mode, double ca, double cb, double div, double *cfl_dev,
+                   const double *aux)
 {
-    ScArgs A;
     memset(&A, 0, sizeof(A));
     A.q = q; A.qa = qa; A.out = out; A.dq_out = dq_out;
     A.mstride = p->mstride; A.pitch = p->pitch;
@@ -110,12 +110,43 @@ int sharpclaw_launch(const clawb200_problem *p, const double *q, const double *q
     A.amstride = p->mstride;
     A.mode = mode; A.ca = ca; A.cb = cb; A.div = div;
     A.cfl_bits = (unsigned long long *)cfl_dev;
-    const bool old = (p->weno_variant == CLAWB200_WENO_OLD);
     if (p->weno_variant == CLAWB200_RECON_TVD2) {
         if (p->meqn > CLAWB200_MAXWAVES) return fail(CLAWB200_ERR_INVALID, "tvd2: meqn exceeds the limiter array");
         A.tvd = 1;
         for (int m = 0; m < p->meqn; m++) A.mthlim[m] = p->mthlim[m];
     }
+    return 0;
+}
+
+// 3-D (sharpclaw3.cuh): WENO5 (both literal readings), hand-written weno5 and tvd2; the caller
+// (clawb200_sharpclaw_stage3) has rejected everything else
+int sharpclaw_launch3(const clawb200_problem *p, int mz, double dz, const double *q, const double *qa, double *out,
+                      double *dq_out, double dt, int mode, double ca, double cb, double div,
+                      double *cfl_dev, cudaStream_t st, const double *aux)
+{
+    ScArgs A;
+    int rc = sc_args(A, p, q, qa, out, dq_out, dt, mode, ca, cb, div, cfl_dev, aux);
+    if (rc) return rc;
+    A.plane = (long long)p->pitch * (p->my + 2 * p->mbc);
+    A.mz = mz;
+    A.dtdz = dt / dz;
+    const bool old = (p->weno_variant == CLAWB200_WENO_OLD);
+    switch (p->rp_id) {
+    case CLAWB200_RP_ACOUSTICS3D_VC: return claw_sc3_acoustics(old, A, st);
+    case CLAWB200_RP_EULER3D: return claw_sc3_euler(old, A, st);
+    case CLAWB200_RP_ADVECTION3D: return claw_sc3_advection(old, A, st);
+    default: return claw_sc3_user(old, A, st);
+    }
+}
+
+int sharpclaw_launch(const clawb200_problem *p, const double *q, const double *qa, double *out,
+                            double *dq_out, double dt, int mode, double ca, double cb, double div,
+                            double *cfl_dev, cudaStream_t st, const double *aux)
+{
+    ScArgs A;
+    int rc = sc_args(A, p, q, qa, out, dq_out, dt, mode, ca, cb, div, cfl_dev, aux);
+    if (rc) return rc;
+    const bool old = (p->weno_variant == CLAWB200_WENO_OLD);
     if (p->weno_variant == CLAWB200_WENO_TABLES) {
         const int wk = p->weno_k;
         if (wk < 3 || wk > 9 || !p->weno_tab)

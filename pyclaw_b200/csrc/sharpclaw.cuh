@@ -45,6 +45,10 @@ struct ScArgs {
     // lim_type = 1 (flux1.f90:79-83): second-order TVD reconstruction, limiter id per COMPONENT
     int tvd;
     int mthlim[8];
+    // 3-D (sharpclaw3.cuh): doubles per z-plane, mz, dt/dz
+    long long plane;
+    int mz;
+    double dtdz;
 };
 
 // aux of the cell at array offset `off` (row offset + clamped column)
@@ -311,11 +315,13 @@ __device__ __forceinline__ void sc_xrow_solve(const ScArgs &A, const double (&ql
 
 // ---------------------------------------------------------------------------
 // 2-D: thread t <-> column ic = i0-1+t, output columns t = 1 .. NT-2.
+// D3: the x and y directions of one z-plane k = blockIdx.z of [0, mz+1] of a 3-D field
+// (sharpclaw3.cuh).  The ghost planes 0 and mz+1 add to the Courant number only.
 // ---------------------------------------------------------------------------
 #ifndef CLAW_SC_MINB
 #define CLAW_SC_MINB 3 // 168 registers, 44 B of spills: 35.96 -> 32.49 ms per step (strict), 25.8 -> 21.6 ms (fma) at 8192^2; 4 CTAs spill 270 B
 #endif
-template <class RPX, class RPY, bool OLD, int NT, bool CAPA = false>
+template <class RPX, class RPY, bool OLD, int NT, bool CAPA = false, bool D3 = false>
 __global__ void __launch_bounds__(NT, (RPX::MEQN <= 3) ? CLAW_SC_MINB : 2) sc2d_kernel(const ScArgs A)
 {
     constexpr int MEQN = RPX::MEQN, MW = RPX::MWAVES, NROE = RPX::NROE;
@@ -339,6 +345,8 @@ __global__ void __launch_bounds__(NT, (RPX::MEQN <= 3) ? CLAW_SC_MINB : 2) sc2d_
     const bool ycol = (ic >= 0) && (ic <= A.mx + 1);
     const int j0 = 1 + blockIdx.y * A.rows_per_cta;
     const int j1 = min(j0 + A.rows_per_cta, A.my + 1);
+    const long long po = D3 ? A.plane * (long long)(blockIdx.z + mbc - 1) : 0; // plane offset
+    const bool gp = D3 && (blockIdx.z == 0 || blockIdx.z == A.mz + 1);         // ghost plane
 
     double cfl = 0.0;
     double dtdy_c = A.dtdy, dtdy_p = A.dtdy; // dt/(dy capa) of rows c and c-1
@@ -355,7 +363,7 @@ __global__ void __launch_bounds__(NT, (RPX::MEQN <= 3) ? CLAW_SC_MINB : 2) sc2d_
     // cp.async staging: row k+1 is requested into the other half of a double-buffered
     // shared-memory row before row k is processed (index kk <-> cell i0-3+kk)
     {
-        const long long ro = (long long)A.pitch * (j0 - 3 + mbc - 1);
+        const long long ro = (long long)A.pitch * (j0 - 3 + mbc - 1) + po;
 #pragma unroll
         for (int m = 0; m < MEQN; m++) {
             cp_async8(&qs0[m * QS + t], &A.q[m * A.mstride + ro + cstage]);
@@ -365,7 +373,7 @@ __global__ void __launch_bounds__(NT, (RPX::MEQN <= 3) ? CLAW_SC_MINB : 2) sc2d_
     }
     int qb = 0;
     for (int k = j0 - 3; k <= j1 + 2; k++) {
-        const long long rowoff = (long long)A.pitch * (k + mbc - 1);
+        const long long rowoff = (long long)A.pitch * (k + mbc - 1) + po;
         cp_async_wait_all();
         __syncthreads();
         const double *qs = qs0 + qb * (MEQN * QS);
@@ -386,8 +394,8 @@ __global__ void __launch_bounds__(NT, (RPX::MEQN <= 3) ? CLAW_SC_MINB : 2) sc2d_
             w4[m] = qs[m * QS + t + 2]; // this thread's own column
             dx4[m] = dx3[m]; dx3[m] = dx2[m]; dx2[m] = dx1[m];
         }
-        const bool xfull = (k >= j0) && (k < j1);
-        const bool xcfl_only = (k == 0 && j0 == 1) || (k == A.my + 1 && j1 == A.my + 1);
+        const bool xfull = (k >= j0) && (k < j1) && !gp;
+        const bool xcfl_only = (k == 0 && j0 == 1) || (k == A.my + 1 && j1 == A.my + 1) || (gp && k >= j0 && k < j1);
         if (xfull || xcfl_only) {
             double dtdx_c = A.dtdx, dtdx_l = A.dtdx;
             if (CAPA) {
@@ -422,7 +430,7 @@ __global__ void __launch_bounds__(NT, (RPX::MEQN <= 3) ? CLAW_SC_MINB : 2) sc2d_
             if (c >= j0) {
                 const AuxCell nocell{nullptr, 0};
                 const bool AUXRP = (RPY::MAUX > 0);
-                const long long offc = (long long)A.pitch * (c + mbc - 1) + icl;
+                const long long offc = (long long)A.pitch * (c + mbc - 1) + icl + po;
                 const AuxCell ayc = AUXRP ? sc_aux(A, offc) : nocell;
                 const AuxCell aym = AUXRP ? sc_aux(A, offc - A.pitch) : nocell;
                 with_arith_fz([&](auto &ar) { RPY::solve(ar, A.rp, qr_prev, ql, aym, ayc, wave, s, amdq, apdq, roe); });
@@ -431,18 +439,18 @@ __global__ void __launch_bounds__(NT, (RPX::MEQN <= 3) ? CLAW_SC_MINB : 2) sc2d_
                     for (int mw = 0; mw < MW; mw++)
                         cfl = dmax2(dmax2(cfl, dtdy_c * s[mw]), -dtdy_p * s[mw]);
                 }
-                if (c < j1)
+                if (c < j1 && !gp)
                     with_arith_fz([&](auto &ar) { RPY::solve(ar, A.rp, ql, qr, ayc, ayc, wave, s, amdq2, apdq2, roe); });
                 // cell c-1 = k-3 is complete
                 const int jc = c - 1;
-                if (jc >= j0 && jc < j1 && col_out) {
+                if (jc >= j0 && jc < j1 && col_out && !gp) {
                     double dq[MEQN];
 #pragma unroll
                     for (int m = 0; m < MEQN; m++) {
                         double dqy = 0.0 - dtdy_p * (amdq[m] + apdq_prev[m] + amdq2_prev[m] + apdq2_prev[m]);
                         dq[m] = (0.0 + dx4[m]) + dqy;
                     }
-                    stage_store<MEQN>(A, (long long)A.pitch * (jc + mbc - 1) + icl, w1, dq);
+                    stage_store<MEQN>(A, (long long)A.pitch * (jc + mbc - 1) + icl + po, w1, dq);
                 }
             }
 #pragma unroll

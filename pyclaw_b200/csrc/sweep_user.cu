@@ -11,7 +11,8 @@
 //     solver.rp = pyclaw.riemann.from_header("my_rp.cuh", name="mine", meqn=..., mwaves=...)
 // A 3-D solver is `template <int IXYZ> struct RpUser3` with the 3-D interface of rp.cuh (rpn3 / rpt3 /
 // rptt3, e.g. examples/user_rp/rp_acoustics3d_user.cuh); with -DCLAWB200_USER_RP3 this unit also
-// instantiates the 3-D steps (step3.cuh) and the 3-D pointwise solve for it.  A header that defines
+// instantiates the 3-D steps (step3.cuh), the 3-D SharpClaw stage (sharpclaw3.cuh) and the 3-D
+// pointwise solve for it.  A header that defines
 // RpUser3 only is compiled with -DCLAWB200_USER_NO_RP as well (no 1-D / 2-D kernels).
 //     solver.rp = pyclaw.riemann.from_header("my_rp3.cuh", meqn=..., mwaves=..., ndims=(3,))
 // A library built without a user header answers CLAWB200_ERR_UNSUPPORTED for that id.
@@ -26,7 +27,7 @@ struct ScArgs;
 
 #ifdef CLAWB200_USER_RP_HEADER
 #include CLAWB200_USER_RP_HEADER
-#include "sharpclaw.cuh"
+#include "sharpclaw3.cuh"
 #include "step3.cuh"
 
 template <class RP>
@@ -39,12 +40,15 @@ static int user_shape(int *meqn, int *mwaves, int *maux)
 }
 
 #ifdef CLAWB200_USER_RP3
+int claw_sc3_user(bool old, const ScArgs &A, cudaStream_t st) { return sc_stage3_generic<RpUser3>(old, A, st); }
+
 int claw_step3_user(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
                     const double *aux, double dt, int idir, double *scratch, double *cfl_dev, cudaStream_t st)
 {
     return claw_step3_generic<RpUser3>(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
 }
 #else
+int claw_sc3_user(bool, const ScArgs &, cudaStream_t) { return none3(); }
 int claw_step3_user(const clawb200_problem *, int, double, const double *, double *, const double *, double, int,
                     double *, double *, cudaStream_t) { return none3(); }
 #endif
@@ -194,6 +198,7 @@ int claw_sc_user(int, bool, const ScArgs &, cudaStream_t) { return none12(); }
 #else // ---- no user solver in this build ----
 
 int claw_user_shape(int, int *, int *, int *) { return none(); }
+int claw_sc3_user(bool, const ScArgs &, cudaStream_t) { return none(); }
 int claw_step3_user(const clawb200_problem *, int, double, const double *, double *, const double *, double, int,
                     double *, double *, cudaStream_t) { return none(); }
 int claw_x_user(bool, const SweepArgs &, cudaStream_t) { return none(); }

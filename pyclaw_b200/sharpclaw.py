@@ -3,7 +3,8 @@
 Each Runge-Kutta stage is ONE kernel launch that reconstructs, solves the interface and
 in-cell Riemann problems, sums the fluctuations and applies the stage's linear
 combination (clawb200_sharpclaw_stage), where the reference calls ``sharpclaw2.flux2``
-and then combines full-field numpy temporaries (sharpclaw.py:172-206).
+and then combines full-field numpy temporaries (sharpclaw.py:172-206).  In 3-D a stage is
+two launches (clawb200_sharpclaw_stage3: x and y plane by plane, then z).
 """
 import ctypes
 
@@ -65,9 +66,15 @@ class SharpClawSolver(Solver):
 
     # ---- one dq evaluation fused with a stage update ----
     def _stage(self, q_buf, qa_buf, out_buf, mode, ca, cb, div, slot, dq_buf=None):
+        cfl = ctypes.c_void_p(self._cfl_dev.data_ptr() + 8 * slot)
+        if self.ndim == 3:
+            _lib.call("clawb200_sharpclaw_stage3", ctypes.byref(self._problem), int(self._mz), float(self._dz),
+                      _ptr(q_buf), _ptr(qa_buf), _ptr(out_buf), _ptr(dq_buf), self._aux_ptr, float(self.dt), mode,
+                      float(ca), float(cb), float(div), cfl, _stream())
+            return
         _lib.call("clawb200_sharpclaw_stage", ctypes.byref(self._problem), _ptr(q_buf), _ptr(qa_buf),
                   _ptr(out_buf), _ptr(dq_buf), self._aux_ptr, float(self.dt), mode, float(ca), float(cb),
-                  float(div), ctypes.c_void_p(self._cfl_dev.data_ptr() + 8 * slot), _stream())
+                  float(div), cfl, _stream())
 
     def _bcs_on(self, state, buf, t=None):
         """apply_q_bcs on an arbitrary padded buffer of this state's shape (the stage
@@ -222,6 +229,16 @@ class SharpClawSolver(Solver):
         if self.weno_order not in (5, 7, 9, 11, 13, 15, 17):
             # reconstruct.f90:111-113
             raise Exception("weno_order must be an odd number between 5 and 17 (inclusive).")
+        if self.ndim == 3:
+            # the 3-D stage (clawb200_sharpclaw_stage3) is WENO5 / tvd2 on the components of q
+            if self.weno_order != 5:
+                raise NotImplementedError("SharpClawSolver3D: weno_order must be 5 (orders 7-17 are 1-D / 2-D only)")
+            if self.char_decomp != 0:
+                raise NotImplementedError("SharpClawSolver3D: char_decomp must be 0 (the reconstruction is "
+                                          "component-wise in 3-D)")
+            if solution.state.mcapa >= 0:
+                raise NotImplementedError("SharpClawSolver3D: capacity functions (state.mcapa) are not supported "
+                                          "in 3-D, as in ClawSolver3D")
         if self.weno_order != 5:
             # weno7 .. weno17 (weno.f90:104-2425): table-driven kernels, component-wise only
             if self.lim_type != 2 or self.char_decomp != 0:
@@ -290,3 +307,13 @@ class SharpClawSolver2D(SharpClawSolver):
     def __init__(self, data=None):
         self.ndim = 2
         super(SharpClawSolver2D, self).__init__(data)
+
+
+class SharpClawSolver3D(SharpClawSolver):
+    """SharpClaw in 3-D: dq is flux1 summed over the x-, y- and z-slices (DESIGN.md §1), with
+    weno_order = 5 and lim_type 1 (tvd2), 2 (PyWENO weno5) or 3 (hand-written weno5), char_decomp = 0,
+    no capacity function.  The Courant number is the largest over the three directions, not their sum."""
+
+    def __init__(self, data=None):
+        self.ndim = 3
+        super(SharpClawSolver3D, self).__init__(data)
