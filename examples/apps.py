@@ -444,9 +444,52 @@ def advection3d(mx=32, my=32, mz=32, petsc=False, tfinal=1.0, dim_split=True, u=
     return _run(pyclaw, solver, state, tfinal, 10, outdir)
 
 
+def deformation_field(X, Y, Z):
+    """LeVeque's 3-D deformation flow on the unit cube (divergence free, zero normal velocity on the faces)"""
+    s2 = lambda a: np.sin(np.pi * a) ** 2
+    s = lambda a: np.sin(2 * np.pi * a)
+    return np.stack([2 * s2(X) * s(Y) * s(Z), -s(X) * s2(Y) * s(Z), -s(X) * s(Y) * s2(Z)])
+
+
+def transport3d(mx=32, my=32, mz=32, petsc=False, period=1.0, tfinal=None, dim_split=True, outdir=None,
+                solver_type='classic'):
+    """Conservative transport q_t + div(u q) = 0 of a cosine bell in LeVeque's 3-D deformation field on the
+    periodic unit cube (pyclaw.riemann.vc_advection_fwave_3d, solver.fwave = True).  A start_step hook
+    scales the field by cos(pi t / period), evaluated at the middle of each step, and rewrites state.aux
+    (ghost cells included): the flow reverses, so at t = period (the default tfinal) the exact solution
+    is the initial data again.  dim_split / solver_type select the split or unsplit classic step or
+    SharpClawSolver3D."""
+    pyclaw = _pc(petsc)
+    import torch
+    solver = _solver3d(pyclaw, solver_type, dim_split)
+    solver.rp = pyclaw.riemann.vc_advection_fwave_3d
+    solver.fwave = True
+    solver.mwaves, solver.limiters = 1, pyclaw.limiters.tvd.MC
+    for i in range(3):
+        solver.bc_lower[i] = solver.bc_upper[i] = pyclaw.BC.periodic
+        solver.aux_bc_lower[i] = solver.aux_bc_upper[i] = pyclaw.BC.periodic
+    grid = pyclaw.Grid([pyclaw.Dimension('x', 0.0, 1.0, mx), pyclaw.Dimension('y', 0.0, 1.0, my),
+                        pyclaw.Dimension('z', 0.0, 1.0, mz)])
+    state = pyclaw.State(grid, 1, 3)
+    grid.compute_c_center()
+    X, Y, Z = grid._c_center
+    aux0 = deformation_field(X, Y, Z)
+    state.aux = aux0
+    r = np.sqrt((X - 0.35) ** 2 + (Y - 0.35) ** 2 + (Z - 0.35) ** 2)
+    state.q[0] = 0.5 * (1.0 + np.cos(np.pi * np.minimum(r / 0.2, 1.0)))
+    field = torch.as_tensor(np.ascontiguousarray(aux0), device=state.aux.device)
+
+    def reverse_flow(solver, solution):                      # the script's b4step
+        st = solution.states[0]
+        st.aux[...] = field * float(np.cos(np.pi * (solution.t + 0.5 * solver.dt) / period))
+        solver.apply_aux_bcs(st)
+    solver.start_step = reverse_flow
+    return _run(pyclaw, solver, state, period if tfinal is None else tfinal, 10, outdir)
+
+
 APPS = {f.__name__: f for f in (acoustics1d, acoustics2d, vc_acoustics2d, shockbubble, shallow1d, shallow2d,
                                 shallow_sphere, stegoton, psystem, acoustics3d, burgers, wcblast,
-                                vc_advection1d, annulus, euler3d, advection3d)}
+                                vc_advection1d, annulus, euler3d, advection3d, transport3d)}
 
 
 def main(argv):

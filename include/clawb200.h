@@ -67,6 +67,9 @@ extern "C" {
 #define CLAWB200_RP_ADVECTION3D 14   /* rpn3/rpt3/rptt3_advection; params {u, v, w}; meqn = mwaves = 1 */
 #define CLAWB200_RP_EULER3D 15       /* rpn3/rpt3/rptt3_euler, Roe + Harten-Hyman entropy fix; params {gamma,
                                         gamma1}; q = (rho, rho u, rho v, rho w, E), meqn 5, mwaves 3 */
+#define CLAWB200_RP_ADVECTION3D_VC_FWAVE 16 /* conservative transport q_t + div(u q) = 0, f-waves (the 3-D
+                                               f-wave step, sign(s) correction); aux {u, v, w} per cell,
+                                               maux >= 3; meqn = mwaves = 1 */
 
 /* Boundary condition ids = pyclaw.BC (src/pyclaw/solver.py:17-23) */
 #define CLAWB200_BC_CUSTOM 0

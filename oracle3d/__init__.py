@@ -1,5 +1,5 @@
-"""CPU restatement of the 3-D classic steps for the aux-free 3-D solvers and of SharpClaw in 3-D (flux3,
-sc_flux3) -- TEST INFRASTRUCTURE ONLY (never imported by pyclaw_b200/).  ctypes driver of
+"""CPU restatement of the 3-D classic steps for the 3-D solvers other than vc-acoustics and of SharpClaw in
+3-D (flux3, sc_flux3) -- TEST INFRASTRUCTURE ONLY (never imported by pyclaw_b200/).  ctypes driver of
 oracle3d/liboracle3d.so (claw_oracle3d.c), with the array conventions of oracle/pyclaw_oracle.py:
 Fortran-ordered q[m, i, j, k]."""
 import ctypes
@@ -13,6 +13,7 @@ _LIB = None
 
 RP_ADVECTION3D, RP_EULER3D = 14, 15  # 3-D advection {u, v, w}; 3-D Euler, Roe + entropy fix {gamma, gamma1}
 RP_ACOUSTICS3D_VC = 8                # 3-D acoustics, aux = {impedance, sound speed} (SharpClaw only here)
+RP_ADVECTION3D_VC_FWAVE = 16         # 3-D f-wave transport, aux = {u, v, w} per cell
 WENO_PYWENO_F32, WENO_PYWENO_F64, WENO_OLD, RECON_TVD2 = 0, 1, 2, 4  # as oracle/pyclaw_oracle.py
 
 _dp = ctypes.POINTER(ctypes.c_double)
@@ -36,6 +37,13 @@ def lib():
         L.oracle3d_step3ds.argtypes = [i, _dp, i, i, i, i, i, i, _dp, _dp, d, d, d, d, _ip, _ip, i]
         L.oracle3d_step3.restype = d
         L.oracle3d_step3.argtypes = [i, _dp, i, i, i, i, i, i, _dp, _dp, d, d, d, d, _ip, _ip]
+        L.oracle3d_step3ds_aux.restype = d
+        L.oracle3d_step3ds_aux.argtypes = [i, _dp, i, i, i, i, i, i, _dp, _dp, _dp, i, d, d, d, d, _ip, _ip, i]
+        L.oracle3d_step3_aux.restype = d
+        L.oracle3d_step3_aux.argtypes = [i, _dp, i, i, i, i, i, i, _dp, _dp, _dp, i, d, d, d, d, _ip, _ip]
+        L.oracle3d_rp_point_aux.restype = None
+        L.oracle3d_rp_point_aux.argtypes = [i, _dp, i, i, i, i, ctypes.c_longlong, _dp, _dp, _dp, _dp, _dp, _dp, _dp,
+                                            _dp, i, i, i, _dp, _dp, _dp, _dp]
         L.oracle3d_sc_flux1.restype = d
         L.oracle3d_sc_flux1.argtypes = [i, _dp, i, i, i, i, i, _dp, _dp, _dp, d, d, i, i, _ip]
         L.oracle3d_sc_flux3.restype = d
@@ -63,24 +71,36 @@ def _check(cfl):
     return cfl
 
 
-def step3ds(rp_id, rp_params, mbc, mx, my, mz, qold, qnew, dx, dy, dz, dt, method, mthlim, idir):
-    """classic3.step3ds: one directional sweep (idir = 1, 2, 3); qnew (== qold on entry) updated in place."""
+def _aux(aux):
+    """(pointer, maux) of an optional aux array [maux, mx+2mbc, my+2mbc, mz+2mbc] (Fortran order)"""
+    if aux is None:
+        return ctypes.cast(None, _dp), 0
+    assert aux.flags["F_CONTIGUOUS"] and aux.dtype == np.float64
+    return _p(aux), aux.shape[0]
+
+
+def step3ds(rp_id, rp_params, mbc, mx, my, mz, qold, qnew, dx, dy, dz, dt, method, mthlim, idir, aux=None):
+    """classic3.step3ds: one directional sweep (idir = 1, 2, 3); qnew (== qold on entry) updated in place.
+    aux [maux, ...] (Fortran order, ghost cells filled) for the solvers that read aux data."""
     method = np.ascontiguousarray(method, dtype=np.int32)
     mthlim = np.ascontiguousarray(mthlim, dtype=np.int32)
     assert qold.flags["F_CONTIGUOUS"] and qnew.flags["F_CONTIGUOUS"]
-    return _check(lib().oracle3d_step3ds(rp_id, _p(_params(rp_params)), qold.shape[0], len(mthlim), mbc, mx, my, mz,
-                                         _p(qold), _p(qnew), dx, dy, dz, dt, method.ctypes.data_as(_ip),
-                                         mthlim.ctypes.data_as(_ip), idir))
+    a, maux = _aux(aux)
+    return _check(lib().oracle3d_step3ds_aux(rp_id, _p(_params(rp_params)), qold.shape[0], len(mthlim), mbc, mx, my,
+                                             mz, _p(qold), _p(qnew), a, maux, dx, dy, dz, dt,
+                                             method.ctypes.data_as(_ip), mthlim.ctypes.data_as(_ip), idir))
 
 
-def step3(rp_id, rp_params, mbc, mx, my, mz, qold, qnew, dx, dy, dz, dt, method, mthlim):
-    """classic3.step3 (step3.f + flux3.f with rpt3 / rptt3); qnew (== qold on entry) updated in place."""
+def step3(rp_id, rp_params, mbc, mx, my, mz, qold, qnew, dx, dy, dz, dt, method, mthlim, aux=None):
+    """classic3.step3 (step3.f + flux3.f with rpt3 / rptt3); qnew (== qold on entry) updated in place.
+    aux [maux, ...] (Fortran order, ghost cells filled) for the solvers that read aux data."""
     method = np.ascontiguousarray(method, dtype=np.int32)
     mthlim = np.ascontiguousarray(mthlim, dtype=np.int32)
     assert qold.flags["F_CONTIGUOUS"] and qnew.flags["F_CONTIGUOUS"]
-    return _check(lib().oracle3d_step3(rp_id, _p(_params(rp_params)), qold.shape[0], len(mthlim), mbc, mx, my, mz,
-                                       _p(qold), _p(qnew), dx, dy, dz, dt, method.ctypes.data_as(_ip),
-                                       mthlim.ctypes.data_as(_ip)))
+    a, maux = _aux(aux)
+    return _check(lib().oracle3d_step3_aux(rp_id, _p(_params(rp_params)), qold.shape[0], len(mthlim), mbc, mx, my, mz,
+                                           _p(qold), _p(qnew), a, maux, dx, dy, dz, dt, method.ctypes.data_as(_ip),
+                                           mthlim.ctypes.data_as(_ip)))
 
 
 def rp_point(rp_id, rp_params, ixyz, mwaves, ql, qr):
@@ -107,6 +127,35 @@ def rp3_transverse(rp_id, rp_params, ixyz, icoor, ql, qr, asdq):
     null = ctypes.cast(None, _dp)
     lib().oracle3d_rp_point(rp_id, _p(_params(rp_params)), ixyz, meqn, 1, n, _p(ql), _p(qr), null, null, null, null,
                             icoor, _p(asdq), _p(bm), _p(bp))
+    return bm, bp
+
+
+def rp_point_aux(rp_id, rp_params, ixyz, mwaves, ql, qr, auxl, auxr):
+    """rpn3 of a solver with aux data on n interfaces ql | qr ([meqn, n]); auxl / auxr [maux, n] are the
+    cells left / right of each interface.  Returns (wave[meqn, mwaves, n], s[mwaves, n], amdq, apdq)."""
+    ql, qr = (np.ascontiguousarray(a, dtype=np.float64) for a in (ql, qr))
+    auxl, auxr = (np.ascontiguousarray(a, dtype=np.float64) for a in (auxl, auxr))
+    meqn, n = ql.shape
+    wave, s = np.zeros((meqn, mwaves, n)), np.zeros((mwaves, n))
+    amdq, apdq = np.zeros((meqn, n)), np.zeros((meqn, n))
+    null = ctypes.cast(None, _dp)
+    lib().oracle3d_rp_point_aux(rp_id, _p(_params(rp_params)), ixyz, meqn, mwaves, auxl.shape[0], n, _p(ql), _p(qr),
+                                _p(auxl), _p(auxr), _p(wave), _p(s), _p(amdq), _p(apdq), 0, 0, 0, null, null, null, null)
+    return wave, s, amdq, apdq
+
+
+def rp3_transverse_aux(rp_id, rp_params, ixyz, icoor, imp, impt, aux9, asdq):
+    """rpt3 (impt = 0) or rptt3 (impt = 1, 2) of a solver with aux data on n fluctuations asdq [meqn, n]
+    entering a cell on side imp = 1 | 2 of their interface: aux9 [maux, 3, 3, n] holds the 3x3 cells around
+    that cell, [ma, e+1, f+1] at the offset e / f in the y-like / z-like direction.  Returns (bm, bp)."""
+    asdq = np.ascontiguousarray(asdq, dtype=np.float64)
+    aux9 = np.ascontiguousarray(aux9, dtype=np.float64)
+    meqn, n = asdq.shape
+    bm, bp = np.zeros((meqn, n)), np.zeros((meqn, n))
+    null = ctypes.cast(None, _dp)
+    q = np.zeros((meqn, n))
+    lib().oracle3d_rp_point_aux(rp_id, _p(_params(rp_params)), ixyz, meqn, 1, aux9.shape[0], n, _p(q), _p(q), null,
+                                null, null, null, null, null, icoor, imp, impt, _p(aux9), _p(asdq), _p(bm), _p(bp))
     return bm, bp
 
 

@@ -1,6 +1,6 @@
 /*
- * claw_oracle3d.c -- CPU restatement of the 3-D classic steps for the 3-D Riemann solvers without
- * aux data (TEST INFRASTRUCTURE ONLY, never linked into the product), next to oracle/claw_oracle.c,
+ * claw_oracle3d.c -- CPU restatement of the 3-D classic steps for the 3-D Riemann solvers other
+ * than vc-acoustics (TEST INFRASTRUCTURE ONLY, never linked into the product), next to oracle/claw_oracle.c,
  * which holds the same steps for the variable-coefficient acoustics solver:
  *   src/fortran/3d/classic/step3ds.f:2-376 with flux3.f:176-237 (dimensional splitting)
  *   src/fortran/3d/classic/step3.f:2-594 with flux3.f:5-595 (unsplit, method(3) = 0, 10, 11, 20, 21, 22)
@@ -9,7 +9,8 @@
  * limiter, philim), with the rp_id switch of this file's solvers.  The solvers live in the external
  * clawpack/riemann repository (un-vendored): rpn3 / rpt3 / rptt3_advection and rpn3 / rpt3 /
  * rptt3_euler (Roe + Harten-Hyman entropy fix), restated from the published algorithm (LeVeque 2002,
- * sec. 15.3 and 18.8), parity unpinned.
+ * sec. 15.3 and 18.8), parity unpinned.  The f-wave transport solver (aux = {u, v, w} per cell) runs the
+ * 3-D f-wave step: flux3.f with the delta of flux2fw.f (sign(s) leads the correction flux), DESIGN.md §1.
  * Strict IEEE double: compiled without FMA contraction (oracle3d/Makefile).
  */
 #include <math.h>
@@ -18,10 +19,17 @@
 
 #define RP_ADVECTION3D 14 /* p[0..2] = u, v, w          */
 #define RP_EULER3D 15     /* p[0] = gamma, p[1] = gamma1 */
+#define RP_ADVECTION3D_VC_FWAVE 16 /* aux = u, v, w of each cell; f-waves */
+#define RP_IS_FWAVE3(id) ((id) == RP_ADVECTION3D_VC_FWAVE)
 
+/* aux1d (maux, slice): the aux data of the slice's cells; aux9 (maux, 3, 3, slice): the 3x3 cells
+   around each cell of the slice in the plane normal to it, aux9[ma + maux * ((e+1) + 3 * (f+1))] at the
+   offset e / f in the y-like / z-like direction.  Both NULL for the solvers without aux data. */
 typedef struct {
     int rp_id;
     double p[8];
+    int maux;
+    const double *aux1d, *aux9;
 } rp_ctx3;
 
 static inline double dmax2(double a, double b) { return (a > b) ? a : b; }
@@ -60,6 +68,46 @@ static void rpt3_advection(const rp_ctx3 *c, int ixyz, int icoor, int mbc, int m
         Q2(bmasdq, 0, i) = dmin2(st, 0.0) * Q2(asdq, 0, i);
         Q2(bpasdq, 0, i) = dmax2(st, 0.0) * Q2(asdq, 0, i);
     }
+}
+
+/* ---- the f-wave transport solver (rpn3 / rpt3 / rptt3; rp.cuh RpVcAdvectionFwave3) ---- */
+/* interface i between cell i-1 (qr, auxr) and cell i (ql, auxl): ul = u_d(i-1), ur = u_d(i);
+   fwave = ur q(i) - ul q(i-1), s = (ul + ur) / 2, the whole f-wave to the side s points to */
+static void rpn3_vc_fwave(int ixyz, int mbc, int mx, int maux, const double *ql, const double *qr,
+                          const double *auxl, const double *auxr, double *wave, double *s, double *amdq,
+                          double *apdq)
+{
+    const int meqn = 1, mwaves = 1, d = rp3_dir(ixyz, 1) - 1;
+    for (int i = 2 - mbc; i <= mx + mbc; i++) {
+        double ul = auxr[d + maux * IX(i - 1)], ur = auxl[d + maux * IX(i)];
+        double fwave = (ur * Q2(ql, 0, i)) - (ul * Q2(qr, 0, i - 1));
+        double sp = 0.5 * (ul + ur);
+        WV(0, 0, i) = fwave;
+        SP(0, i) = sp;
+        if (sp > 0.0) { Q2(amdq, 0, i) = 0.0; Q2(apdq, 0, i) = fwave; }
+        else if (sp < 0.0) { Q2(amdq, 0, i) = fwave; Q2(apdq, 0, i) = 0.0; }
+        else { Q2(amdq, 0, i) = 0.5 * fwave; Q2(apdq, 0, i) = 0.5 * fwave; }
+    }
+}
+
+/* rpt3 (impt = 0) / rptt3 (impt = 1, 2): asdq of interface i enters cell i-1 (imp = 1) or i (imp = 2); split
+   along the line of three cells in direction icoor through that cell (rpt3) or through the cell one step
+   down (impt = 1) / up (impt = 2) in the other transverse direction (rptt3) */
+static void rpt3_vc_fwave(const rp_ctx3 *c, int ixyz, int icoor, int imp, int impt, int mbc, int mx,
+                          const double *asdq, double *bmasdq, double *bpasdq)
+{
+    const int meqn = 1, maux = c->maux, ma = rp3_dir(ixyz, icoor) - 1;
+    const int de = (icoor == 2) ? 1 : 0, df = (icoor == 3) ? 1 : 0;
+    const int off = (impt == 1) ? -1 : 1;
+    const int e0 = (impt != 0 && icoor == 3) ? off : 0, f0 = (impt != 0 && icoor == 2) ? off : 0;
+#define A9(cell, e, f) c->aux9[ma + maux * (((e) + 1) + 3 * ((f) + 1)) + (size_t)9 * maux * IX(cell)]
+    for (int i = 2 - mbc; i <= mx + mbc; i++) {
+        const int cell = (imp == 1) ? i - 1 : i;
+        double vm = A9(cell, e0 - de, f0 - df), v0 = A9(cell, e0, f0), vp = A9(cell, e0 + de, f0 + df);
+        Q2(bmasdq, 0, i) = dmin2(0.5 * (vm + v0), 0.0) * Q2(asdq, 0, i);
+        Q2(bpasdq, 0, i) = dmax2(0.5 * (v0 + vp), 0.0) * Q2(asdq, 0, i);
+    }
+#undef A9
 }
 
 /* ---- rpn3 / rpt3 / rptt3_euler ---- */
@@ -183,16 +231,26 @@ static void rpn3(const rp_ctx3 *c, int ixyz, int mbc, int mx, const double *ql, 
                  double *s, double *amdq, double *apdq)
 {
     if (c->rp_id == RP_EULER3D) rpn3_euler(c, ixyz, mbc, mx, ql, qr, wave, s, amdq, apdq);
+    else if (c->rp_id == RP_ADVECTION3D_VC_FWAVE)
+        rpn3_vc_fwave(ixyz, mbc, mx, c->maux, ql, qr, c->aux1d, c->aux1d, wave, s, amdq, apdq);
     else rpn3_advection(c, ixyz, mbc, mx, ql, qr, wave, s, amdq, apdq);
 }
-/* rpt3 and rptt3: neither solver reads aux data, so neither depends on imp / impt */
-static void rpt3(const rp_ctx3 *c, int ixyz, int icoor, int mbc, int mx, const double *q1d, const double *asdq,
-                 double *bmasdq, double *bpasdq)
+/* rpt3 (impt = 0) and rptt3 (impt = 1, 2): advection and Euler read no aux data, so they depend on
+   neither imp nor impt */
+static void rpt3(const rp_ctx3 *c, int ixyz, int icoor, int imp, int impt, int mbc, int mx, const double *q1d,
+                 const double *asdq, double *bmasdq, double *bpasdq)
 {
     if (c->rp_id == RP_EULER3D) rpt3_euler(c, ixyz, icoor, mbc, mx, q1d, asdq, bmasdq, bpasdq);
+    else if (c->rp_id == RP_ADVECTION3D_VC_FWAVE) rpt3_vc_fwave(c, ixyz, icoor, imp, impt, mbc, mx, asdq, bmasdq, bpasdq);
     else rpt3_advection(c, ixyz, icoor, mbc, mx, asdq, bmasdq, bpasdq);
 }
-static int known(int rp_id) { return rp_id == RP_ADVECTION3D || rp_id == RP_EULER3D; }
+static int known(int rp_id) { return rp_id == RP_ADVECTION3D || rp_id == RP_EULER3D || rp_id == RP_ADVECTION3D_VC_FWAVE; }
+/* the f-wave transport solver reads aux {u, v, w}, the 3x3 neighbourhood of each cell included */
+static int aux_ok(int rp_id, const double *aux, int maux, int mbc)
+{
+    if (rp_id != RP_ADVECTION3D_VC_FWAVE) return 1;
+    return aux != NULL && maux >= 3 && mbc >= 2;
+}
 
 /* ---- limiter.f / philim.f (as oracle/claw_oracle.c) ---- */
 static double philim(double a, double b, int meth)
@@ -258,29 +316,61 @@ static double flux3_normal(const rp_ctx3 *c, int ixyz, int meqn, int mwaves, int
     for (int i = 2 - mbc; i <= mx + mbc; i++) {
         double dtdxave = 0.5 * (dtdx + dtdx);
         for (int m = 0; m < meqn; m++) Q2(cqxx, m, i) = 0.0;
-        for (int mw = 0; mw < mwaves; mw++)
+        for (int mw = 0; mw < mwaves; mw++) {
+            /* flux2fw.f:151-152: an f-wave solver leads with sign(s) */
+            double lead = RP_IS_FWAVE3(c->rp_id) ? copysign(1.0, SP(mw, i)) : fabs(SP(mw, i));
             for (int m = 0; m < meqn; m++)
-                Q2(cqxx, m, i) = Q2(cqxx, m, i) + 0.5 * fabs(SP(mw, i)) * (1.0 - fabs(SP(mw, i)) * dtdxave) * WV(m, mw, i);
+                Q2(cqxx, m, i) = Q2(cqxx, m, i) + 0.5 * lead * (1.0 - fabs(SP(mw, i)) * dtdxave) * WV(m, mw, i);
+        }
         for (int m = 0; m < meqn; m++) Q2(fadd, m, i) = Q2(fadd, m, i) + Q2(cqxx, m, i);
     }
     return cfl1d;
+}
+
+/* the aux data of one slice in direction d (cells l = 1-mbc .. len[d]+mbc at the transverse position idx):
+   aux1d (maux, n) and, where the neighbours exist, the 3x3 neighbourhood aux9 (maux, 3, 3, n) */
+static void slice_aux(const double *aux, int maux, int mbc, int mx, int my, int mz, int d, const int *idx,
+                      double *aux1d, double *aux9)
+{
+    const size_t NXs = mx + 2 * mbc, NYs = my + 2 * mbc;
+    const int len[3] = {mx, my, mz}, e = (d + 1) % 3, f = (d + 2) % 3;
+    for (int l = 1 - mbc; l <= len[d] + mbc; l++)
+        for (int fo = -1; fo <= 1; fo++)
+            for (int eo = -1; eo <= 1; eo++) {
+                int p[3] = {idx[0], idx[1], idx[2]};
+                p[d] = l; p[e] += eo; p[f] += fo;
+                if (p[e] < 1 - mbc || p[e] > len[e] + mbc || p[f] < 1 - mbc || p[f] > len[f] + mbc) continue;
+                const size_t off = ((p[0] + mbc - 1) + NXs * ((p[1] + mbc - 1) + NYs * (p[2] + mbc - 1)));
+                for (int ma = 0; ma < maux; ma++) {
+                    double v = aux[ma + (size_t)maux * off];
+                    aux9[ma + maux * ((eo + 1) + 3 * (fo + 1)) + (size_t)9 * maux * IX(l)] = v;
+                    if (eo == 0 && fo == 0) aux1d[ma + maux * IX(l)] = v;
+                }
+            }
 }
 
 /* ------------------------------------------------------------------------- */
 /* step3ds.f:2-376 (method(3) < 0), idir = 1, 2, 3; sweeps cover one ghost     */
 /* layer of the other two directions.  q(meqn, 1-mbc:mx+mbc, ..., 1-mbc:mz+mbc) */
 /* ------------------------------------------------------------------------- */
-double oracle3d_step3ds(int rp_id, const double *rp_params, int meqn, int mwaves, int mbc, int mx, int my, int mz,
-                        const double *qold, double *qnew, double dx, double dy, double dz, double dt,
-                        const int *method, const int *mthlim, int idir)
+/* aux (maux, 1-mbc:mx+mbc, ...) or NULL: the f-wave transport solver needs it */
+double oracle3d_step3ds_aux(int rp_id, const double *rp_params, int meqn, int mwaves, int mbc, int mx, int my, int mz,
+                            const double *qold, double *qnew, const double *aux, int maux, double dx, double dy,
+                            double dz, double dt, const int *method, const int *mthlim, int idir)
 {
-    if (!known(rp_id) || method[5] > 0) return -1.0;
-    rp_ctx3 c;
+    if (!known(rp_id) || method[5] > 0 || !aux_ok(rp_id, aux, maux, mbc)) return -1.0;
+    rp_ctx3 c = {0};
     c.rp_id = rp_id;
     memcpy(c.p, rp_params, 8 * sizeof(double));
     int maxm = mx > my ? mx : my;
     if (mz > maxm) maxm = mz;
     const int n = maxm + 2 * mbc;
+    const int ma = aux ? maux : 0;
+    double *aux1d = (double *)calloc((size_t)n * (ma > 0 ? ma : 1), sizeof(double));
+    double *aux9 = (double *)calloc((size_t)n * 9 * (ma > 0 ? ma : 1), sizeof(double));
+    c.maux = ma;
+    c.aux1d = aux1d;
+    c.aux9 = aux9;
     double *v[7];
     for (int a = 0; a < 7; a++) v[a] = (double *)calloc((size_t)n * meqn * mwaves, sizeof(double));
     double *q1d = v[0], *wave = v[1], *s = v[2], *amdq = v[3], *apdq = v[4], *qadd = v[5], *fadd = v[6];
@@ -299,6 +389,7 @@ double oracle3d_step3ds(int rp_id, const double *rp_params, int meqn, int mwaves
                 idx[d] = l;
                 for (int m = 0; m < meqn; m++) Q2(q1d, m, l) = Q4(qold, m, idx[0], idx[1], idx[2]);
             }
+            if (ma > 0) slice_aux(aux, ma, mbc, mx, my, mz, d, idx, aux1d, aux9);
             double cfl1d = flux3_normal(&c, idir, meqn, mwaves, mbc, len[d], q1d, dtd[d], method[1], mthlim, wave, s,
                                         amdq, apdq, cqxx, qadd, fadd);
             cfl = dmax2(cfl, cfl1d);
@@ -311,8 +402,16 @@ double oracle3d_step3ds(int rp_id, const double *rp_params, int meqn, int mwaves
             }
         }
     for (int a = 0; a < 7; a++) free(v[a]);
-    free(cqxx);
+    free(cqxx); free(aux1d); free(aux9);
     return cfl;
+}
+
+double oracle3d_step3ds(int rp_id, const double *rp_params, int meqn, int mwaves, int mbc, int mx, int my, int mz,
+                        const double *qold, double *qnew, double dx, double dy, double dz, double dt,
+                        const int *method, const int *mthlim, int idir)
+{
+    return oracle3d_step3ds_aux(rp_id, rp_params, meqn, mwaves, mbc, mx, my, mz, qold, qnew, NULL, 0, dx, dy, dz, dt,
+                                method, mthlim, idir);
 }
 
 /* gadd / hadd (meqn, 2, -1:1, 1-mbc:maxm+mbc): k = 1..2, j = -1..1 */
@@ -343,16 +442,16 @@ static double flux3(const rp_ctx3 *c, int ixyz, int meqn, int mwaves, int mbc, i
                                 cqxx, qadd, fadd);
     if (m3 <= 0) return cfl1d;
 
-#define RPT3(icoor, as, bm, bp) rpt3(c, ixyz, icoor, mbc, mx, q1d, as, bm, bp)
-    RPT3(2, amdq, bmamdq, bpamdq);
-    RPT3(2, apdq, bmapdq, bpapdq);
-    RPT3(3, amdq, cmamdq, cpamdq);
-    RPT3(3, apdq, cmapdq, cpapdq);
-    if (m3 == 2) { /* cqxx split with imp = 1 and imp = 2 (flux3.f:262-283): the same split here */
-        RPT3(2, cqxx, bmcqxxm, bpcqxxm);
-        RPT3(2, cqxx, bmcqxxp, bpcqxxp);
-        RPT3(3, cqxx, cmcqxxm, cpcqxxm);
-        RPT3(3, cqxx, cmcqxxp, cpcqxxp);
+#define RPT3(icoor, imp, impt, as, bm, bp) rpt3(c, ixyz, icoor, imp, impt, mbc, mx, q1d, as, bm, bp)
+    RPT3(2, 1, 0, amdq, bmamdq, bpamdq);
+    RPT3(2, 2, 0, apdq, bmapdq, bpapdq);
+    RPT3(3, 1, 0, amdq, cmamdq, cpamdq);
+    RPT3(3, 2, 0, apdq, cmapdq, cpapdq);
+    if (m3 == 2) { /* cqxx split with imp = 1 and imp = 2 (flux3.f:262-283) */
+        RPT3(2, 1, 0, cqxx, bmcqxxm, bpcqxxm);
+        RPT3(2, 2, 0, cqxx, bmcqxxp, bpcqxxp);
+        RPT3(3, 1, 0, cqxx, cmcqxxm, cpcqxxm);
+        RPT3(3, 2, 0, cqxx, cmcqxxp, cpcqxxp);
     }
     /* ---- G fluxes (y-like direction) ---- */
     if (m4 == 1) {
@@ -371,10 +470,10 @@ static double flux3(const rp_ctx3 *c, int ixyz, int meqn, int mwaves, int mbc, i
             }
     }
     if (m4 > 0) { /* rptt3 */
-        RPT3(2, cpapdq2, bmcpapdq, bpcpapdq);
-        RPT3(2, cpamdq2, bmcpamdq, bpcpamdq);
-        RPT3(2, cmapdq2, bmcmapdq, bpcmapdq);
-        RPT3(2, cmamdq2, bmcmamdq, bpcmamdq);
+        RPT3(2, 2, 2, cpapdq2, bmcpapdq, bpcpapdq);
+        RPT3(2, 1, 2, cpamdq2, bmcpamdq, bpcpamdq);
+        RPT3(2, 2, 1, cmapdq2, bmcmapdq, bpcmapdq);
+        RPT3(2, 1, 1, cmamdq2, bmcmamdq, bpcmamdq);
     }
     const double sixth = 1.0 / 6.0;
     for (int i = 1; i <= mx + 1; i++)
@@ -416,10 +515,10 @@ static double flux3(const rp_ctx3 *c, int ixyz, int meqn, int mwaves, int mbc, i
             }
     }
     if (m4 > 0) { /* rptt3 */
-        RPT3(3, bpapdq, bmcpapdq, bpcpapdq);
-        RPT3(3, bpamdq, bmcpamdq, bpcpamdq);
-        RPT3(3, bmapdq, bmcmapdq, bpcmapdq);
-        RPT3(3, bmamdq, bmcmamdq, bpcmamdq);
+        RPT3(3, 2, 2, bpapdq, bmcpapdq, bpcpapdq);
+        RPT3(3, 1, 2, bpamdq, bmcpamdq, bpcpamdq);
+        RPT3(3, 2, 1, bmapdq, bmcmapdq, bpcmapdq);
+        RPT3(3, 1, 1, bmamdq, bmcmamdq, bpcmamdq);
     }
     for (int i = 1; i <= mx + 1; i++)
         for (int m = 0; m < meqn; m++) {
@@ -454,17 +553,23 @@ static double flux3(const rp_ctx3 *c, int ixyz, int meqn, int mwaves, int mbc, i
 }
 
 /* step3.f:2-594.  qnew == qold on entry; q(meqn, 1-mbc:mx+mbc, ...). */
-double oracle3d_step3(int rp_id, const double *rp_params, int meqn, int mwaves, int mbc, int mx, int my, int mz,
-                      const double *qold, double *qnew, double dx, double dy, double dz, double dt,
-                      const int *method, const int *mthlim)
+double oracle3d_step3_aux(int rp_id, const double *rp_params, int meqn, int mwaves, int mbc, int mx, int my, int mz,
+                          const double *qold, double *qnew, const double *aux, int maux, double dx, double dy,
+                          double dz, double dt, const int *method, const int *mthlim)
 {
-    if (!known(rp_id) || method[5] > 0) return -1.0;
-    rp_ctx3 c;
+    if (!known(rp_id) || method[5] > 0 || !aux_ok(rp_id, aux, maux, mbc)) return -1.0;
+    rp_ctx3 c = {0};
     c.rp_id = rp_id;
     memcpy(c.p, rp_params, 8 * sizeof(double));
     int maxm = mx > my ? mx : my;
     if (mz > maxm) maxm = mz;
     const int n1d = maxm + 2 * mbc;
+    const int ma = aux ? maux : 0;
+    double *aux1d = (double *)calloc((size_t)n1d * (ma > 0 ? ma : 1), sizeof(double));
+    double *aux9 = (double *)calloc((size_t)n1d * 9 * (ma > 0 ? ma : 1), sizeof(double));
+    c.maux = ma;
+    c.aux1d = aux1d;
+    c.aux9 = aux9;
     const size_t nm = (size_t)n1d * meqn;
     double *q1d = (double *)calloc(nm, sizeof(double)), *qadd = (double *)calloc(nm, sizeof(double));
     double *fadd = (double *)calloc(nm, sizeof(double));
@@ -488,6 +593,7 @@ double oracle3d_step3(int rp_id, const double *rp_params, int meqn, int mwaves, 
                     idx[d] = l;
                     for (int m = 0; m < meqn; m++) Q2(q1d, m, l) = Q4(qold, m, idx[0], idx[1], idx[2]);
                 }
+                if (ma > 0) slice_aux(aux, ma, mbc, mx, my, mz, d, idx, aux1d, aux9);
                 double cfl1d = flux3(&c, d + 1, meqn, mwaves, mbc, len[d], n1d, q1d, dtd[d], dtde, dtdf, method, mthlim,
                                      wave, s, qadd, fadd, gadd, hadd, v);
                 cfl = dmax2(cfl, cfl1d);
@@ -521,9 +627,17 @@ double oracle3d_step3(int rp_id, const double *rp_params, int meqn, int mwaves, 
                     }
             }
     }
-    free(q1d); free(qadd); free(fadd); free(gadd); free(hadd); free(wave); free(s);
+    free(q1d); free(qadd); free(fadd); free(gadd); free(hadd); free(wave); free(s); free(aux1d); free(aux9);
     for (int a = 0; a < 31; a++) free(v[a]);
     return cfl;
+}
+
+double oracle3d_step3(int rp_id, const double *rp_params, int meqn, int mwaves, int mbc, int mx, int my, int mz,
+                      const double *qold, double *qnew, double dx, double dy, double dz, double dt,
+                      const int *method, const int *mthlim)
+{
+    return oracle3d_step3_aux(rp_id, rp_params, meqn, mwaves, mbc, mx, my, mz, qold, qnew, NULL, 0, dx, dy, dz, dt,
+                              method, mthlim);
 }
 #undef Q4
 
@@ -533,14 +647,24 @@ double oracle3d_step3(int rp_id, const double *rp_params, int meqn, int mwaves, 
 /* mx = 1, interface i = 1).  asdq == NULL: rpn3 into wave, s, amdq, apdq;     */
 /* otherwise rpt3 / rptt3 of asdq in direction icoor into bm, bp.              */
 /* ------------------------------------------------------------------------- */
-void oracle3d_rp_point(int rp_id, const double *rp_params, int ixyz, int meqn, int mwaves, long long n,
-                       const double *ql, const double *qr, double *wave_o, double *s_o, double *amdq_o,
-                       double *apdq_o, int icoor, const double *asdq_i, double *bm_o, double *bp_o)
+/* With aux data (maux > 0): auxl / auxr [maux][n] are the cells left / right of each interface (rpn3),
+   aux9 [maux][3][3][n] the 3x3 cells around the cell the fluctuation enters, [ma][e+1][f+1] at the
+   offset e / f in the y-like / z-like direction (rpt3; rptt3 with impt = 1, 2). */
+void oracle3d_rp_point_aux(int rp_id, const double *rp_params, int ixyz, int meqn, int mwaves, int maux, long long n,
+                           const double *ql, const double *qr, const double *auxl_i, const double *auxr_i,
+                           double *wave_o, double *s_o, double *amdq_o, double *apdq_o, int icoor, int imp,
+                           int impt, const double *aux9_i, const double *asdq_i, double *bm_o, double *bp_o)
 {
     const int mbc = 1, mx = 1, nc = 3;
-    rp_ctx3 c;
+    rp_ctx3 c = {0};
     c.rp_id = rp_id;
     memcpy(c.p, rp_params, 8 * sizeof(double));
+    const int ma = maux > 0 ? maux : 1;
+    double *aux1d = (double *)calloc((size_t)ma * nc, sizeof(double));
+    double *aux9 = (double *)calloc((size_t)ma * 9 * nc, sizeof(double));
+    c.maux = maux;
+    c.aux1d = aux1d;
+    c.aux9 = aux9;
     double *q = (double *)calloc((size_t)meqn * nc, sizeof(double));
     double *wave = (double *)calloc((size_t)meqn * mwaves * nc, sizeof(double));
     double *s = (double *)calloc((size_t)mwaves * nc, sizeof(double));
@@ -555,6 +679,18 @@ void oracle3d_rp_point(int rp_id, const double *rp_params, int ixyz, int meqn, i
             Q2(q, m, 1) = qr[m * n + k];
             Q2(q, m, 2) = qr[m * n + k];
         }
+        for (int a = 0; a < maux; a++) {
+            if (auxl_i) {
+                aux1d[a + maux * 0] = auxl_i[a * n + k];
+                aux1d[a + maux * 1] = auxr_i[a * n + k];
+                aux1d[a + maux * 2] = auxr_i[a * n + k];
+            }
+            if (aux9_i)
+                for (int e = 0; e < 3; e++)
+                    for (int f = 0; f < 3; f++)
+                        for (int i = 0; i <= 2; i++)
+                            aux9[a + maux * (e + 3 * f) + (size_t)9 * maux * i] = aux9_i[(((size_t)a * 3 + e) * 3 + f) * n + k];
+        }
         if (!asdq_i) {
             rpn3(&c, ixyz, mbc, mx, q, q, wave, s, amdq, apdq);
             for (int m = 0; m < meqn; m++) {
@@ -566,14 +702,22 @@ void oracle3d_rp_point(int rp_id, const double *rp_params, int ixyz, int meqn, i
         } else {
             for (int m = 0; m < meqn; m++)
                 for (int i = 0; i <= 2; i++) Q2(asdq, m, i) = asdq_i[m * n + k];
-            rpt3(&c, ixyz, icoor, mbc, mx, q, asdq, bm, bp);
+            rpt3(&c, ixyz, icoor, imp, impt, mbc, mx, q, asdq, bm, bp);
             for (int m = 0; m < meqn; m++) {
                 bm_o[m * n + k] = Q2(bm, m, 1);
                 bp_o[m * n + k] = Q2(bp, m, 1);
             }
         }
     }
-    free(q); free(wave); free(s); free(amdq); free(apdq); free(asdq); free(bm); free(bp);
+    free(q); free(wave); free(s); free(amdq); free(apdq); free(asdq); free(bm); free(bp); free(aux1d); free(aux9);
+}
+
+void oracle3d_rp_point(int rp_id, const double *rp_params, int ixyz, int meqn, int mwaves, long long n,
+                       const double *ql, const double *qr, double *wave_o, double *s_o, double *amdq_o,
+                       double *apdq_o, int icoor, const double *asdq_i, double *bm_o, double *bp_o)
+{
+    oracle3d_rp_point_aux(rp_id, rp_params, ixyz, meqn, mwaves, 0, n, ql, qr, NULL, NULL, wave_o, s_o, amdq_o, apdq_o,
+                          icoor, 2, 0, NULL, asdq_i, bm_o, bp_o);
 }
 
 /* =========================================================================================== */
@@ -624,6 +768,8 @@ static void rpn3_sc(const rp_ctx3 *c, int ixyz, int meqn, int mwaves, int mbc, i
 {
     if (c->rp_id == RP_ACOUSTICS3D_VC)
         rpn3_vc_acoustics(ixyz, meqn, mwaves, mbc, mx, maux, ql, qr, auxl, auxr, wave, s, amdq, apdq);
+    else if (c->rp_id == RP_ADVECTION3D_VC_FWAVE)
+        rpn3_vc_fwave(ixyz, mbc, mx, maux, ql, qr, auxl, auxr, wave, s, amdq, apdq);
     else rpn3(c, ixyz, mbc, mx, ql, qr, wave, s, amdq, apdq);
 }
 
@@ -848,7 +994,7 @@ double oracle3d_sc_flux1(int rp_id, const double *rp_params, int meqn, int mwave
                          int weno_variant, const int *mthlim)
 {
     if (!sc_known(rp_id, weno_variant)) return -1.0;
-    rp_ctx3 c;
+    rp_ctx3 c = {0};
     c.rp_id = rp_id;
     memcpy(c.p, rp_params, 8 * sizeof(double));
     sc_work w;
@@ -868,7 +1014,8 @@ double oracle3d_sc_flux3(int rp_id, const double *rp_params, int meqn, int mwave
 {
     if (!sc_known(rp_id, weno_variant)) return -1.0;
     if (rp_id == RP_ACOUSTICS3D_VC && (!aux || maux < 2)) return -1.0;
-    rp_ctx3 c;
+    if (rp_id == RP_ADVECTION3D_VC_FWAVE && (!aux || maux < 3)) return -1.0;
+    rp_ctx3 c = {0};
     c.rp_id = rp_id;
     memcpy(c.p, rp_params, 8 * sizeof(double));
     int maxm = mx > my ? mx : my;

@@ -1,8 +1,10 @@
 """Time the 3-D SharpClaw stage of every built-in 3-D solver on the GPU.
 
-    python profiles/time3d_sharpclaw.py [--sizes 128,256] [--stages 20] [--steps 5] [--parent DIR --bench-reps 3]
+    python profiles/time3d_sharpclaw.py [--sizes 128,256] [--stages 20] [--steps 5] [--solvers a,b]
+                                        [--parent DIR --bench-reps 3]
 
-For each 3-D solver (vc_acoustics_3d, advection_3d, euler_3d) at n^3 cells, strict build, PyWENO weno5
+For each 3-D solver (vc_acoustics_3d, advection_3d, euler_3d, vc_advection_fwave_3d; --solvers picks some)
+at n^3 cells, strict build, PyWENO weno5
 with f32 literals:
   - ms per RK stage (clawb200_sharpclaw_stage3, mode 0): CUDA events around `stages` stages after 3
     warm-up stages;
@@ -34,7 +36,8 @@ def card():
     return out[0] if out else "unknown"
 
 
-PARAMS = {"advection_3d": dict(u=1.0, v=0.5, w=0.25), "euler_3d": dict(gamma=1.4, gamma1=0.4), "vc_acoustics_3d": {}}
+PARAMS = {"advection_3d": dict(u=1.0, v=0.5, w=0.25), "euler_3d": dict(gamma=1.4, gamma1=0.4), "vc_acoustics_3d": {},
+          "vc_advection_fwave_3d": {}}
 
 
 def make(torch, name, n):
@@ -42,6 +45,7 @@ def make(torch, name, n):
     rs = getattr(pyclaw.riemann, name)
     solver = pyclaw.SharpClawSolver3D()
     solver.rp = rs
+    solver.fwave = rs.fwave
     solver.mwaves = rs.nwaves(3)
     solver.dt_variable, solver.dt_initial = False, 0.3 / n
     solver.cfl_desired, solver.cfl_max = 0.8, 10.0
@@ -59,7 +63,9 @@ def make(torch, name, n):
         q[1:4] -= 0.5
         q[4] = 2.5 + 0.5 * (q[1:4] ** 2).sum(0) / q[0]
     state.q = q
-    if rs.maux:
+    if name == "vc_advection_fwave_3d":   # cell velocities of both signs
+        state.aux = 2.0 * torch.rand((rs.maux, n, n, n), dtype=torch.float64, device='cuda', generator=g) - 1.0
+    elif rs.maux:
         state.aux = 1.0 + torch.randint(0, 2, (rs.maux, n, n, n), device='cuda', generator=g).to(torch.float64)
     sol = pyclaw.Solution(state)
     solver.setup(sol)
@@ -130,12 +136,13 @@ def main():
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--parent", default=None)
     ap.add_argument("--bench-reps", type=int, default=3)
+    ap.add_argument("--solvers", default="vc_acoustics_3d,advection_3d,euler_3d,vc_advection_fwave_3d")
     args = ap.parse_args()
     import torch
     print("card: %s" % card(), flush=True)
     rows = []
     for n in [int(s) for s in args.sizes.split(",")]:
-        for name in ("vc_acoustics_3d", "advection_3d", "euler_3d"):
+        for name in args.solvers.split(","):
             solver, sol = make(torch, name, n)
             st = sol.states[0]
             ms_stage = time_stages(torch, solver, st, args.stages)

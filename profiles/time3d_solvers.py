@@ -1,8 +1,9 @@
 """Time the 3-D classic steps of every built-in 3-D solver on the GPU.
 
-    python profiles/time3d_solvers.py [--sizes 128,256] [--steps 10] [--parent path/to/libclawb200.so]
+    python profiles/time3d_solvers.py [--sizes 128,256] [--steps 10] [--solvers a,b] [--parent path/to/libclawb200.so]
 
-For each 3-D solver (vc_acoustics_3d, advection_3d, euler_3d) and each algorithm (dimensional
+For each 3-D solver (vc_acoustics_3d, advection_3d, euler_3d, vc_advection_fwave_3d; --solvers picks some)
+and each algorithm (dimensional
 splitting: three step3ds sweeps; unsplit: step3 with order_trans = 22) at n^3 cells: ms per step
 (CUDA events around `steps` steps after 2 warm-up steps, strict build) and cell-updates per second.
 Every working set exceeds the 126 MB L2 except the advection split step at 128^3 (three 18 MB
@@ -33,7 +34,7 @@ def card():
 def setup(torch, _lib, name, n, method):
     from pyclaw_b200 import riemann
     rs = {"vc_acoustics_3d": riemann.vc_acoustics_3d, "advection_3d": riemann.advection_3d,
-          "euler_3d": riemann.euler_3d}[name]
+          "euler_3d": riemann.euler_3d, "vc_advection_fwave_3d": riemann.vc_advection_fwave_3d}[name]
     mbc = 2
     nx = ny = nz = n + 2 * mbc
     meqn, mw = rs.meqn(3), rs.nwaves(3)
@@ -47,7 +48,9 @@ def setup(torch, _lib, name, n, method):
         q[1:4] -= 0.5
         q[4] = 2.5 + 0.5 * (q[1:4] ** 2).sum(0) / q[0]
     aux = None
-    if rs.maux:
+    if name == "vc_advection_fwave_3d":   # cell velocities of both signs
+        aux = 2.0 * torch.rand((rs.maux, nz, ny, nx), dtype=torch.float64, device='cuda', generator=g) - 1.0
+    elif rs.maux:
         aux = 1.0 + torch.randint(0, 2, (rs.maux, nz, ny, nx), device='cuda', generator=g).to(torch.float64)
     return rs, P, q, aux
 
@@ -98,6 +101,7 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--parent", default=None, help="another build of libclawb200.so to compare with")
     ap.add_argument("--repeats", type=int, default=5)
+    ap.add_argument("--solvers", default="vc_acoustics_3d,advection_3d,euler_3d,vc_advection_fwave_3d")
     args = ap.parse_args()
     import torch
     from pyclaw_b200 import _lib
@@ -105,9 +109,10 @@ def main():
         raise SystemExit("no CUDA device: nothing to time")
     dev = card()
     print("card: %s" % dev, flush=True)
-    ids = {"vc_acoustics_3d": _lib.RP_ACOUSTICS3D_VC, "advection_3d": _lib.RP_ADVECTION3D, "euler_3d": _lib.RP_EULER3D}
+    ids = {"vc_acoustics_3d": _lib.RP_ACOUSTICS3D_VC, "advection_3d": _lib.RP_ADVECTION3D, "euler_3d": _lib.RP_EULER3D,
+           "vc_advection_fwave_3d": _lib.RP_ADVECTION3D_VC_FWAVE}
     for n in [int(s) for s in args.sizes.split(",")]:
-        for name in ("vc_acoustics_3d", "advection_3d", "euler_3d"):
+        for name in args.solvers.split(","):
             for dim_split in (True, False):
                 ms = time_step(torch, _lib, "strict", ids[name], name, n, dim_split, args.steps)
                 r = dict(solver=name, n=n, algorithm="split" if dim_split else "unsplit22", ms_per_step=round(ms, 3),

@@ -218,6 +218,7 @@ static int check_rp3(const clawb200_problem *p, bool have_aux)
     case CLAWB200_RP_ACOUSTICS3D_VC: meqn = 4; mwaves = 2; maux = 2; break;
     case CLAWB200_RP_ADVECTION3D: meqn = 1; mwaves = 1; break;
     case CLAWB200_RP_EULER3D: meqn = 5; mwaves = 3; break;
+    case CLAWB200_RP_ADVECTION3D_VC_FWAVE: meqn = 1; mwaves = 1; maux = 3; break;
     case CLAWB200_RP_USER: {
         int rc = claw_user_shape(3, &meqn, &mwaves, &maux);
         if (rc) return rc;
@@ -228,6 +229,8 @@ static int check_rp3(const clawb200_problem *p, bool have_aux)
     if (maux > 0 && (p->maux < maux || !have_aux))
         return fail(CLAWB200_ERR_INVALID, p->rp_id == CLAWB200_RP_ACOUSTICS3D_VC
                                               ? "aux array required: {impedance, sound speed}"
+                                              : p->rp_id == CLAWB200_RP_ADVECTION3D_VC_FWAVE
+                                              ? "aux array required: {u, v, w}"
                                               : "aux array required: the Riemann solver reads more aux components than maux");
     return 0;
 }
@@ -240,6 +243,8 @@ static int step3_dispatch(const clawb200_problem *p, int mz, double dz, const do
     case CLAWB200_RP_ACOUSTICS3D_VC: return claw_step3_acoustics(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
     case CLAWB200_RP_EULER3D: return claw_step3_euler(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
     case CLAWB200_RP_ADVECTION3D: return claw_step3_advection(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
+    case CLAWB200_RP_ADVECTION3D_VC_FWAVE:
+        return claw_step3_vc_advection_fwave(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
     default: return claw_step3_user(p, mz, dz, qold, qnew, aux, dt, idir, scratch, cfl_dev, st);
     }
 }

@@ -131,6 +131,9 @@ int claw_step3_euler(const clawb200_problem *p, int mz, double dz, const double 
                      const double *aux, double dt, int idir, double *scratch, double *cfl_dev, cudaStream_t st);
 int claw_step3_advection(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
                          const double *aux, double dt, int idir, double *scratch, double *cfl_dev, cudaStream_t st);
+int claw_step3_vc_advection_fwave(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
+                                  const double *aux, double dt, int idir, double *scratch, double *cfl_dev,
+                                  cudaStream_t st);
 int claw_step3_user(const clawb200_problem *p, int mz, double dz, const double *qold, double *qnew,
                     const double *aux, double dt, int idir, double *scratch, double *cfl_dev, cudaStream_t st);
 // the user-supplied solver (sweep_user.cu), id CLAWB200_RP_USER
@@ -145,6 +148,7 @@ int claw_sc_user(int ndim, bool old, const ScArgs &A, cudaStream_t st);
 int claw_sc3_acoustics(bool old, const ScArgs &A, cudaStream_t st);
 int claw_sc3_euler(bool old, const ScArgs &A, cudaStream_t st);
 int claw_sc3_advection(bool old, const ScArgs &A, cudaStream_t st);
+int claw_sc3_vc_advection_fwave(bool old, const ScArgs &A, cudaStream_t st);
 int claw_sc3_user(bool old, const ScArgs &A, cudaStream_t st);
 int claw_rp_point_user(const clawb200_problem *p, int ixy, long long n, const double *ql, const double *qr,
                        const double *auxl, const double *auxr, double *wave, double *s, double *amdq,

@@ -37,6 +37,7 @@
 #define CLAW_RP_EULER1D 13
 #define CLAW_RP_ADVECTION3D 14
 #define CLAW_RP_EULER3D 15
+#define CLAW_RP_ADVECTION3D_VC_FWAVE 16
 #define CLAW_RP_USER 100 // a solver compiled in from a user header (sweep_user.cu)
 
 // Solvers that return f-waves (jumps in the flux) instead of waves: the sweeps then use the
@@ -1416,6 +1417,73 @@ struct RpAdvection3 {
                                                              const double (&bsasdq)[1], double (&cm)[1], double (&cp)[1])
     {
         transverse<ICOOR>(ar, P, roe, ql, qr, aux, imp, bsasdq, cm, cp);
+    }
+};
+
+// 3-D conservative transport q_t + (u q)_x + (v q)_y + (w q)_z = 0 in a cell-centred velocity field,
+// f-wave form (the 3-D f-wave step, DESIGN.md §1): aux = {u, v, w} of each cell; restated, parity
+// unpinned.
+//   rpn3, direction IXYZ, velocity component d = rp3_dir(IXYZ, 1):
+//     ul = aux_l(d), ur = aux_r(d);  fwave = (ur*qr) - (ul*ql);  s = 0.5*(ul + ur)
+//     s > 0: apdq = fwave, amdq = 0;  s < 0: amdq = fwave, apdq = 0;  s == 0: amdq = apdq = 0.5*fwave
+//     so amdq + apdq == fwave == f(q_r) - f(q_l) exactly, and the step conserves q for any velocity
+//     field.  The products and the difference of fwave never contract into an FMA, in either build.
+//   rpt3, direction ICOOR: vt = velocity component rp3_dir(IXYZ, ICOOR) of the line of three cells
+//     through the cell asdq enters (aux(ma, e, f) around that cell):
+//       bm = min(0.5*(vt(-1) + vt(0)), 0) * asdq    (the lower edge of that cell)
+//       bp = max(0.5*(vt(0) + vt(+1)), 0) * asdq    (the upper edge)
+//   rptt3: the same split along the line through the cell the first split sent bsasdq to (impt = 1 /
+//     2: one cell down / up in the other transverse direction), the convention of RpAcoustics3D.
+template <int IXYZ>
+struct RpVcAdvectionFwave3 {
+    static constexpr int ID = CLAW_RP_ADVECTION3D_VC_FWAVE;
+    static constexpr int MEQN = 1, MWAVES = 1, NROE = 1, MAUX = 3;
+    static constexpr bool FWAVE = true;
+
+    template <class AR>
+    __device__ __forceinline__ static void solve(AR &, const RpParams &, const double (&l)[1], const double (&r)[1],
+                                                 const AuxCell &axl, const AuxCell &axr, double (&wave)[1][1],
+                                                 double (&s)[1], double (&amdq)[1], double (&apdq)[1],
+                                                 double (&roe)[NROE])
+    {
+        constexpr int D = rp3_dir(IXYZ, 1);
+        const double ul = axl(D - 1), ur = axr(D - 1);
+        const double fwave = __dsub_rn(__dmul_rn(ur, r[0]), __dmul_rn(ul, l[0]));
+        const double sp = 0.5 * (ul + ur);
+        wave[0][0] = fwave;
+        s[0] = sp;
+        if (sp > 0.0) { amdq[0] = 0.0; apdq[0] = fwave; }
+        else if (sp < 0.0) { amdq[0] = fwave; apdq[0] = 0.0; }
+        else { amdq[0] = 0.5 * fwave; apdq[0] = 0.5 * fwave; }
+        roe[0] = 0.0;
+    }
+    // asdq split along the line of three cells through (e0, f0) in direction ICOOR
+    template <int ICOOR>
+    __device__ __forceinline__ static void split(const AuxNbhd<MAUX> &aux, int e0, int f0, const double (&asdq)[1],
+                                                 double (&bm)[1], double (&bp)[1])
+    {
+        constexpr int MA = rp3_dir(IXYZ, ICOOR) - 1;
+        constexpr int de = (ICOOR == 2) ? 1 : 0, df = (ICOOR == 3) ? 1 : 0;
+        const double vm = aux(MA, e0 - de, f0 - df), v0 = aux(MA, e0, f0), vp = aux(MA, e0 + de, f0 + df);
+        bm[0] = dmin2(0.5 * (vm + v0), 0.0) * asdq[0];
+        bp[0] = dmax2(0.5 * (v0 + vp), 0.0) * asdq[0];
+    }
+    template <int ICOOR, class AR>
+    __device__ __forceinline__ static void transverse(AR &, const RpParams &, const double (&)[NROE],
+                                                      const double (&)[1], const double (&)[1], const AuxNbhd<MAUX> &aux,
+                                                      int, const double (&asdq)[1], double (&bm)[1], double (&bp)[1])
+    {
+        split<ICOOR>(aux, 0, 0, asdq, bm, bp);
+    }
+    template <int ICOOR, class AR>
+    __device__ __forceinline__ static void double_transverse(AR &, const RpParams &, const double (&)[NROE],
+                                                             const double (&)[1], const double (&)[1],
+                                                             const AuxNbhd<MAUX> &aux, int, int impt,
+                                                             const double (&bsasdq)[1], double (&cm)[1], double (&cp)[1])
+    {
+        const int off = (impt == 1) ? -1 : 1;
+        if (ICOOR == 2) split<ICOOR>(aux, 0, off, bsasdq, cm, cp);
+        else split<ICOOR>(aux, off, 0, bsasdq, cm, cp);
     }
 };
 

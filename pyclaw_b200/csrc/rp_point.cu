@@ -86,6 +86,7 @@ int claw_rp_point(const clawb200_problem *p, int ixy, long long n, const double 
         case CLAWB200_RP_ACOUSTICS3D_VC: GO3(RpAcoustics3D);
         case CLAWB200_RP_ADVECTION3D: GO3(RpAdvection3);
         case CLAWB200_RP_EULER3D: GO3(RpEuler3);
+        case CLAWB200_RP_ADVECTION3D_VC_FWAVE: GO3(RpVcAdvectionFwave3);
         default: return fail(CLAWB200_ERR_UNSUPPORTED, "pointwise entry: no 3-D version of this solver");
         }
     }

@@ -135,6 +135,7 @@ int sharpclaw_launch3(const clawb200_problem *p, int mz, double dz, const double
     case CLAWB200_RP_ACOUSTICS3D_VC: return claw_sc3_acoustics(old, A, st);
     case CLAWB200_RP_EULER3D: return claw_sc3_euler(old, A, st);
     case CLAWB200_RP_ADVECTION3D: return claw_sc3_advection(old, A, st);
+    case CLAWB200_RP_ADVECTION3D_VC_FWAVE: return claw_sc3_vc_advection_fwave(old, A, st);
     default: return claw_sc3_user(old, A, st);
     }
 }

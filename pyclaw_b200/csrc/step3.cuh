@@ -115,7 +115,8 @@ __device__ __forceinline__ void normal3(AR &ar, const Step3Args &A, const double
     for (int mw = 0; mw < MW; mw++) { smax_update(smax, s[1][mw]); smax_update(smax, s[2][mw]); }
 
     // limiter (limiter.f:29-55) and correction flux (flux3.f:226-241) of the interfaces c (n = 1)
-    // and c+1 (n = 2); the dot products use the unlimited waves of the neighbours
+    // and c+1 (n = 2); the dot products use the unlimited waves of the neighbours.  An f-wave solver
+    // leads with sign(s) instead of |s| (flux2fw.f:151-152, classic.cuh lead_factor): the 3-D f-wave step
 #pragma unroll
     for (int a = 0; a < 2; a++)
 #pragma unroll
@@ -145,7 +146,7 @@ __device__ __forceinline__ void normal3(AR &ar, const Step3Args &A, const double
             for (int mw = 0; mw < MW; mw++)
 #pragma unroll
                 for (int m = 0; m < M; m++)
-                    cqxx[a][m] = cqxx[a][m] + 0.5 * fabs(s[n][mw]) * (1.0 - fabs(s[n][mw]) * dtdxave) * wl[m][mw];
+                    cqxx[a][m] = cqxx[a][m] + 0.5 * lead_factor<RP>(s[n][mw]) * (1.0 - fabs(s[n][mw]) * dtdxave) * wl[m][mw];
         }
     }
 #pragma unroll

@@ -8,7 +8,8 @@ keys of ``state.aux_global`` (the cparam common block the script fills).
 """
 from .._lib import (RP_ACOUSTICS, RP_ADVECTION, RP_EULER5, RP_SHALLOW, RP_SPHERE, RP_NEL_FWAVE,
                     RP_PSYSTEM, RP_ACOUSTICS3D_VC, RP_VC_ACOUSTICS, RP_BURGERS, RP_ADVECTION_COLOR,
-                    RP_VC_ADVECTION, RP_EULER1D, RP_ADVECTION3D, RP_EULER3D)
+                    RP_VC_ADVECTION, RP_EULER1D, RP_ADVECTION3D, RP_EULER3D,
+                    RP_ADVECTION3D_VC_FWAVE)
 
 
 class RiemannSolver(object):
@@ -110,6 +111,10 @@ vc_acoustics_3d = RiemannSolver("vc_acoustics_3d", RP_ACOUSTICS3D_VC, 4, 2, [], 
 # 3-D constant-coefficient advection and 3-D Euler (Roe + entropy fix; q = rho, rho u, rho v, rho w, E)
 advection_3d = RiemannSolver("advection_3d", RP_ADVECTION3D, 1, 1, ["u", "v", "w"], (3,))
 euler_3d = RiemannSolver("euler_3d", RP_EULER3D, 5, 3, ["gamma", "gamma1"], (3,))
+# 3-D conservative transport q_t + (u q)_x + (v q)_y + (w q)_z = 0 in a cell-centred velocity field,
+# aux = {u, v, w}; an f-wave solver (solver.fwave = True): conserves q for any velocity field
+vc_advection_fwave_3d = RiemannSolver("vc_advection_fwave_3d", RP_ADVECTION3D_VC_FWAVE, 1, 1, [], (3,), fwave=True,
+                                      maux=3)
 
 # further solvers of the reference's applications (set solver.rp to use them)
 vc_acoustics = RiemannSolver("vc_acoustics", RP_VC_ACOUSTICS, 3, 2, [], (2,), maux=2)          # aux {rho, c}
@@ -151,7 +156,8 @@ def from_header(header, name=None, meqn=1, mwaves=1, ndims=(2,), param_names=(),
 
 
 _BY_NAME = {s.name: s for s in (vc_acoustics, burgers, advection_color, vc_advection, euler_with_efix,
-                                vc_acoustics_3d, advection_3d, euler_3d, acoustics, advection, euler_5wave, shallow_roe_with_efix, shallow_sphere,
+                                vc_acoustics_3d, advection_3d, euler_3d, vc_advection_fwave_3d,
+                                acoustics, advection, euler_5wave, shallow_roe_with_efix, shallow_sphere,
                                 nonlinear_elasticity_fwave, psystem)}
 _BY_NAME.update({"euler": euler_5wave, "shallow": shallow_roe_with_efix})
 
