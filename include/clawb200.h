@@ -235,9 +235,7 @@ int clawb200_bc_fill(const clawb200_problem *p, double *q, int narr, int idim, i
  * algorithm, idir = 1, 2, 3.  p->ndim = 3; p->mx, my, dx, dy as usual, the third dimension
  * travels as (mz, dz); the field is q[m][k][j][i] with p->pitch = padded row length and
  * p->mstride >= pitch*(my+2mbc)*(mz+2mbc).  q_out receives qold in cells the sweep does not
- * touch; q_in != q_out.  p->rp_id: any 3-D solver above (meqn / mwaves / maux checked per solver);
- * the environment variable CLAWB200_STEP3DS_PLANES=1 (an A/B knob of the vc-acoustics kernels) makes
- * every other solver fail with CLAWB200_ERR_UNSUPPORTED. */
+ * touch; q_in != q_out.  p->rp_id: any 3-D solver above (meqn / mwaves / maux checked per solver). */
 int clawb200_step3ds(const clawb200_problem *p, int mz, double dz, const double *q_in, double *q_out,
                      const double *aux, double dt, int idir, double *cfl_dev, void *stream);
 /* classic3.step3 (src/fortran/3d/classic/step3.f:2-594 with flux3.f:5-595 and the rpt3 / rptt3

@@ -39,12 +39,12 @@ UNITS = {
     "step3.cu": _COMMON + ["step3.cuh"],          # 3-D steps (step3.cuh): vc-acoustics
     "step3_euler.cu": _COMMON + ["step3.cuh"],    # ... 3-D Euler
     "step3_misc.cu": _COMMON + ["step3.cuh"],     # ... 3-D advection, 3-D f-wave transport
-    "rp_point.cu": _COMMON,
+    "rp_point.cu": _COMMON + ["rp_point.cuh"],
     "sharpclaw.cu": _COMMON + ["sharpclaw.cuh"],
     "sharpclaw3.cu": _COMMON + ["sharpclaw.cuh", "sharpclaw3.cuh"],        # 3-D SharpClaw stage: vc-acoustics
     "sharpclaw3_euler.cu": _COMMON + ["sharpclaw.cuh", "sharpclaw3.cuh"],  # ... 3-D Euler
     "sharpclaw3_misc.cu": _COMMON + ["sharpclaw.cuh", "sharpclaw3.cuh"],   # ... 3-D advection, 3-D f-wave transport
-    "sweep_user.cu": _COMMON + ["sharpclaw.cuh", "sharpclaw3.cuh", "step3.cuh"],   # the user-supplied Riemann solver (a stub without one)
+    "sweep_user.cu": _COMMON + ["rp_point.cuh", "sharpclaw.cuh", "sharpclaw3.cuh", "step3.cuh"],   # the user-supplied Riemann solver (a stub without one)
 }
 SOURCES = list(UNITS)
 HEADERS = sorted({h for hs in UNITS.values() for h in hs})

@@ -170,8 +170,8 @@ extern "C" int clawb200_step1(const clawb200_problem *p, const double *q_in, dou
     if ((rc = check_aux(p, aux, false))) return rc;
     SweepArgs A = make_args(p, q_in, q_out, dt, cfl_dev, aux);
     cudaStream_t st = (cudaStream_t)stream;
-    if (p->rp_id == CLAWB200_RP_USER) return claw_step1_user(A, p->mx, st);
-    return claw_step1(p->rp_id, A, p->mx, st);
+    if (p->rp_id == CLAWB200_RP_USER) return claw_step1_user(A, st);
+    return claw_step1(p->rp_id, A, st);
 }
 
 extern "C" int clawb200_step2ds(const clawb200_problem *p, const double *q_in, double *q_out,
@@ -204,11 +204,7 @@ extern "C" int clawb200_step2ds(const clawb200_problem *p, const double *q_in, d
 
 // ---------------------------------------------------------------------------
 // 3-D, dimensional splitting (step3ds.f:2-376; clawpack.py:656-676) and the unsplit step.  A 3-D
-// field is q[m][k][j][i].  Both run the kernels of step3.cuh for every 3-D solver; for vc-acoustics
-// CLAWB200_STEP3DS_PLANES=1 runs a split sweep on the 2-D engines instead, on 2-D views of the array:
-// x- and y-sweeps plane by plane (k = 0..mz+1), z-sweeps on the (i, k) slices j = 0..my+1 (row
-// stride = one plane).  The arithmetic of flux3.f with method(3) < 0 is that of flux2.f (the 0.5 of
-// the correction flux is applied per term instead of to the sum, an exact scaling).
+// field is q[m][k][j][i].  Both run the kernels of step3.cuh for every 3-D solver.
 // ---------------------------------------------------------------------------
 // The Riemann solver of a 3-D step: the shape it is compiled for and the aux data it reads.
 static int check_rp3(const clawb200_problem *p, bool have_aux)
@@ -261,52 +257,10 @@ extern "C" int clawb200_step3ds(const clawb200_problem *p, int mz, double dz, co
     if (mz < 1 || !(dz > 0.0)) return fail(CLAWB200_ERR_INVALID, "mz, dz must be positive");
     if (q_in == q_out) return fail(CLAWB200_ERR_INVALID, "q_in and q_out must differ");
     if (idir < 1 || idir > 3) return fail(CLAWB200_ERR_INVALID, "idir must be 1, 2 or 3");
-    const int mbc = p->mbc, nx = p->pitch, ny = p->my + 2 * mbc, nz = mz + 2 * mbc;
-    const long long plane = (long long)nx * ny;
-    if (p->mstride < plane * nz) return fail(CLAWB200_ERR_INVALID, "mstride smaller than the padded field");
-    cudaStream_t st = (cudaStream_t)stream;
-    // One launch over the whole padded field (step3.cuh): swept cells are updated, all others copied.
-    // CLAWB200_STEP3DS_PLANES=1 keeps round 1's composition from the 2-D engines (one launch per
-    // plane after a copy of the field) for A/B measurements.
-    static const bool planes = [] { const char *e = getenv("CLAWB200_STEP3DS_PLANES"); return e && atoi(e) != 0; }();
-    if (!planes) return step3_dispatch(p, mz, dz, q_in, q_out, aux, dt, idir, nullptr, cfl_dev, st);
-    if (p->rp_id != CLAWB200_RP_ACOUSTICS3D_VC)
-        return fail(CLAWB200_ERR_UNSUPPORTED, "CLAWB200_STEP3DS_PLANES is compiled for the vc-acoustics solver only");
-    // step3ds.f: "qold and qnew are identical on entry"; cells the sweep does not touch keep qold
-    CUDA_OK(cudaMemcpyAsync(q_out, q_in, sizeof(double) * (size_t)p->meqn * p->mstride,
-                            cudaMemcpyDeviceToDevice, st));
-    clawb200_problem P2 = *p;
-    P2.ndim = 2;
-    if (idir == 1 || idir == 2) {
-        for (int k = 0; k <= mz + 1; k++) {
-            const long long off = plane * (k + mbc - 1);
-            SweepArgs A = make_args(&P2, q_in + off, q_out + off, dt, cfl_dev, aux + off);
-            A.trans = -1;
-            if (idir == 1) {
-                A.ilo = 1; A.ihi = p->mx; A.jlo = 0; A.jhi = p->my + 1;
-                A.rows_per_cta = pick_rows(A.jhi - A.jlo + 1, (p->mx + XNT - 4) / (XNT - 3));
-                if ((rc = claw_x_ac3d(A, st))) return rc;
-            } else {
-                A.ilo = 0; A.ihi = p->mx + 1; A.jlo = 1; A.jhi = p->my;
-                A.rows_per_cta = pick_rows(p->my, (p->mx + 2 + YNT - 1) / YNT);
-                if ((rc = claw_y_ac3d(2, A, st))) return rc;
-            }
-        }
-    } else {
-        clawb200_problem P3 = P2;
-        P3.my = mz;
-        P3.dy = dz;
-        P3.pitch = (int)plane;
-        for (int j = 0; j <= p->my + 1; j++) {
-            const long long off = (long long)nx * (j + mbc - 1);
-            SweepArgs A = make_args(&P3, q_in + off, q_out + off, dt, cfl_dev, aux + off);
-            A.trans = -1;
-            A.ilo = 0; A.ihi = p->mx + 1; A.jlo = 1; A.jhi = mz;
-            A.rows_per_cta = pick_rows(mz, (p->mx + 2 + YNT - 1) / YNT);
-            if ((rc = claw_y_ac3d(3, A, st))) return rc;
-        }
-    }
-    return 0;
+    const long long plane = (long long)p->pitch * (p->my + 2 * p->mbc);
+    if (p->mstride < plane * (mz + 2 * p->mbc)) return fail(CLAWB200_ERR_INVALID, "mstride smaller than the padded field");
+    // one launch over the whole padded field (step3.cuh): swept cells are updated, all others copied
+    return step3_dispatch(p, mz, dz, q_in, q_out, aux, dt, idir, nullptr, cfl_dev, (cudaStream_t)stream);
 }
 
 // classic3.step3 (step3.f:2-594 + flux3.f:5-595; clawpack.py:680-682): the unsplit 3-D step.
@@ -395,11 +349,9 @@ static int step2_impl(const clawb200_problem *p, const double *qold, double *qne
     A.ilo = 1; A.ihi = p->mx; A.jlo = jlo; A.jhi = jhi;
     const int nrows = jhi - jlo + 1;
     // both sweeps in one walk over q where a single-pass kernel exists (fused.cuh): q read once,
-    // written once.  problem.step2_mode = 1 (or CLAWB200_TWO_PASS=1 in the environment, for A/B
-    // measurements) keeps the two sweep kernels.
-    static const bool env_two_pass = [] { const char *e = getenv("CLAWB200_TWO_PASS"); return e && atoi(e) != 0; }();
+    // written once.  problem.step2_mode = 1 keeps the two sweep kernels.
     if (p->step2_mode < 0 || p->step2_mode > 2) return fail(CLAWB200_ERR_INVALID, "step2_mode must be 0, 1 or 2");
-    if (parts == 3 && p->step2_mode != 1 && !(env_two_pass && p->step2_mode == 0)) {
+    if (parts == 3 && p->step2_mode != 1) {
         if (claw_fused_available(p->rp_id, A)) return claw_fused(p->rp_id, A, st);
         if (p->step2_mode == 2) return fail(CLAWB200_ERR_UNSUPPORTED, "no single-pass kernel for this solver / problem (step2_mode = 2)");
     }
@@ -427,8 +379,7 @@ extern "C" int clawb200_step2_launches(const clawb200_problem *p)
     if (!p) return fail(CLAWB200_ERR_INVALID, "null problem");
     int rc = check_problem(p, 2);
     if (rc) return rc;
-    static const bool env_two_pass = [] { const char *e = getenv("CLAWB200_TWO_PASS"); return e && atoi(e) != 0; }();
-    if (p->step2_mode == 1 || (env_two_pass && p->step2_mode == 0)) return 2;
+    if (p->step2_mode == 1) return 2;
     SweepArgs A = make_args(p, nullptr, nullptr, 0.0, nullptr, nullptr);
     return claw_fused_available(p->rp_id, A) ? 1 : 2;
 }
@@ -900,12 +851,8 @@ static int host_pipeline(const clawb200_problem *p, const double *qold, double *
     const int out1 = (mode == 1) ? ny_tot : mbc + p->my;
     const int halo = (mode == 1) ? 0 : mbc; // input rows needed beyond the output rows
     // slab height: PCIe time is the bound, the first upload and the last download are the only
-    // transfers that do not overlap, so slabs are kept small (CLAWB200_SLAB_ROWS overrides)
-    static const int slab_rows = [] {
-        const char *e = getenv("CLAWB200_SLAB_ROWS");
-        int v = e ? atoi(e) : 0;
-        return (v >= 16) ? v : 128;
-    }();
+    // transfers that do not overlap, so slabs are kept small
+    constexpr int slab_rows = 128;
     int nslab = (out1 - out0 + slab_rows - 1) / slab_rows;
     if (nslab < 1) nslab = 1;
     const int rows_per = (out1 - out0 + nslab - 1) / nslab;

@@ -1,5 +1,6 @@
 // launch.cuh -- shared by the translation units of libclawb200.so: error reporting, shared-
-// memory opt-in and the launchers of the two classic sweep engines (classic.cuh).
+// memory opt-in and the launchers of the classic kernels (classic.cuh): the two sweep engines and
+// the 1-D step.  The built-in solvers and the user solver (sweep_user.cu) launch through them.
 //
 // The library is built from several translation units (pyclaw_b200/build.py compiles them in
 // parallel): clawb200.cu (C ABI, boundary fills, layout / halo kernels, host entry points),
@@ -63,13 +64,14 @@ static void hint_carveout(K kernel, size_t smem_per_cta, int ctas)
 constexpr int XNT = 128; // threads per CTA of the x-engine
 constexpr int YNT = 128; // threads per CTA of the y-engine
 
-template <class RP, bool TRANS, bool CAPA = false>
-static int launch_x(SweepArgs A, cudaStream_t st)
+// the classic sweeps: trans selects the unsplit (transverse) form, CAPA the capacity-function form
+template <class RP, bool CAPA = false>
+static int launch_x(bool trans, const SweepArgs &A, cudaStream_t st)
 {
     constexpr int NC = XNT - 3;
     size_t smem = sizeof(double) * (2 * RP::MEQN * (XNT + 1) + RP::MEQN * RP::MWAVES * XNT + 4 * RP::MEQN * XNT +
-                                    ((rp_x_aux_smem<RP>::value && TRANS) ? 4 * RP::MAUX * (XNT + 2) : 0));
-    auto k = xsweep_kernel<RP, TRANS, CAPA, XNT>;
+                                    ((rp_x_aux_smem<RP>::value && trans) ? 4 * RP::MAUX * (XNT + 2) : 0));
+    auto k = trans ? xsweep_kernel<RP, true, CAPA, XNT> : xsweep_kernel<RP, false, CAPA, XNT>;
     CUDA_OK(set_smem(k, smem));
     if (RP::MAUX >= 8) hint_carveout(k, smem, RP::X_MINB);
     int ncols = A.ihi - A.ilo + 1, nrows = A.jhi - A.jlo + 1;
@@ -79,12 +81,12 @@ static int launch_x(SweepArgs A, cudaStream_t st)
     return 0;
 }
 
-template <class RP, bool TRANS, bool CAPA = false>
-static int launch_y(SweepArgs A, cudaStream_t st)
+template <class RP, bool CAPA = false>
+static int launch_y(bool trans, const SweepArgs &A, cudaStream_t st)
 {
-    constexpr int NC = TRANS ? YNT - 2 : YNT;
-    size_t smem = sizeof(double) * YNT * ((TRANS ? 4 * RP::MEQN : 0) + YSlots<RP, TRANS>::COUNT);
-    auto k = ysweep_kernel<RP, TRANS, CAPA, YNT>;
+    const int NC = trans ? YNT - 2 : YNT;
+    size_t smem = sizeof(double) * YNT * (trans ? 4 * RP::MEQN + YSlots<RP, true>::COUNT : YSlots<RP, false>::COUNT);
+    auto k = trans ? ysweep_kernel<RP, true, CAPA, YNT> : ysweep_kernel<RP, false, CAPA, YNT>;
     CUDA_OK(set_smem(k, smem));
     if (RP::MAUX >= 8) hint_carveout(k, smem, RP::Y_MINB);
     int ncols = A.ihi - A.ilo + 1, nrows = A.jhi - A.jlo + 1;
@@ -94,12 +96,24 @@ static int launch_y(SweepArgs A, cudaStream_t st)
     return 0;
 }
 
+// the 1-D step; CAPA: the solver has a capacity-function form, the others refuse mcapa
+template <class RP, bool CAPA>
+static int launch_step1(const SweepArgs &A, cudaStream_t st)
+{
+    constexpr int NT = 128, NC = NT - 3;
+    size_t smem = sizeof(double) * (RP::MEQN * (NT + 1) + RP::MEQN * RP::MWAVES * NT + 2 * RP::MEQN * NT);
+    dim3 grid((A.mx + NC - 1) / NC);
+    if (A.mcapa <= 0) step1_kernel<RP, NT><<<grid, NT, smem, st>>>(A);
+    else if constexpr (CAPA) step1_kernel<RP, NT, true><<<grid, NT, smem, st>>>(A);
+    else return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for this solver");
+    CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
 static inline int pick_rows(int nrows, int ncol_ctas, bool tall = true)
 {
     // enough CTAs to fill 148 SMs a few times over, but strips tall enough that the
     // start-up rows of the streaming engines stay a small fraction of the work
-    static const int forced = [] { const char *e = getenv("CLAWB200_ROWS_PER_CTA"); return e ? atoi(e) : 0; }();
-    if (forced > 0) return forced; // tuning experiments
     // very large grids: 128-row strips halve the start-up rows again and still leave ~10 waves of
     // CTAs (Euler 8192^2: 9.10 -> 8.89 ms per step; 4096^2 and the sphere are flat or worse, the
     // SharpClaw stage kernel too: tall = false)
@@ -117,8 +131,6 @@ int claw_x_sphere(bool trans, const SweepArgs &A, cudaStream_t st);
 int claw_y_sphere(bool trans, const SweepArgs &A, cudaStream_t st);
 int claw_x_misc(int rp_id, bool trans, const SweepArgs &A, cudaStream_t st);
 int claw_y_misc(int rp_id, bool trans, const SweepArgs &A, cudaStream_t st);
-int claw_x_ac3d(const SweepArgs &A, cudaStream_t st);           // 3-D acoustics, x-engine (idir = 1)
-int claw_y_ac3d(int idir, const SweepArgs &A, cudaStream_t st); // 3-D acoustics, y-engine (idir = 2, 3)
 // single-pass unsplit step (sweep_fused.cu): solvers without aux / capa whose windows fit in registers
 bool claw_fused_available(int rp_id, const SweepArgs &A);
 int claw_fused(int rp_id, const SweepArgs &A, cudaStream_t st);
@@ -141,7 +153,7 @@ struct ScArgs;
 int claw_user_shape(int ndim, int *meqn, int *mwaves, int *maux); // ndim = 3: RpUser3
 int claw_x_user(bool trans, const SweepArgs &A, cudaStream_t st);
 int claw_y_user(bool trans, const SweepArgs &A, cudaStream_t st);
-int claw_step1_user(const SweepArgs &A, int mx, cudaStream_t st);
+int claw_step1_user(const SweepArgs &A, cudaStream_t st);
 int claw_sc_user(int ndim, bool old, const ScArgs &A, cudaStream_t st);
 // 3-D SharpClaw stage (sharpclaw3.cuh), one translation unit per solver family (sharpclaw3.cu,
 // sharpclaw3_euler.cu, sharpclaw3_misc.cu, sweep_user.cu)
@@ -156,7 +168,7 @@ int claw_rp_point_user(const clawb200_problem *p, int ixy, long long n, const do
 int claw_rp_point(const clawb200_problem *p, int ixy, long long n, const double *ql, const double *qr,
                   const double *auxl, const double *auxr, double *wave, double *s, double *amdq, double *apdq,
                   int imp, const double *asdq, double *bm, double *bp, cudaStream_t st);
-int claw_step1(int rp_id, const SweepArgs &A, int mx, cudaStream_t st);
+int claw_step1(int rp_id, const SweepArgs &A, cudaStream_t st);
 int sharpclaw_launch(const clawb200_problem *p, const double *q, const double *qa, double *out,
                      double *dq_out, double dt, int mode, double ca, double cb, double div,
                      double *cfl_dev, cudaStream_t st, const double *aux);

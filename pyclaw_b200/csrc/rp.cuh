@@ -1036,18 +1036,14 @@ struct RpElasticFwave {
 // 3-D acoustics in a heterogeneous medium.  clawpack/riemann rpn3_vc_acoustics.f (external;
 // test/acoustics/3d).  q = (p, u, v, w); aux = {impedance Z, sound speed c} of each cell.
 // IXYZ = 1, 2, 3 is the sweep direction.  The 3-D interface (transverse<ICOOR> = rpt3,
-// double_transverse<ICOOR> = rptt3) is defined below with the other 3-D solvers; the 2-D
-// `transverse` is the one the 2-D engines compile (CLAWB200_STEP3DS_PLANES: split sweeps only).
+// double_transverse<ICOOR> = rptt3) is defined below with the other 3-D solvers.
 // ---------------------------------------------------------------------------
 template <int IXYZ>
 struct RpAcoustics3D {
     static constexpr int ID = CLAW_RP_ACOUSTICS3D_VC;
     static constexpr int MEQN = 4, MWAVES = 2, NROE = 1;
-    static constexpr int X_MINB = 4, Y_MINB = 4;
     static constexpr int MAUX = 2;
-    static constexpr bool QCOR = false;
     static constexpr int MU = IXYZ;
-    __host__ __device__ static constexpr bool nz(int m, int mw) { return m == 0 || m == MU; }
 
     template <class AR>
     __device__ __forceinline__ static void solve(AR &ar, const RpParams &P, const double (&l)[4],
@@ -1075,16 +1071,6 @@ struct RpAcoustics3D {
             apdq[m] = s[1] * wave[m][1];
         }
         roe[0] = 0.0;
-    }
-
-    template <class AR>
-    __device__ __forceinline__ static void transverse(AR &, const RpParams &, const double (&)[NROE],
-                                                      const double (&)[4], const AuxCell &, const AuxCell &,
-                                                      const AuxCell &, const double (&)[4], double (&bm)[4],
-                                                      double (&bp)[4])
-    {
-#pragma unroll
-        for (int m = 0; m < 4; m++) { bm[m] = 0.0; bp[m] = 0.0; }
     }
 
     // rpt3 / rptt3_vc_acoustics: asdq split along the line of three cells through (e0, f0) of the

@@ -5,11 +5,6 @@
 
 using RpColor1D = RpColor<1, 1>;
 
-// ---------------------------------------------------------------------------
-// SharpClaw
-// ---------------------------------------------------------------------------
-constexpr int SNT = 128;
-
 extern "C" int clawb200_weno_table_doubles(void) { return (int)(sizeof(WenoTab) / sizeof(double)); }
 
 extern "C" int clawb200_pack_weno_tables(int k, const double *S, const double *CL, const double *CR,
@@ -43,12 +38,14 @@ static int sc_launch1_tab(const ScArgs &A, int weno_k, cudaStream_t st)
 }
 
 template <class RPX, class RPY>
-static int sc_launch2_tab(const ScArgs &A, int weno_k, cudaStream_t st)
+static int sc_launch2_tab(ScArgs A, int weno_k, cudaStream_t st)
 {
     constexpr int NC = SNT - 2;
     const int H = weno_k - 1;
     size_t smem = sizeof(double) * (RPX::MEQN * (SNT + 2 * H) + 2 * RPX::MEQN * SNT);
-    dim3 grid((A.mx + NC - 1) / NC, (A.my + A.rows_per_cta - 1) / A.rows_per_cta);
+    const int nxcta = (A.mx + NC - 1) / NC;
+    A.rows_per_cta = pick_rows(A.my, nxcta, false);
+    dim3 grid(nxcta, (A.my + A.rows_per_cta - 1) / A.rows_per_cta);
     sc2d_tab_kernel<RPX, RPY, SNT><<<grid, SNT, smem, st>>>(A);
     CUDA_OK(cudaGetLastError());
     return 0;
@@ -68,29 +65,6 @@ static void weno_constants(ScArgs &A, int variant)
     A.r0166 = LIT(0.166666666666667);
 #undef LIT
     A.epweno = (double)1.e-36f; // reconstruct.f90:7, a REAL(4) literal
-}
-
-template <class RPX, class RPY, bool OLD, bool CAPA = false>
-static int sc_launch2(const ScArgs &A, cudaStream_t st)
-{
-    constexpr int NC = SNT - 2;
-    size_t smem = sizeof(double) * (2 * RPX::MEQN * (SNT + 4) + 2 * RPX::MEQN * SNT);
-    auto k = sc2d_kernel<RPX, RPY, OLD, SNT, CAPA>;
-    CUDA_OK(set_smem(k, smem));
-    dim3 grid((A.mx + NC - 1) / NC, (A.my + A.rows_per_cta - 1) / A.rows_per_cta);
-    k<<<grid, SNT, smem, st>>>(A);
-    CUDA_OK(cudaGetLastError());
-    return 0;
-}
-
-template <class RP, bool OLD, bool CAPA = false>
-static int sc_launch1(const ScArgs &A, cudaStream_t st)
-{
-    constexpr int NC = SNT - 2;
-    size_t smem = sizeof(double) * (RP::MEQN * (SNT + 4) + 2 * RP::MEQN * SNT);
-    sc1d_kernel<RP, OLD, SNT, CAPA><<<(A.mx + NC - 1) / NC, SNT, smem, st>>>(A);
-    CUDA_OK(cudaGetLastError());
-    return 0;
 }
 
 // the stage arguments common to 1-D, 2-D and 3-D
@@ -157,7 +131,6 @@ int sharpclaw_launch(const clawb200_problem *p, const double *q, const double *q
         A.tab = reinterpret_cast<const WenoTab *>(p->weno_tab);
         if (p->method[5] > 0) return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for WENO orders above 5");
         if (p->ndim == 2) {
-            A.rows_per_cta = pick_rows(p->my, (p->mx + SNT - 3) / (SNT - 2), false);
             switch (p->rp_id) {
             case CLAWB200_RP_ACOUSTICS: return sc_launch2_tab<RpAcoustics<2, 1>, RpAcoustics<2, 2>>(A, wk, st);
             case CLAWB200_RP_ADVECTION: return sc_launch2_tab<RpAdvection<2, 1>, RpAdvection<2, 2>>(A, wk, st);
@@ -209,7 +182,6 @@ int sharpclaw_launch(const clawb200_problem *p, const double *q, const double *q
     }
     if (p->rp_id == CLAWB200_RP_USER) {
         if (p->method[5] > 0) return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa is not compiled for the user solver in SharpClaw");
-        if (p->ndim == 2) A.rows_per_cta = pick_rows(p->my, (p->mx + SNT - 3) / (SNT - 2), false);
         return claw_sc_user(p->ndim, old, A, st);
     }
     if (p->method[5] > 0) {
@@ -218,61 +190,38 @@ int sharpclaw_launch(const clawb200_problem *p, const double *q, const double *q
         A.dt = dt; A.dx = p->dx; A.dy = (p->ndim > 1) ? p->dy : 1.0;
         if (p->ndim == 1) {
             switch (p->rp_id) {
-            case CLAWB200_RP_ACOUSTICS:
-                return old ? sc_launch1<RpAcoustics<1, 1>, true, true>(A, st) : sc_launch1<RpAcoustics<1, 1>, false, true>(A, st);
-            case CLAWB200_RP_ADVECTION:
-                return old ? sc_launch1<RpAdvection<1, 1>, true, true>(A, st) : sc_launch1<RpAdvection<1, 1>, false, true>(A, st);
+            case CLAWB200_RP_ACOUSTICS: return sc_launch1<RpAcoustics<1, 1>, true>(old, A, st);
+            case CLAWB200_RP_ADVECTION: return sc_launch1<RpAdvection<1, 1>, true>(old, A, st);
             default: return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for this solver");
             }
         }
-        A.rows_per_cta = pick_rows(p->my, (p->mx + SNT - 3) / (SNT - 2), false);
         switch (p->rp_id) {
-        case CLAWB200_RP_ACOUSTICS: return old ? sc_launch2<RpAcoustics<2, 1>, RpAcoustics<2, 2>, true, true>(A, st)
-                                               : sc_launch2<RpAcoustics<2, 1>, RpAcoustics<2, 2>, false, true>(A, st);
-        case CLAWB200_RP_ADVECTION: return old ? sc_launch2<RpAdvection<2, 1>, RpAdvection<2, 2>, true, true>(A, st)
-                                               : sc_launch2<RpAdvection<2, 1>, RpAdvection<2, 2>, false, true>(A, st);
+        case CLAWB200_RP_ACOUSTICS: return sc_launch2<RpAcoustics<2, 1>, RpAcoustics<2, 2>, true>(old, A, st);
+        case CLAWB200_RP_ADVECTION: return sc_launch2<RpAdvection<2, 1>, RpAdvection<2, 2>, true>(old, A, st);
         default: return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for this solver");
         }
     }
     if (p->ndim == 1) {
         switch (p->rp_id) {
-        case CLAWB200_RP_ACOUSTICS:
-            return old ? sc_launch1<RpAcoustics<1, 1>, true>(A, st) : sc_launch1<RpAcoustics<1, 1>, false>(A, st);
-        case CLAWB200_RP_ADVECTION:
-            return old ? sc_launch1<RpAdvection<1, 1>, true>(A, st) : sc_launch1<RpAdvection<1, 1>, false>(A, st);
-        case CLAWB200_RP_SHALLOW:
-            return old ? sc_launch1<RpShallow1D, true>(A, st) : sc_launch1<RpShallow1D, false>(A, st);
-        case CLAWB200_RP_BURGERS:
-            return old ? sc_launch1<RpBurgers, true>(A, st) : sc_launch1<RpBurgers, false>(A, st);
-        case CLAWB200_RP_EULER1D:
-            return old ? sc_launch1<RpEuler1D, true>(A, st) : sc_launch1<RpEuler1D, false>(A, st);
+        case CLAWB200_RP_ACOUSTICS: return sc_launch1<RpAcoustics<1, 1>>(old, A, st);
+        case CLAWB200_RP_ADVECTION: return sc_launch1<RpAdvection<1, 1>>(old, A, st);
+        case CLAWB200_RP_SHALLOW: return sc_launch1<RpShallow1D>(old, A, st);
+        case CLAWB200_RP_BURGERS: return sc_launch1<RpBurgers>(old, A, st);
+        case CLAWB200_RP_EULER1D: return sc_launch1<RpEuler1D>(old, A, st);
         case CLAWB200_RP_NEL_FWAVE: // with char_decomp = 0 an f-wave solver only contributes amdq / apdq
-            return old ? sc_launch1<RpElasticFwave<1, 1>, true>(A, st) : sc_launch1<RpElasticFwave<1, 1>, false>(A, st);
-        case CLAWB200_RP_ADVECTION_COLOR:
-            return old ? sc_launch1<RpColor1D, true>(A, st) : sc_launch1<RpColor1D, false>(A, st);
+            return sc_launch1<RpElasticFwave<1, 1>>(old, A, st);
+        case CLAWB200_RP_ADVECTION_COLOR: return sc_launch1<RpColor1D>(old, A, st);
         default: return fail(CLAWB200_ERR_UNSUPPORTED, "no 1-D version of this Riemann solver");
         }
     }
-    A.rows_per_cta = pick_rows(p->my, (p->mx + SNT - 3) / (SNT - 2), false);
-#define SC2(RPT)                                                                         \
-    return old ? sc_launch2<RPT, true>(A, st) : sc_launch2<RPT, false>(A, st)
     switch (p->rp_id) {
-    case CLAWB200_RP_ACOUSTICS: return old ? sc_launch2<RpAcoustics<2, 1>, RpAcoustics<2, 2>, true>(A, st)
-                                           : sc_launch2<RpAcoustics<2, 1>, RpAcoustics<2, 2>, false>(A, st);
-    case CLAWB200_RP_ADVECTION: return old ? sc_launch2<RpAdvection<2, 1>, RpAdvection<2, 2>, true>(A, st)
-                                           : sc_launch2<RpAdvection<2, 1>, RpAdvection<2, 2>, false>(A, st);
-    case CLAWB200_RP_EULER5: return old ? sc_launch2<RpEuler5<1>, RpEuler5<2>, true>(A, st)
-                                        : sc_launch2<RpEuler5<1>, RpEuler5<2>, false>(A, st);
-    case CLAWB200_RP_SHALLOW: return old ? sc_launch2<RpShallow<1>, RpShallow<2>, true>(A, st)
-                                         : sc_launch2<RpShallow<1>, RpShallow<2>, false>(A, st);
-    case CLAWB200_RP_PSYSTEM: return old ? sc_launch2<RpElasticFwave<2, 1>, RpElasticFwave<2, 2>, true>(A, st)
-                                         : sc_launch2<RpElasticFwave<2, 1>, RpElasticFwave<2, 2>, false>(A, st);
-    case CLAWB200_RP_VC_ACOUSTICS: return old ? sc_launch2<RpVcAcoustics<1>, RpVcAcoustics<2>, true>(A, st)
-                                              : sc_launch2<RpVcAcoustics<1>, RpVcAcoustics<2>, false>(A, st);
-    case CLAWB200_RP_VC_ADVECTION: return old ? sc_launch2<RpColor<2, 1>, RpColor<2, 2>, true>(A, st)
-                                              : sc_launch2<RpColor<2, 1>, RpColor<2, 2>, false>(A, st);
+    case CLAWB200_RP_ACOUSTICS: return sc_launch2<RpAcoustics<2, 1>, RpAcoustics<2, 2>>(old, A, st);
+    case CLAWB200_RP_ADVECTION: return sc_launch2<RpAdvection<2, 1>, RpAdvection<2, 2>>(old, A, st);
+    case CLAWB200_RP_EULER5: return sc_launch2<RpEuler5<1>, RpEuler5<2>>(old, A, st);
+    case CLAWB200_RP_SHALLOW: return sc_launch2<RpShallow<1>, RpShallow<2>>(old, A, st);
+    case CLAWB200_RP_PSYSTEM: return sc_launch2<RpElasticFwave<2, 1>, RpElasticFwave<2, 2>>(old, A, st);
+    case CLAWB200_RP_VC_ACOUSTICS: return sc_launch2<RpVcAcoustics<1>, RpVcAcoustics<2>>(old, A, st);
+    case CLAWB200_RP_VC_ADVECTION: return sc_launch2<RpColor<2, 1>, RpColor<2, 2>>(old, A, st);
     default: return fail(CLAWB200_ERR_UNSUPPORTED, "unknown rp_id");
     }
-#undef SC2
 }
-

@@ -11,7 +11,7 @@
 // window private to the thread, so q is read once and the stage result written once.
 // dq = (0 + dq_x) + dq_y exactly as flux2.f90 accumulates it.
 #pragma once
-#include "rp.cuh"
+#include "launch.cuh"
 
 struct WenoTab;
 struct ScArgs {
@@ -511,7 +511,39 @@ __global__ void __launch_bounds__(NT) sc1d_kernel(const ScArgs A)
     sc_cfl_commit(cfl, A.cfl_bits);
 }
 
+// ---- launchers of the WENO5 stage kernels, for the built-in solvers (sharpclaw.cu), the user
+// solver (sweep_user.cu) and the plane kernel of the 3-D stage (sharpclaw3.cuh).  old selects the
+// literal reading of weno5 (weno_variant), CAPA the capacity-function form.
+constexpr int SNT = 128; // threads per CTA
 
+template <class RP, bool CAPA = false>
+static int sc_launch1(bool old, const ScArgs &A, cudaStream_t st)
+{
+    constexpr int NC = SNT - 2;
+    size_t smem = sizeof(double) * (RP::MEQN * (SNT + 4) + 2 * RP::MEQN * SNT);
+    auto k = old ? sc1d_kernel<RP, true, SNT, CAPA> : sc1d_kernel<RP, false, SNT, CAPA>;
+    k<<<(A.mx + NC - 1) / NC, SNT, smem, st>>>(A);
+    CUDA_OK(cudaGetLastError());
+    return 0;
+}
+
+template <class RPX>
+constexpr size_t sc2d_smem() { return sizeof(double) * (2 * RPX::MEQN * (SNT + 4) + 2 * RPX::MEQN * SNT); }
+
+template <class RPX, class RPY, bool CAPA = false>
+static int sc_launch2(bool old, ScArgs A, cudaStream_t st)
+{
+    constexpr int NC = SNT - 2;
+    constexpr size_t smem = sc2d_smem<RPX>();
+    auto k = old ? sc2d_kernel<RPX, RPY, true, SNT, CAPA> : sc2d_kernel<RPX, RPY, false, SNT, CAPA>;
+    CUDA_OK(set_smem(k, smem));
+    const int nxcta = (A.mx + NC - 1) / NC;
+    A.rows_per_cta = pick_rows(A.my, nxcta, false);
+    dim3 grid(nxcta, (A.my + A.rows_per_cta - 1) / A.rows_per_cta);
+    k<<<grid, SNT, smem, st>>>(A);
+    CUDA_OK(cudaGetLastError());
+    return 0;
+}
 
 // ---------------------------------------------------------------------------
 // 1-D, char_decomp = 1 (flux1.f90:95-105): wave-based WENO5, reconstruct.f90:393-471 (weno5_wave)

@@ -111,7 +111,7 @@ __global__ void __launch_bounds__(NT, (RPZ::MEQN <= 3) ? CLAW_SC_MINB : 2) sc3d_
 template <template <int> class RPF, bool OLD>
 int sc_launch3(ScArgs A, cudaStream_t st)
 {
-    constexpr int NT = 128, NC = NT - 2;
+    constexpr int NT = SNT, NC = NT - 2;
     using RX = RPF<1>;
     // x and y, plane by plane: the partial goes to dq_out (or out) through stage mode 3
     {
@@ -120,7 +120,7 @@ int sc_launch3(ScArgs A, cudaStream_t st)
         B.dq_out = A.dq_out ? A.dq_out : A.out;
         const int nxcta = (A.mx + NC - 1) / NC;
         B.rows_per_cta = pick_rows(A.my, nxcta * (A.mz + 2), false);
-        size_t smem = sizeof(double) * (2 * RX::MEQN * (NT + 4) + 2 * RX::MEQN * NT);
+        constexpr size_t smem = sc2d_smem<RX>();
         auto k = sc2d_kernel<RX, RPF<2>, OLD, NT, false, true>;
         CUDA_OK(set_smem(k, smem));
         dim3 grid(nxcta, (A.my + B.rows_per_cta - 1) / B.rows_per_cta, A.mz + 2);

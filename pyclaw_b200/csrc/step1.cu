@@ -1,51 +1,16 @@
 // step1.cu -- the 1-D classic step (step1.f) for every 1-D Riemann solver.
 #include "launch.cuh"
 
-using RpColor1D = RpColor<1, 1>; // (a template-id with a comma cannot be a macro argument)
-
-int claw_step1(int rp_id, const SweepArgs &A, int mx, cudaStream_t st)
+int claw_step1(int rp_id, const SweepArgs &A, cudaStream_t st)
 {
-    constexpr int NT = 128, NC = NT - 3;
-    dim3 grid((mx + NC - 1) / NC);
-    const bool capa = A.mcapa > 0;
     switch (rp_id) {
-    case CLAWB200_RP_ACOUSTICS: {
-        using RP = RpAcoustics<1, 1>;
-        size_t smem = sizeof(double) * (RP::MEQN * (NT + 1) + RP::MEQN * RP::MWAVES * NT + 2 * RP::MEQN * NT);
-        if (capa) step1_kernel<RP, NT, true><<<grid, NT, smem, st>>>(A);
-        else step1_kernel<RP, NT><<<grid, NT, smem, st>>>(A);
-    } break;
-    case CLAWB200_RP_ADVECTION: {
-        using RP = RpAdvection<1, 1>;
-        size_t smem = sizeof(double) * (RP::MEQN * (NT + 1) + RP::MEQN * RP::MWAVES * NT + 2 * RP::MEQN * NT);
-        if (capa) step1_kernel<RP, NT, true><<<grid, NT, smem, st>>>(A);
-        else step1_kernel<RP, NT><<<grid, NT, smem, st>>>(A);
-    } break;
-    case CLAWB200_RP_SHALLOW: {
-        using RP = RpShallow1D;
-        if (capa) return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for this solver");
-        size_t smem = sizeof(double) * (RP::MEQN * (NT + 1) + RP::MEQN * RP::MWAVES * NT + 2 * RP::MEQN * NT);
-        step1_kernel<RP, NT><<<grid, NT, smem, st>>>(A);
-    } break;
-    case CLAWB200_RP_NEL_FWAVE: {
-        using RP = RpElasticFwave<1, 1>;
-        size_t smem = sizeof(double) * (RP::MEQN * (NT + 1) + RP::MEQN * RP::MWAVES * NT + 2 * RP::MEQN * NT);
-        step1_kernel<RP, NT><<<grid, NT, smem, st>>>(A);
-    } break;
-#define STEP1_PLAIN(RPT)                                                                                     \
-    {                                                                                                        \
-        using RP = RPT;                                                                                      \
-        if (capa) return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for this solver");               \
-        size_t smem = sizeof(double) * (RP::MEQN * (NT + 1) + RP::MEQN * RP::MWAVES * NT + 2 * RP::MEQN * NT); \
-        step1_kernel<RP, NT><<<grid, NT, smem, st>>>(A);                                                     \
-    }                                                                                                        \
-    break
-    case CLAWB200_RP_BURGERS: STEP1_PLAIN(RpBurgers);
-    case CLAWB200_RP_ADVECTION_COLOR: STEP1_PLAIN(RpColor1D);
-    case CLAWB200_RP_EULER1D: STEP1_PLAIN(RpEuler1D);
-#undef STEP1_PLAIN
+    case CLAWB200_RP_ACOUSTICS: return launch_step1<RpAcoustics<1, 1>, true>(A, st);
+    case CLAWB200_RP_ADVECTION: return launch_step1<RpAdvection<1, 1>, true>(A, st);
+    case CLAWB200_RP_SHALLOW: return launch_step1<RpShallow1D, false>(A, st);
+    case CLAWB200_RP_NEL_FWAVE: return launch_step1<RpElasticFwave<1, 1>, false>(A, st);
+    case CLAWB200_RP_BURGERS: return launch_step1<RpBurgers, false>(A, st);
+    case CLAWB200_RP_ADVECTION_COLOR: return launch_step1<RpColor<1, 1>, false>(A, st);
+    case CLAWB200_RP_EULER1D: return launch_step1<RpEuler1D, false>(A, st);
     default: return fail(CLAWB200_ERR_UNSUPPORTED, "no 1-D version of this Riemann solver");
     }
-    CUDA_OK(cudaGetLastError());
-    return 0;
 }

@@ -3,7 +3,5 @@
 
 int claw_x_euler(bool trans, const SweepArgs &A, cudaStream_t st)
 {
-    if (A.mcapa > 0)
-        return trans ? launch_x<RpEuler5<1>, true, true>(A, st) : launch_x<RpEuler5<1>, false, true>(A, st);
-    return trans ? launch_x<RpEuler5<1>, true>(A, st) : launch_x<RpEuler5<1>, false>(A, st);
+    return A.mcapa > 0 ? launch_x<RpEuler5<1>, true>(trans, A, st) : launch_x<RpEuler5<1>>(trans, A, st);
 }

@@ -3,7 +3,5 @@
 
 int claw_y_euler(bool trans, const SweepArgs &A, cudaStream_t st)
 {
-    if (A.mcapa > 0)
-        return trans ? launch_y<RpEuler5<2>, true, true>(A, st) : launch_y<RpEuler5<2>, false, true>(A, st);
-    return trans ? launch_y<RpEuler5<2>, true>(A, st) : launch_y<RpEuler5<2>, false>(A, st);
+    return A.mcapa > 0 ? launch_y<RpEuler5<2>, true>(trans, A, st) : launch_y<RpEuler5<2>>(trans, A, st);
 }

@@ -1,32 +1,25 @@
 // sweep_misc.cu -- classic sweeps for the light solvers: acoustics, advection, shallow water
-// (Roe + entropy fix), p-system f-waves, variable-coefficient acoustics / advection, and the
-// 3-D acoustics solver of the dimension-split 3-D path.
+// (Roe + entropy fix), p-system f-waves, variable-coefficient acoustics / advection.
 #include "launch.cuh"
-
-#define BOTH(FN, RPT, CAPA) (trans ? FN<RPT, true, CAPA>(A, st) : FN<RPT, false, CAPA>(A, st))
-using AcX = RpAcoustics<2, 1>; using AcY = RpAcoustics<2, 2>;
-using AdX = RpAdvection<2, 1>; using AdY = RpAdvection<2, 2>;
-using CoX = RpColor<2, 1>; using CoY = RpColor<2, 2>;
-using PsX = RpElasticFwave<2, 1>; using PsY = RpElasticFwave<2, 2>;
 
 int claw_x_misc(int rp_id, bool trans, const SweepArgs &A, cudaStream_t st)
 {
     if (A.mcapa > 0) {
         switch (rp_id) {
-        case CLAWB200_RP_ACOUSTICS: return BOTH(launch_x, AcX, true);
-        case CLAWB200_RP_ADVECTION: return BOTH(launch_x, AdX, true);
-        case CLAWB200_RP_SHALLOW: return BOTH(launch_x, RpShallow<1>, true);
-        case CLAWB200_RP_VC_ADVECTION: return BOTH(launch_x, CoX, true);
+        case CLAWB200_RP_ACOUSTICS: return launch_x<RpAcoustics<2, 1>, true>(trans, A, st);
+        case CLAWB200_RP_ADVECTION: return launch_x<RpAdvection<2, 1>, true>(trans, A, st);
+        case CLAWB200_RP_SHALLOW: return launch_x<RpShallow<1>, true>(trans, A, st);
+        case CLAWB200_RP_VC_ADVECTION: return launch_x<RpColor<2, 1>, true>(trans, A, st);
         default: return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for this solver");
         }
     }
     switch (rp_id) {
-    case CLAWB200_RP_ACOUSTICS: return BOTH(launch_x, AcX, false);
-    case CLAWB200_RP_ADVECTION: return BOTH(launch_x, AdX, false);
-    case CLAWB200_RP_SHALLOW: return BOTH(launch_x, RpShallow<1>, false);
-    case CLAWB200_RP_PSYSTEM: return BOTH(launch_x, PsX, false);
-    case CLAWB200_RP_VC_ACOUSTICS: return BOTH(launch_x, RpVcAcoustics<1>, false);
-    case CLAWB200_RP_VC_ADVECTION: return BOTH(launch_x, CoX, false);
+    case CLAWB200_RP_ACOUSTICS: return launch_x<RpAcoustics<2, 1>>(trans, A, st);
+    case CLAWB200_RP_ADVECTION: return launch_x<RpAdvection<2, 1>>(trans, A, st);
+    case CLAWB200_RP_SHALLOW: return launch_x<RpShallow<1>>(trans, A, st);
+    case CLAWB200_RP_PSYSTEM: return launch_x<RpElasticFwave<2, 1>>(trans, A, st);
+    case CLAWB200_RP_VC_ACOUSTICS: return launch_x<RpVcAcoustics<1>>(trans, A, st);
+    case CLAWB200_RP_VC_ADVECTION: return launch_x<RpColor<2, 1>>(trans, A, st);
     default: return fail(CLAWB200_ERR_UNSUPPORTED, "unknown rp_id");
     }
 }
@@ -35,26 +28,20 @@ int claw_y_misc(int rp_id, bool trans, const SweepArgs &A, cudaStream_t st)
 {
     if (A.mcapa > 0) {
         switch (rp_id) {
-        case CLAWB200_RP_ACOUSTICS: return BOTH(launch_y, AcY, true);
-        case CLAWB200_RP_ADVECTION: return BOTH(launch_y, AdY, true);
-        case CLAWB200_RP_SHALLOW: return BOTH(launch_y, RpShallow<2>, true);
-        case CLAWB200_RP_VC_ADVECTION: return BOTH(launch_y, CoY, true);
+        case CLAWB200_RP_ACOUSTICS: return launch_y<RpAcoustics<2, 2>, true>(trans, A, st);
+        case CLAWB200_RP_ADVECTION: return launch_y<RpAdvection<2, 2>, true>(trans, A, st);
+        case CLAWB200_RP_SHALLOW: return launch_y<RpShallow<2>, true>(trans, A, st);
+        case CLAWB200_RP_VC_ADVECTION: return launch_y<RpColor<2, 2>, true>(trans, A, st);
         default: return fail(CLAWB200_ERR_UNSUPPORTED, "mcapa not compiled for this solver");
         }
     }
     switch (rp_id) {
-    case CLAWB200_RP_ACOUSTICS: return BOTH(launch_y, AcY, false);
-    case CLAWB200_RP_ADVECTION: return BOTH(launch_y, AdY, false);
-    case CLAWB200_RP_SHALLOW: return BOTH(launch_y, RpShallow<2>, false);
-    case CLAWB200_RP_PSYSTEM: return BOTH(launch_y, PsY, false);
-    case CLAWB200_RP_VC_ACOUSTICS: return BOTH(launch_y, RpVcAcoustics<2>, false);
-    case CLAWB200_RP_VC_ADVECTION: return BOTH(launch_y, CoY, false);
+    case CLAWB200_RP_ACOUSTICS: return launch_y<RpAcoustics<2, 2>>(trans, A, st);
+    case CLAWB200_RP_ADVECTION: return launch_y<RpAdvection<2, 2>>(trans, A, st);
+    case CLAWB200_RP_SHALLOW: return launch_y<RpShallow<2>>(trans, A, st);
+    case CLAWB200_RP_PSYSTEM: return launch_y<RpElasticFwave<2, 2>>(trans, A, st);
+    case CLAWB200_RP_VC_ACOUSTICS: return launch_y<RpVcAcoustics<2>>(trans, A, st);
+    case CLAWB200_RP_VC_ADVECTION: return launch_y<RpColor<2, 2>>(trans, A, st);
     default: return fail(CLAWB200_ERR_UNSUPPORTED, "unknown rp_id");
     }
-}
-
-int claw_x_ac3d(const SweepArgs &A, cudaStream_t st) { return launch_x<RpAcoustics3D<1>, false>(A, st); }
-int claw_y_ac3d(int idir, const SweepArgs &A, cudaStream_t st)
-{
-    return (idir == 2) ? launch_y<RpAcoustics3D<2>, false>(A, st) : launch_y<RpAcoustics3D<3>, false>(A, st);
 }

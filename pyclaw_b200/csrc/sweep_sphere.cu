@@ -2,11 +2,5 @@
 // step2qcor correction).
 #include "launch.cuh"
 
-int claw_x_sphere(bool trans, const SweepArgs &A, cudaStream_t st)
-{
-    return trans ? launch_x<RpSphere<1>, true, true>(A, st) : launch_x<RpSphere<1>, false, true>(A, st);
-}
-int claw_y_sphere(bool trans, const SweepArgs &A, cudaStream_t st)
-{
-    return trans ? launch_y<RpSphere<2>, true, true>(A, st) : launch_y<RpSphere<2>, false, true>(A, st);
-}
+int claw_x_sphere(bool trans, const SweepArgs &A, cudaStream_t st) { return launch_x<RpSphere<1>, true>(trans, A, st); }
+int claw_y_sphere(bool trans, const SweepArgs &A, cudaStream_t st) { return launch_y<RpSphere<2>, true>(trans, A, st); }
