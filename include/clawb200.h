@@ -292,6 +292,36 @@ int clawb200_rp_transverse_host(const clawb200_problem *p, int ixy, long long n,
                                 const double *qr, int imp, const double *asdq, double *bmasdq,
                                 double *bpasdq);
 
+/* ---- the library's division / square-root arithmetic on HOST arrays (a test entry point) -----
+ * out3[k][n] receives, per element, the results of `op` under `policy`; bad[n] the fast path's
+ * sticky flag (1 where it would fall back to the IEEE operators; 0 for EXACT).
+ *   policy: FAST      the build's FastArith (integer zero test of a numerator)
+ *           FAST_FZ   its floating-point zero-test twin (what with_arith_fz runs first)
+ *           EXACT     the IEEE operators
+ *           GUARDED   with_arith: FAST, repeated with EXACT if the flag is set (what kernels compute)
+ *           GUARDED_FZ with_arith_fz
+ *   op (a: numerator / radicand, b: denominator): out3[0] =
+ *           RCP 1/b   RCP_NC 1/b (unchecked)   DIV_RCP div(a, rcp(b))   DIV div(a, b)
+ *           DIV_NZ div_nz(a, rcp_nc(b))   SQRT sqrt(a)
+ *           SQRT_RCP    sqrt(a); out3[1] = 1/sqrt(a)
+ *           SQRT_RCPS   sqrt(a); out3[1] = 1/sqrt(a), out3[2] = 1/a
+ *           SQRT_RCP2S  sqrt(a); out3[1] = 1/(2 sqrt(a)), out3[2] = 1/a */
+#define CLAWB200_ARITH_FAST 0
+#define CLAWB200_ARITH_FAST_FZ 1
+#define CLAWB200_ARITH_EXACT 2
+#define CLAWB200_ARITH_GUARDED 3
+#define CLAWB200_ARITH_GUARDED_FZ 4
+#define CLAWB200_ARITH_RCP 0
+#define CLAWB200_ARITH_RCP_NC 1
+#define CLAWB200_ARITH_DIV_RCP 2
+#define CLAWB200_ARITH_DIV 3
+#define CLAWB200_ARITH_DIV_NZ 4
+#define CLAWB200_ARITH_SQRT 5
+#define CLAWB200_ARITH_SQRT_RCP 6
+#define CLAWB200_ARITH_SQRT_RCPS 7
+#define CLAWB200_ARITH_SQRT_RCP2S 8
+int clawb200_arith_probe(int policy, int op, long long n, const double *a, const double *b, double *out3, int *bad);
+
 /* ---- host-pointer entry points (the f2py signatures) -----------------------------
  * As the Fortran documents (step2.f:8-9), qold and qnew are taken to be identical on entry:
  * only qold is uploaded, qnew receives the result (untouched cells = qold).  Large 2-D

@@ -22,6 +22,10 @@ RP_USER = 100   # a solver compiled in from a user header (riemann.from_header)
 WENO_PYWENO_F32, WENO_PYWENO_F64, WENO_OLD, WENO_TABLES, RECON_TVD2 = 0, 1, 2, 3, 4
 RECON_WENO_WAVE, RECON_WENO_FWAVE = 5, 6
 STAGE_AXPY, STAGE_CONVEX, STAGE_FINAL104, STAGE_DQ_ONLY = 0, 1, 2, 3
+# clawb200_arith_probe: policies and operations
+ARITH_FAST, ARITH_FAST_FZ, ARITH_EXACT, ARITH_GUARDED, ARITH_GUARDED_FZ = 0, 1, 2, 3, 4
+(ARITH_RCP, ARITH_RCP_NC, ARITH_DIV_RCP, ARITH_DIV, ARITH_DIV_NZ, ARITH_SQRT, ARITH_SQRT_RCP, ARITH_SQRT_RCPS,
+ ARITH_SQRT_RCP2S) = range(9)
 
 
 class ClawB200Error(RuntimeError):
@@ -127,6 +131,7 @@ SIGNATURES = {
     "clawb200_rp_transverse": [_pp, _i, ctypes.c_longlong, _dp, _dp, _i, _dp, _dp, _dp, _vp],
     "clawb200_rp_solve_host": [_pp, _i, ctypes.c_longlong, _dp, _dp, _dp, _dp, _dp, _dp, _dp, _dp],
     "clawb200_rp_transverse_host": [_pp, _i, ctypes.c_longlong, _dp, _dp, _i, _dp, _dp, _dp],
+    "clawb200_arith_probe": [_i, _i, ctypes.c_longlong, _dp, _dp, _dp, _vp],
 }
 
 
