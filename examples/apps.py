@@ -239,6 +239,58 @@ def psystem(cells_per_layer=20, petsc=False, tfinal=2.0, outdir=None):
     return _run(pyclaw, solver, state, tfinal, 10, outdir)
 
 
+def bump1d(mx=200, petsc=False, tfinal=0.7, eps=1e-3, outdir=None):
+    """Shallow water over a bump (pyclaw.riemann.shallow_bathymetry_fwave): LeVeque's perturbed steady
+    state (J. Comput. Phys. 146, 1998, sec. 5).  Bottom b = 0.25 (cos(10 pi (x - 0.5)) + 1) for
+    |x - 0.5| < 0.1, else 0, on [0, 1]; the lake at rest eta = h + b = 1 carries a pulse eta = 1 + eps
+    on 0.1 < x < 0.2; g = 9.81, outflow boundaries.  The well-balanced solver keeps the undisturbed
+    water exactly at rest while the pulse crosses the bump."""
+    pyclaw = _pc(petsc)
+    solver = pyclaw.ClawSolver1D()
+    solver.rp = pyclaw.riemann.shallow_bathymetry_fwave
+    solver.fwave = True
+    solver.mwaves, solver.limiters = 2, pyclaw.limiters.tvd.MC
+    solver.bc_lower[0] = solver.bc_upper[0] = pyclaw.BC.outflow
+    solver.aux_bc_lower[0] = solver.aux_bc_upper[0] = pyclaw.BC.outflow
+    grid = pyclaw.Grid(pyclaw.Dimension('x', 0.0, 1.0, mx))
+    state = pyclaw.State(grid, 2, 1)
+    state.aux_global['grav'] = 9.81
+    xc = grid.x.center
+    b = np.where(np.abs(xc - 0.5) < 0.1, 0.25 * (np.cos(10 * np.pi * (xc - 0.5)) + 1.0), 0.0)
+    state.aux[0, :] = b
+    state.q[0, :] = 1.0 + eps * ((xc > 0.1) & (xc < 0.2)) - b
+    state.q[1, :] = 0.
+    solver.dt_initial = 0.2 * grid.d[0]
+    return _run(pyclaw, solver, state, tfinal, 10, outdir)
+
+
+def seamount2d(mx=200, my=200, dim_split=True, petsc=False, tfinal=1.0, outdir=None):
+    """Shallow water over bathymetry in a closed basin (pyclaw.riemann.shallow_bathymetry_fwave): a
+    Gaussian hump on the surface west of a Gaussian seamount, reflecting walls on [-1, 1]^2, g = 9.81.
+    The bottom rises from b = -1 to b = -0.2 at the seamount's top (0.25, 0), so h >= 0.2 everywhere.
+    dim_split=False runs the unsplit step with transverse corrections (order_trans = 2)."""
+    pyclaw = _pc(petsc)
+    solver = pyclaw.ClawSolver2D()
+    solver.rp = pyclaw.riemann.shallow_bathymetry_fwave
+    solver.fwave = True
+    solver.mwaves, solver.limiters = 3, pyclaw.limiters.tvd.MC
+    solver.dim_split, solver.order_trans = bool(dim_split), 2
+    for i in range(2):
+        solver.bc_lower[i] = solver.bc_upper[i] = pyclaw.BC.reflecting
+        solver.aux_bc_lower[i] = solver.aux_bc_upper[i] = pyclaw.BC.reflecting
+    grid = pyclaw.Grid([pyclaw.Dimension('x', -1.0, 1.0, mx), pyclaw.Dimension('y', -1.0, 1.0, my)])
+    state = pyclaw.State(grid, 3, 1)
+    state.aux_global['grav'] = 9.81
+    Y, X = np.meshgrid(grid.y.center, grid.x.center)
+    b = -1.0 + 0.8 * np.exp(-((X - 0.25) ** 2 + Y ** 2) / 0.2 ** 2)
+    state.aux[0, :, :] = b
+    state.q[0, :, :] = 0.1 * np.exp(-((X + 0.5) ** 2 + Y ** 2) / 0.1 ** 2) - b
+    state.q[1, :, :] = 0.
+    state.q[2, :, :] = 0.
+    solver.dt_initial = 0.2 * min(grid.d)
+    return _run(pyclaw, solver, state, tfinal, 10, outdir)
+
+
 def acoustics3d(mx=256, my=4, mz=4, petsc=False, tfinal=2.0, outdir=None, test='hom', upper_bc=None):
     """test/acoustics/3d/acoustics.py: 'hom' (homogeneous medium, dimensional splitting, periodic) or
     'het' (impedance and sound speed double at x = 0, unsplit with order_trans = 22, reflecting lower
@@ -488,8 +540,8 @@ def transport3d(mx=32, my=32, mz=32, petsc=False, period=1.0, tfinal=None, dim_s
 
 
 APPS = {f.__name__: f for f in (acoustics1d, acoustics2d, vc_acoustics2d, shockbubble, shallow1d, shallow2d,
-                                shallow_sphere, stegoton, psystem, acoustics3d, burgers, wcblast,
-                                vc_advection1d, annulus, euler3d, advection3d, transport3d)}
+                                shallow_sphere, stegoton, psystem, bump1d, seamount2d, acoustics3d, burgers,
+                                wcblast, vc_advection1d, annulus, euler3d, advection3d, transport3d)}
 
 
 def main(argv):

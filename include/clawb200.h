@@ -49,6 +49,8 @@ extern "C" {
 #define CLAWB200_RP_NEL_FWAVE 6 /* rp1_nonlinear_elasticity_fwave (apps/elasticity/1d/stegoton);
                                    aux {rho, K}; params {stress law: 1 linear, 2 exponential} */
 #define CLAWB200_RP_PSYSTEM 7   /* rpn2/rpt2_psystem (test/psystem); aux {rho, E, law, eps} */
+#define CLAWB200_RP_SHALLOW_BATHY_FWAVE 17 /* shallow water over bathymetry, well-balanced f-waves (1-D, 2-D);
+                                              aux {b}; params {grav, dry_tolerance} */
 /* further solvers of the reference's applications (external clawpack/riemann sources) */
 #define CLAWB200_RP_VC_ACOUSTICS 9    /* rpn2/rpt2_vc_acoustics (apps/acoustics/2d/variable); aux {rho, c} */
 #define CLAWB200_RP_BURGERS 10        /* rp1_burgers with entropy fix (apps/burgers/1d)                   */

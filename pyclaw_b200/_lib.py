@@ -18,6 +18,7 @@ RP_ACOUSTICS, RP_ADVECTION, RP_EULER5, RP_SHALLOW, RP_SPHERE = 1, 2, 3, 4, 5
 RP_NEL_FWAVE, RP_PSYSTEM, RP_ACOUSTICS3D_VC = 6, 7, 8
 RP_VC_ACOUSTICS, RP_BURGERS, RP_ADVECTION_COLOR, RP_VC_ADVECTION, RP_EULER1D = 9, 10, 11, 12, 13
 RP_ADVECTION3D, RP_EULER3D, RP_ADVECTION3D_VC_FWAVE = 14, 15, 16
+RP_SHALLOW_BATHY_FWAVE = 17
 RP_USER = 100   # a solver compiled in from a user header (riemann.from_header)
 WENO_PYWENO_F32, WENO_PYWENO_F64, WENO_OLD, WENO_TABLES, RECON_TVD2 = 0, 1, 2, 3, 4
 RECON_WENO_WAVE, RECON_WENO_FWAVE = 5, 6

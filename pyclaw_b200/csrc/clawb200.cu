@@ -45,7 +45,8 @@ static int check_problem(const clawb200_problem *p, int ndim)
 static int check_aux(const clawb200_problem *p, const double *aux, bool classic2d)
 {
     const bool capa = p->method[5] > 0;
-    const bool fw = p->rp_id == CLAWB200_RP_NEL_FWAVE || p->rp_id == CLAWB200_RP_PSYSTEM;
+    const bool bathy = p->rp_id == CLAWB200_RP_SHALLOW_BATHY_FWAVE;
+    const bool fw = p->rp_id == CLAWB200_RP_NEL_FWAVE || p->rp_id == CLAWB200_RP_PSYSTEM || bathy;
     const bool vc = p->rp_id == CLAWB200_RP_VC_ACOUSTICS || p->rp_id == CLAWB200_RP_ADVECTION_COLOR ||
                     p->rp_id == CLAWB200_RP_VC_ADVECTION;
     const bool need_aux = capa || fw || vc || p->rp_id == CLAWB200_RP_SPHERE;
@@ -53,6 +54,7 @@ static int check_aux(const clawb200_problem *p, const double *aux, bool classic2
     if (!aux) return fail(CLAWB200_ERR_INVALID, "aux array required (mcapa > 0 or aux-dependent Riemann solver)");
     if (fw) { // classic step1 / step2 / step2ds only (the callers check the solver's dimension)
         if (capa) return fail(CLAWB200_ERR_UNSUPPORTED, "capacity function is not compiled for the f-wave solvers");
+        if (bathy) return p->maux < 1 ? fail(CLAWB200_ERR_INVALID, "shallow water over bathymetry: aux = {b}, maux >= 1") : 0;
         if (p->rp_id == CLAWB200_RP_NEL_FWAVE ? p->maux < 2 : p->maux != 4)
             return fail(CLAWB200_ERR_INVALID, "f-wave elasticity solvers: aux = {rho, K} (1-D) or {rho, E, law, eps} (2-D)");
         return 0;
@@ -140,6 +142,10 @@ static int check_rp_shape(const clawb200_problem *p)
     case CLAWB200_RP_ADVECTION_COLOR: meqn = 1; mwaves = 1; break;
     case CLAWB200_RP_VC_ADVECTION: meqn = 1; mwaves = 1; break;
     case CLAWB200_RP_EULER1D: meqn = 3; mwaves = 3; break;
+    case CLAWB200_RP_SHALLOW_BATHY_FWAVE:
+        if (p->ndim != 1 && p->ndim != 2) return fail(CLAWB200_ERR_UNSUPPORTED, "this Riemann solver is 1-D / 2-D only");
+        if (!(p->rp_params[1] >= 0.0)) return fail(CLAWB200_ERR_INVALID, "dry_tolerance (rp_params[1]) must be >= 0");
+        meqn = p->ndim + 1; mwaves = p->ndim + 1; break;
     case CLAWB200_RP_USER: {
         int maux = 0;
         int rc = claw_user_shape(p->ndim, &meqn, &mwaves, &maux);

@@ -38,6 +38,7 @@
 #define CLAW_RP_ADVECTION3D 14
 #define CLAW_RP_EULER3D 15
 #define CLAW_RP_ADVECTION3D_VC_FWAVE 16
+#define CLAW_RP_SHALLOW_BATHY_FWAVE 17
 #define CLAW_RP_USER 100 // a solver compiled in from a user header (sweep_user.cu)
 
 // Solvers that return f-waves (jumps in the flux) instead of waves: the sweeps then use the
@@ -1028,6 +1029,134 @@ struct RpElasticFwave {
         bp[0] = cp * a2;
         bp[mu] = 0.0;
         bp[mv] = cp * a2 * (-zp);
+    }
+};
+
+// ---------------------------------------------------------------------------
+// Shallow water over bathymetry, f-wave solver (Bale, LeVeque, Mitran & Rossmanith 2002, SIAM J.
+// Sci. Comput. 24; LeVeque 2002 sec. 15.5): the source -g h b_x is folded into the flux jump of each
+// interface, so at a lake at rest (u = v = 0, h + b constant) every f-wave is round-off and the step
+// keeps the lake at rest (well balanced).  Restated, parity unpinned.
+// q = (h, hu) (NDIM = 1) or (h, hu, hv); aux = {b}, the bottom elevation; params {grav, dry_tolerance}.
+//   velocity u = hu / h where h > dry_tolerance, else 0; phi = hu u + g h^2 / 2
+//   u^ = (sqrt(h_l) u_l + sqrt(h_r) u_r) / (sqrt(h_l) + sqrt(h_r)) (v^ alike), c^ = sqrt(g (h_l + h_r) / 2),
+//   with h clamped at 0 under every square root
+//   s1 = min(u_l - sqrt(g h_l), u^ - c^), s3 = max(u_r + sqrt(g h_r), u^ + c^) (Einfeldt); 2-D: s2 = u^
+//   d1 = hu_r - hu_l, d2 = phi_r - phi_l + g (h_l + h_r) (b_r - b_l) / 2, 2-D: d3 = hu_r v_r - hu_l v_l
+//   b1 = (s3 d1 - d2) / (s3 - s1), b3 = (d2 - s1 d1) / (s3 - s1)
+//   Z1 = b1 (1, s1, v_l), Z2 = (0, 0, d3 - b1 v_l - b3 v_r) (2-D only), Z3 = b3 (1, s3, v_r)
+//   amdq / apdq = sum of the f-waves with s < 0 / s > 0, half of each wave with s = 0 to either side.
+// An interface dry on both sides has no waves.  roe[] = {u^, v^, c^, 0.5 / c^}: the transverse solve is
+// RpShallow's at these averages (it reads no aux; the bathymetry enters through the normal f-waves).
+// ---------------------------------------------------------------------------
+template <int NDIM, int IXY>
+struct RpShallowBathyFwave {
+    static constexpr int ID = CLAW_RP_SHALLOW_BATHY_FWAVE;
+    static constexpr int MEQN = NDIM + 1, MWAVES = NDIM + 1, NROE = 4;
+    static constexpr int X_MINB = 3, Y_MINB = 3; // -Xptxas -v: the unsplit x-sweep spills at 4 CTAs/SM (128 registers)
+    static constexpr int MAUX = 1;
+    static constexpr bool QCOR = false;
+    static constexpr bool FWAVE = true;
+    static constexpr int MU = (IXY == 2) ? 2 : 1, MV = (IXY == 2) ? 1 : 2;
+    // the 2-D shear wave has its MV component only
+    __host__ __device__ static constexpr bool nz(int m, int mw) { return !(NDIM == 2 && mw == 1 && m != MV); }
+
+    template <class AR>
+    __device__ __forceinline__ static void solve(AR &ar, const RpParams &P, const double (&l)[MEQN],
+                                                 const double (&r)[MEQN], const AuxCell &axl, const AuxCell &axr,
+                                                 double (&wave)[MEQN][MWAVES],
+                                                 double (&s)[MWAVES], double (&amdq)[MEQN],
+                                                 double (&apdq)[MEQN], double (&roe)[NROE])
+    {
+        constexpr int mv = (NDIM == 2) ? MV : 0, NW = MWAVES;
+        const double grav = P.p[0], dry = P.p[1];
+        const double hl = l[0], hr = r[0];
+        const bool wetl = hl > dry, wetr = hr > dry;
+        if (!wetl && !wetr) {
+#pragma unroll
+            for (int m = 0; m < MEQN; m++) {
+#pragma unroll
+                for (int mw = 0; mw < NW; mw++) wave[m][mw] = 0.0;
+                amdq[m] = 0.0;
+                apdq[m] = 0.0;
+            }
+#pragma unroll
+            for (int mw = 0; mw < NW; mw++) s[mw] = 0.0;
+            roe[0] = roe[1] = roe[2] = roe[3] = 0.0;
+            return;
+        }
+        // a dry cell's quotient is discarded: divide by 1 there so that it stays finite
+        const Recip rhl = ar.rcp(wetl ? hl : 1.0), rhr = ar.rcp(wetr ? hr : 1.0);
+        const double ul = wetl ? ar.div(l[MU], rhl) : 0.0, ur = wetr ? ar.div(r[MU], rhr) : 0.0;
+        double vl = 0.0, vr = 0.0;
+        if (NDIM == 2) {
+            vl = wetl ? ar.div(l[mv], rhl) : 0.0;
+            vr = wetr ? ar.div(r[mv], rhr) : 0.0;
+        }
+        const double phil = l[MU] * ul + 0.5 * grav * (hl * hl);
+        const double phir = r[MU] * ur + 0.5 * grav * (hr * hr);
+        const double hl0 = dmax2(hl, 0.0), hr0 = dmax2(hr, 0.0);
+        const double sql = ar.sqrt(hl0), sqr = ar.sqrt(hr0);
+        const Recip rsq = ar.rcp(sql + sqr);
+        const double ubar = ar.div(sql * ul + sqr * ur, rsq);
+        const double vbar = (NDIM == 2) ? ar.div(sql * vl + sqr * vr, rsq) : 0.0;
+        double cbar;
+        Recip rc;
+        ar.sqrt_rcp(0.5 * grav * (hl0 + hr0), cbar, rc);
+        const double s1 = dmin2(ul - ar.sqrt(grav * hl0), ubar - cbar);
+        const double s3 = dmax2(ur + ar.sqrt(grav * hr0), ubar + cbar);
+        const double d1 = r[MU] - l[MU];
+        const double d2 = phir - phil + 0.5 * grav * (hl + hr) * (axr(0) - axl(0));
+        const Recip rds = ar.rcp(s3 - s1);
+        const double b1 = ar.div(s3 * d1 - d2, rds);
+        const double b3 = ar.div(d2 - s1 * d1, rds);
+        wave[0][0] = b1;
+        wave[MU][0] = b1 * s1;
+        s[0] = s1;
+        wave[0][NW - 1] = b3;
+        wave[MU][NW - 1] = b3 * s3;
+        s[NW - 1] = s3;
+        if (NDIM == 2) {
+            const double d3 = r[MU] * vr - l[MU] * vl;
+            wave[mv][0] = b1 * vl;
+            wave[0][1] = 0.0;
+            wave[MU][1] = 0.0;
+            wave[mv][1] = d3 - b1 * vl - b3 * vr;
+            s[1] = ubar;
+            wave[mv][NW - 1] = b3 * vr;
+        }
+#pragma unroll
+        for (int m = 0; m < MEQN; m++) {
+            double am = 0.0, ap = 0.0;
+#pragma unroll
+            for (int mw = 0; mw < NW; mw++) {
+                if (!nz(m, mw)) continue; // literal zeros: adding them to sums that start at +0 changes nothing
+                const double z = wave[m][mw];
+                if (s[mw] < 0.0) am = am + z;
+                else if (s[mw] > 0.0) ap = ap + z;
+                else { am = am + 0.5 * z; ap = ap + 0.5 * z; }
+            }
+            amdq[m] = am;
+            apdq[m] = ap;
+        }
+        roe[0] = ubar; roe[1] = vbar; roe[2] = cbar; roe[3] = ar.div(0.50, rc);
+    }
+
+    template <class AR>
+    __device__ __forceinline__ static void transverse(AR &ar, const RpParams &P, const double (&roe)[NROE],
+                                                      const double (&qc)[MEQN], const AuxCell &ax1,
+                                                      const AuxCell &ax2, const AuxCell &ax3,
+                                                      const double (&asdq)[MEQN],
+                                                      double (&bm)[MEQN], double (&bp)[MEQN])
+    {
+        if constexpr (NDIM == 2) {
+            if (roe[2] != 0.0) {
+                RpShallow<IXY>::transverse(ar, P, roe, qc, ax1, ax2, ax3, asdq, bm, bp);
+                return;
+            }
+        }
+#pragma unroll
+        for (int m = 0; m < MEQN; m++) { bm[m] = 0.0; bp[m] = 0.0; }
     }
 };
 

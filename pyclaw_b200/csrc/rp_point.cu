@@ -43,6 +43,7 @@ int claw_rp_point(const clawb200_problem *p, int ixy, long long n, const double 
         case CLAWB200_RP_EULER1D: GO(RpEuler1D);
         case CLAWB200_RP_NEL_FWAVE: { using R = RpElasticFwave<1, 1>; GO(R); }
         case CLAWB200_RP_ADVECTION_COLOR: { using R = RpColor<1, 1>; GO(R); }
+        case CLAWB200_RP_SHALLOW_BATHY_FWAVE: { using R = RpShallowBathyFwave<1, 1>; GO(R); }
         default: return fail(CLAWB200_ERR_UNSUPPORTED, "pointwise entry: no 1-D version of this solver");
         }
     }
@@ -54,6 +55,7 @@ int claw_rp_point(const clawb200_problem *p, int ixy, long long n, const double 
         case CLAWB200_RP_SHALLOW: GO(RpShallow<1>);
         case CLAWB200_RP_PSYSTEM: { using R = RpElasticFwave<2, 1>; GO(R); }
         case CLAWB200_RP_VC_ACOUSTICS: GO(RpVcAcoustics<1>);
+        case CLAWB200_RP_SHALLOW_BATHY_FWAVE: { using R = RpShallowBathyFwave<2, 1>; GO(R); }
         default: return fail(CLAWB200_ERR_UNSUPPORTED, "pointwise entry: not compiled for this solver");
         }
     }
@@ -64,6 +66,7 @@ int claw_rp_point(const clawb200_problem *p, int ixy, long long n, const double 
     case CLAWB200_RP_SHALLOW: GO(RpShallow<2>);
     case CLAWB200_RP_PSYSTEM: { using R = RpElasticFwave<2, 2>; GO(R); }
     case CLAWB200_RP_VC_ACOUSTICS: GO(RpVcAcoustics<2>);
+    case CLAWB200_RP_SHALLOW_BATHY_FWAVE: { using R = RpShallowBathyFwave<2, 2>; GO(R); }
     default: return fail(CLAWB200_ERR_UNSUPPORTED, "pointwise entry: not compiled for this solver");
     }
 #undef GO

@@ -9,7 +9,7 @@ keys of ``state.aux_global`` (the cparam common block the script fills).
 from .._lib import (RP_ACOUSTICS, RP_ADVECTION, RP_EULER5, RP_SHALLOW, RP_SPHERE, RP_NEL_FWAVE,
                     RP_PSYSTEM, RP_ACOUSTICS3D_VC, RP_VC_ACOUSTICS, RP_BURGERS, RP_ADVECTION_COLOR,
                     RP_VC_ADVECTION, RP_EULER1D, RP_ADVECTION3D, RP_EULER3D,
-                    RP_ADVECTION3D_VC_FWAVE)
+                    RP_ADVECTION3D_VC_FWAVE, RP_SHALLOW_BATHY_FWAVE)
 
 
 class RiemannSolver(object):
@@ -105,6 +105,12 @@ nonlinear_elasticity_fwave = RiemannSolver("nonlinear_elasticity_fwave", RP_NEL_
                                            (1,), optional=["stress_law"], defaults={"stress_law": 2.0},
                                            fwave=True, maux=2)
 psystem = RiemannSolver("psystem", RP_PSYSTEM, 3, 2, [], (2,), fwave=True, maux=4)
+# shallow water over bathymetry (1-D, 2-D), well balanced: aux = {b}, the bottom elevation (surface
+# eta = h + b); cells with h <= dry_tolerance have zero velocity.  Classic solvers only.
+shallow_bathymetry_fwave = RiemannSolver("shallow_bathymetry_fwave", RP_SHALLOW_BATHY_FWAVE, lambda ndim: ndim + 1,
+                                         lambda ndim: ndim + 1, ["grav", "dry_tolerance"], (1, 2),
+                                         optional=["dry_tolerance"], defaults={"dry_tolerance": 1e-3},
+                                         fwave=True, maux=1)
 
 # 3-D acoustics in a heterogeneous medium (test/acoustics/3d): aux = {impedance, sound speed}
 vc_acoustics_3d = RiemannSolver("vc_acoustics_3d", RP_ACOUSTICS3D_VC, 4, 2, [], (3,), maux=2)
@@ -158,7 +164,7 @@ def from_header(header, name=None, meqn=1, mwaves=1, ndims=(2,), param_names=(),
 _BY_NAME = {s.name: s for s in (vc_acoustics, burgers, advection_color, vc_advection, euler_with_efix,
                                 vc_acoustics_3d, advection_3d, euler_3d, vc_advection_fwave_3d,
                                 acoustics, advection, euler_5wave, shallow_roe_with_efix, shallow_sphere,
-                                nonlinear_elasticity_fwave, psystem)}
+                                nonlinear_elasticity_fwave, psystem, shallow_bathymetry_fwave)}
 _BY_NAME.update({"euler": euler_5wave, "shallow": shallow_roe_with_efix})
 
 

@@ -287,6 +287,12 @@ class SharpClawSolver(Solver):
         # clawparams.mcapa = state.mcapa + 1 (sharpclaw.py:270)
         method = [int(self.dt_variable), 2, 0, 0, 0, state.mcapa + 1, state.maux]
         self._setup_device(state, method=method, mthlim=self.mthlim, weno_variant=variant)
+        if self._rp.rp_id == _lib.RP_SHALLOW_BATHY_FWAVE:
+            # WENO reconstructs h rather than the surface h + b: the in-cell solve is not balanced and a
+            # lake at rest would move (that needs a surface / hydrostatic reconstruction)
+            raise NotImplementedError("shallow_bathymetry_fwave runs with ClawSolver1D / ClawSolver2D only: "
+                                      "SharpClaw's component-wise WENO reconstruction is not well balanced "
+                                      "over bathymetry")
         self._weno_tab = tab if variant == _lib.WENO_TABLES else None
         self._upload_weno_tables()
         self.allocate_bc_arrays(state)
