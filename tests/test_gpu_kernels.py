@@ -337,8 +337,9 @@ def test_host_slab_pipeline(rp):
 @pytest.mark.parametrize("shape", [(1, 1), (2, 3), (4, 4), (125, 64), (126, 65), (124, 63), (250, 128),
                                    (251, 129), (127, 1), (1, 130), (376, 5)])
 def test_tile_boundary_shapes(shape):
-    """Grid sizes at and around the CTA tile sizes (125 / 126 columns, 64-row strips) and
-    degenerate grids: classic unsplit + dim-split (Euler) and SharpClaw (shallow)."""
+    """Grid sizes at and around the CTA column tiles (125 / 126 columns) and degenerate grids:
+    classic unsplit + dim-split (Euler) and SharpClaw (shallow).  All of them run at 8-row strips;
+    the taller strips of large grids are tested in test_gpu_strip_heights.py."""
     mx, my = shape
     dx, dy, dt = 0.01, 0.013, 0.0011
     cfl_g = ctypes.c_double()
