@@ -36,6 +36,9 @@ static int check_problem(const clawb200_problem *p, int ndim)
     if (p->mx < 1 || p->my < 1) return fail(CLAWB200_ERR_INVALID, "mx, my must be positive");
     if (p->mwaves < 1 || p->mwaves > CLAWB200_MAXWAVES) return fail(CLAWB200_ERR_INVALID, "bad mwaves");
     if (p->pitch < p->mx + 2 * p->mbc) return fail(CLAWB200_ERR_INVALID, "pitch smaller than padded row");
+    // a smaller component stride would make the sweeps' ghost rows of one component the first rows of the next
+    if (ndim == 2 && p->mstride < (long long)p->pitch * (p->my + 2 * p->mbc))
+        return fail(CLAWB200_ERR_INVALID, "mstride smaller than the padded field");
     if (p->method[5] < 0 || p->method[5] > p->maux)
         return fail(CLAWB200_ERR_INVALID, "method[5] (mcapa+1) must index an aux component");
     return 0;
@@ -859,10 +862,16 @@ static int host_pipeline(const clawb200_problem *p, const double *qold, double *
     // slab height: PCIe time is the bound, the first upload and the last download are the only
     // transfers that do not overlap, so slabs are kept small
     constexpr int slab_rows = 128;
-    int nslab = (out1 - out0 + slab_rows - 1) / slab_rows;
+    const int nout = out1 - out0;
+    int nslab = (nout + slab_rows - 1) / slab_rows;
     if (nslab < 1) nslab = 1;
-    const int rows_per = (out1 - out0 + nslab - 1) / nslab;
-    const size_t nmax = rowd * (size_t)(rows_per + 2 * mbc);
+    // Slab k produces rows out0 + [k nout / nslab, (k + 1) nout / nslab): every slab has
+    // floor(nout / nslab) or ceil(nout / nslab) rows, at least 64 for the grids sent here: a
+    // mode-1 slab presents its first and last mbc rows as ghost rows and needs interior rows besides.
+    const int rows_min = nout / nslab, rows_max = (nout + nslab - 1) / nslab;
+    if ((mode == 1 ? rows_min - 2 * mbc : rows_min) < 1)
+        return fail(CLAWB200_ERR_INVALID, "internal: host pipeline slab without interior rows");
+    const size_t nmax = rowd * (size_t)(rows_max + 2 * mbc);
     int rc = g_hs.ensure(16);
     if (rc) return rc;
     if ((rc = g_pipe.ensure(nmax))) return rc;
@@ -871,9 +880,8 @@ static int host_pipeline(const clawb200_problem *p, const double *qold, double *
     int prev_r0 = 0, prev_off = 0, prev_n = 0, last = -1;
     for (int k = 0; k < nslab; k++) {
         const int b = k % SlabPipe::NBUF;
-        const int r0 = out0 + k * rows_per;
-        const int r1 = (r0 + rows_per < out1) ? r0 + rows_per : out1;
-        if (r0 >= r1) break;
+        const int r0 = out0 + (int)((long long)k * nout / nslab);
+        const int r1 = out0 + (int)((long long)(k + 1) * nout / nslab);
         const int in0 = r0 - halo, in1 = r1 + halo; // input rows [in0, in1)
         const int nrow_in = in1 - in0;
         // the slab as a stand-alone problem in device layout
@@ -881,9 +889,7 @@ static int host_pipeline(const clawb200_problem *p, const double *qold, double *
         P.dt_dev = nullptr;
         P.pitch = nx;
         P.my = (mode == 1) ? nrow_in - 2 * mbc : r1 - r0;
-        if (mode == 1 && P.my < 1) P.my = 1;
-        const int ny_s = (mode == 1) ? nrow_in : nrow_in;
-        P.mstride = (long long)nx * ny_s;
+        P.mstride = (long long)nx * nrow_in;
         const size_t nd = rowd * (size_t)nrow_in;
         // buffer b is free once the download of slab k-NBUF has completed
         if (k >= SlabPipe::NBUF) {

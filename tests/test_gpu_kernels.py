@@ -305,7 +305,8 @@ def test_shallow_sphere_step(shape):
 @pytest.mark.parametrize("rp", ["acoustics", "euler"])
 def test_host_slab_pipeline(rp):
     """Tall grids go through the slab pipeline of the host entry points (upload / sweeps /
-    download overlapped); results must equal the oracle's single pass bit for bit."""
+    download overlapped); results must equal the oracle's single pass bit for bit.  Every slab
+    partition, the scratch and the host threads are tested in test_gpu_host_pipeline.py."""
     rp_id, params, meqn, mwaves, lim = RPS[rp]
     mx, my, mbc = 24, 1500, 2
     dx, dy, dt = 0.01, 0.013, 0.0011

@@ -48,17 +48,17 @@ def pick_rows(nrows, ncol_ctas, tall=True):
 
 
 def ctas_x(mx):
-    """x-engine, unsplit and step2ds: XNT - 3 columns per CTA (clawb200.cu:199, :365)"""
+    """x-engine, unsplit and step2ds: XNT - 3 columns per CTA (clawb200.cu:202, :368)"""
     return (mx + XNT - 4) // (XNT - 3)
 
 
 def ctas_y(mx):
-    """y-engine, unsplit: YNT - 2 columns per CTA (clawb200.cu:369)"""
+    """y-engine, unsplit: YNT - 2 columns per CTA (clawb200.cu:372)"""
     return (mx + YNT - 3) // (YNT - 2)
 
 
 def ctas_y_ds(mx, mbc):
-    """y-engine, step2ds: YNT columns of the padded row per CTA (clawb200.cu:204)"""
+    """y-engine, step2ds: YNT columns of the padded row per CTA (clawb200.cu:207)"""
     return (mx + 2 * mbc + YNT - 1) // YNT
 
 
